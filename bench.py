@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """bench.py -- headline benchmark: min-snap solves/s (3-D, N=10, 10 segments) on N B200s.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--skip-configs]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--skip-configs] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 \
         --master-port P bench.py --gpus N --steps K --warmup W
 
@@ -49,6 +49,8 @@ V_MAX, A_MAX, MAGIC = 3.0, 5.0, 6.5
 BOX_LO, BOX_HI = [-10.0, -20.0, -10.0], [10.0, 20.0, 10.0]
 BASE_SEED = 12345
 L2_BYTES = 126e6
+# --dump-outputs writes the coefficients of a fixed sample of the batch: 16,384 x 10 x 3 x 10 doubles = 39 MB
+DUMP_ROWS, DUMP_SEED = 16384, 20261020
 
 
 def bytes_in(K):
@@ -149,6 +151,12 @@ def dist_env():
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
     return rank, world, local
+
+
+def dump_rows(batch):
+    """The trajectories whose outputs --dump-outputs writes: a seeded sample of the batch, in increasing order."""
+    rng = np.random.default_rng(DUMP_SEED)
+    return np.sort(rng.choice(batch, size=min(DUMP_ROWS, batch), replace=False))
 
 
 def coeff_rel_err(c, ref):
@@ -623,6 +631,13 @@ def run_gpu_arm(args):
     elapsed_ms = max(all_ms)
     ms_per_step = elapsed_ms / args.steps
     value = world * B * args.steps / (elapsed_ms * 1e-3)
+    if args.dump_outputs and rank == 0:
+        # The buffer set the last timed step wrote.  Every set is solved from the same pos_h, so any set holds the same
+        # answer; this one is taken so that the file shows what the last step returned.
+        last = coeffs_d[(args.warmup + args.steps - 1) % n_sets]
+        rows = torch.from_numpy(dump_rows(B)).cuda()
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "coeffs.npy"), last.index_select(0, rows).cpu().numpy())
 
     # ---- e2e: host buffers through the C-ABI host entry point, copies inside the timed region
     pos_pin = torch.from_numpy(pos_h).pin_memory()
@@ -817,7 +832,14 @@ def main():
     ap.add_argument("--warmup", type=int, default=20)
     ap.add_argument("--impl", default="native", choices=["native", "reference"])
     ap.add_argument("--skip-configs", action="store_true", help="headline only (no configs[2..4] / target)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the coefficients the last headline step computed for a fixed, "
+                         "seeded sample of %d of rank 0's trajectories to DIR/coeffs.npy (float64)" % DUMP_ROWS)
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "native":
+        ap.error("--dump-outputs applies to the native arm")
     args.warmup = max(args.warmup, 3)
     if args.impl == "reference":
         run_reference_arm(args)

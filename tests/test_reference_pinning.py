@@ -1,24 +1,130 @@
 """The oracle against the REFERENCE ITSELF (CPU).  oracle/_ref/libmav_ref_core.so is the reference's own
-src/vertex.cpp, polynomial.cpp, segment.cpp, trajectory.cpp, motion_defines.cpp and rpoly.cpp compiled from
-/root/reference against the Eigen / glog stand-ins of oracle/ref_shim/ (oracle/Makefile target `ref`; the
-prebuilt file travels to machines without /root/reference).  Everything whose arithmetic order is the same
-is required to agree BIT FOR BIT: the input generator, the segment-time heuristic, the base-coefficient
-table, Horner evaluation, the segment search of Trajectory::evaluate, the time accumulation of
+src/vertex.cpp, polynomial.cpp, segment.cpp, trajectory.cpp, motion_defines.cpp and rpoly.cpp compiled from the
+reference's sources against the Eigen / glog stand-ins of oracle/ref_shim/ (oracle/Makefile target `ref`).  Everything
+whose arithmetic order is the same is required to agree BIT FOR BIT: the input generator, the segment-time heuristic,
+the base-coefficient table, Horner evaluation, the segment search of Trajectory::evaluate, the time accumulation of
 evaluateRange, the candidate polynomial of the extrema search.  Extrema values depend on the root finder
-(Jenkins-Traub in the reference, interval isolation in the oracle) and agree to 1e-8."""
+(Jenkins-Traub in the reference, interval isolation in the oracle) and agree to 1e-8.
+
+Without the library the bit-exact tests compare with what it returned for the same calls, stored in
+tests/golden/reference_pinning.npz (tests/golden/README.md: provenance, and how to regenerate it from the library).
+The tests marked live_only need the library itself."""
+import hashlib
+import os
+
 import numpy as np
 import pytest
 
 from oracle.oracle_py import Oracle, ReferenceCore, standard_mask, vertex_values_from_positions
 
-pytestmark = pytest.mark.skipif(not ReferenceCore.available(), reason="neither oracle/_ref nor /root/reference present")
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_pinning.npz")
+LIVE = ReferenceCore.available()
+live_only = pytest.mark.skipif(not LIVE, reason="needs the reference library oracle/_ref/libmav_ref_core.so")
+INLINE_BYTES = 8192     # larger return values are stored as their SHA-256 and shape
+
+
+def _call_key(name, args, index):
+    h = hashlib.sha256(name.encode())
+    for a in args:
+        h.update(np.ascontiguousarray(np.asarray(a, np.float64)).tobytes() + b"|")
+    return "%s#%s" % (h.hexdigest()[:40], index)
+
+
+class Digest:
+    """A stored return value too large to keep: its shape and the SHA-256 of its float64 bytes."""
+
+    def __init__(self, sha, shape):
+        self.sha, self.shape = sha, shape
+
+    def __len__(self):
+        return self.shape[0]
+
+
+def same(got, want):
+    """np.array_equal, also against a Digest."""
+    if isinstance(want, Digest):
+        got = np.ascontiguousarray(np.asarray(got, np.float64))
+        return got.shape == want.shape and hashlib.sha256(got.tobytes()).hexdigest() == want.sha
+    return np.array_equal(got, want)
+
+
+class GoldenReference:
+    """Answers the bit-exact tests' calls of ReferenceCore's methods from the stored return values."""
+
+    def __init__(self, path):
+        z = np.load(path)
+        self.entries = {}
+        for k, kind, shape, lo, hi, sha in zip(z["key"], z["kind"], z["shape"], z["start"], z["stop"], z["sha"]):
+            shape = tuple(int(n) for n in shape if n >= 0)
+            if kind == 1:
+                self.entries[k.decode()] = Digest(sha.decode(), shape)
+            else:
+                v = z["values"][lo:hi].reshape(shape)
+                self.entries[k.decode()] = float(v) if shape == () else v
+
+    def __getattr__(self, name):
+        def call(*args):
+            single = self.entries.get(_call_key(name, args, -1))
+            if single is not None:
+                return single
+            out, i = [], 0
+            while _call_key(name, args, i) in self.entries:
+                out.append(self.entries[_call_key(name, args, i)])
+                i += 1
+            assert out, "no stored reference result for %s; regenerate %s from the library" % (name, GOLDEN)
+            return tuple(out)
+        return call
+
+
+class RecordingReference:
+    """Wraps the live library and writes every call's return value in GoldenReference's format (regeneration:
+    tests/golden/README.md)."""
+
+    def __init__(self, lib):
+        self.lib, self.calls = lib, {}
+
+    def __getattr__(self, name):
+        def call(*args):
+            r = getattr(self.lib, name)(*args)
+            for i, v in ([(-1, r)] if not isinstance(r, tuple) else enumerate(r)):
+                self.calls[_call_key(name, args, i)] = np.asarray(v, np.float64)
+            return r
+        return call
+
+    def save(self, path):
+        keys, kind, shape, start, stop, sha, values, n = [], [], [], [], [], [], [], 0
+        for k, v in sorted(self.calls.items()):
+            v = np.ascontiguousarray(v)
+            keys.append(k)
+            shape.append(list(v.shape) + [-1] * (2 - v.ndim))
+            big = v.nbytes > INLINE_BYTES
+            kind.append(1 if big else 0)
+            sha.append(hashlib.sha256(v.tobytes()).hexdigest() if big else "")
+            start.append(n)
+            if not big:
+                values.append(v.reshape(-1))
+                n += v.size
+            stop.append(n)
+        np.savez_compressed(path, key=np.array(keys, "S"), kind=np.array(kind, np.int8), shape=np.array(shape, np.int64),
+                            start=np.array(start, np.int64), stop=np.array(stop, np.int64), sha=np.array(sha, "S"),
+                            values=np.concatenate(values))
+
 
 BOX_LO, BOX_HI = [-10.0, -20.0, -10.0], [10.0, 20.0, 10.0]
 
 
 @pytest.fixture(scope="module")
 def ref():
-    return ReferenceCore()
+    """The library when it is present (REFERENCE_PINNING_RECORD=1 also rewrites the golden file from it), else the
+    stored return values."""
+    if not LIVE:
+        yield GoldenReference(GOLDEN)
+    elif os.environ.get("REFERENCE_PINNING_RECORD") == "1":
+        rec = RecordingReference(ReferenceCore())
+        yield rec
+        rec.save(GOLDEN)
+    else:
+        yield ReferenceCore()
 
 
 @pytest.fixture(scope="module")
@@ -92,6 +198,7 @@ def test_polynomial_evaluate_bit_exact(ref, orc):
                     assert got == every[d]
 
 
+@live_only
 def test_candidate_polynomial_bit_exact(ref, orc, solved):
     """ref Segment::computeMinMaxMagnitudeCandidateTimes (src/segment.cpp:93-116): getCoefficients, head, convolve
     and the order in which the dimensions are added."""
@@ -143,10 +250,11 @@ def test_evaluate_range_bit_exact(ref, orc, solved, dt):
                 want, want_t = ref.trajectory_evaluate_range(coeffs, times, t0, t1, dt, d)
                 got, got_t = orc.trajectory_evaluate_range(coeffs, times, t0, t1, dt, d)
                 assert len(got) == len(want)
-                assert np.array_equal(got_t, want_t)
-                assert np.array_equal(got, want)
+                assert same(got_t, want_t)
+                assert same(got, want)
 
 
+@live_only
 def test_minmax_magnitude_against_reference(ref, orc, solved):
     """ref Trajectory::computeMinMaxMagnitude (src/trajectory.cpp:181-217) over the reference's own Jenkins-Traub
     roots, against the oracle's interval isolation: extremal values to 1e-8 relative, same segment."""
@@ -164,6 +272,7 @@ def test_minmax_magnitude_against_reference(ref, orc, solved):
             assert ok and abs(r1["max"][1] - mx1[1]) <= 1e-8 * max(1.0, abs(mx1[1]))
 
 
+@live_only
 def test_segment_candidates_against_reference(ref, orc, solved):
     """ref Segment::computeMinMaxMagnitudeCandidates (src/segment.cpp:132-156): the largest candidate value of an
     inner segment agrees with the oracle's segment maximum."""
@@ -188,6 +297,7 @@ def test_product_input_generator_against_reference(ref):
         assert np.array_equal(got[b], want)
 
 
+@live_only
 @pytest.mark.gpu
 def test_gpu_path_against_reference_itself(ref):
     """Solve on the GPU, then sample and evaluate ranges on the GPU, and compare with the REFERENCE's own
