@@ -134,7 +134,10 @@ MINSNAP_API int minsnap_cost(long B, int K, int D, int N, int derivative, const 
  * End vertices fix derivatives 0..h-1, interior vertices fix position only; N = 10, snap.
  * d_end_derivatives [B][2][h-1][D] (start then end vertex, derivatives 1..h-1) or NULL = zeros.
  * d_times NULL => times are computed on the device from (v_max, a_max, magic) exactly as
- * minsnap_estimate_segment_times does and, when d_times_out != NULL, written there. */
+ * minsnap_estimate_segment_times does and, when d_times_out != NULL, written there.
+ * The environment variable MINSNAP_STANDARD_ROUTE=tm|pair|pair_long|bcr|chunked|general (read on every call) runs
+ * the named kernel instead of the one the shape and batch size select, for tests that compare two kernels:
+ * MINSNAP_ERR_UNSUPPORTED when that kernel cannot take the call, MINSNAP_ERR_ARG for any other name. */
 MINSNAP_API int minsnap_solve_standard(long B, int K, int D, int N, int derivative,
                                        const double* d_positions, const double* d_end_derivatives,
                                        const double* d_times, double v_max, double a_max,

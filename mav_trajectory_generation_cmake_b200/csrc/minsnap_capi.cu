@@ -399,7 +399,18 @@ int minsnap_solve_standard(long B, int K, int D, int N, int derivative, const do
   a.d_positions = d_positions; a.d_end_derivatives = d_end_derivatives; a.d_times = d_times;
   a.v_max = v_max; a.a_max = a_max; a.magic = magic; a.d_times_out = d_times_out;
   a.d_coeffs = d_coeffs; a.d_free_out = d_free_values; a.d_cost = d_cost; a.d_status = d_status;
-  CU(minsnap::launch_solve_standard(a, as_stream(stream)));
+  // MINSNAP_STANDARD_ROUTE=tm|pair|pair_long|bcr|chunked|general runs that kernel, so that tests can compare two
+  // kernels on the same inputs: MINSNAP_ERR_UNSUPPORTED where it cannot take the call, never another kernel;
+  // MINSNAP_ERR_ARG for an unknown name.
+  if (const char* name = std::getenv("MINSNAP_STANDARD_ROUTE")) {
+    for (int r = 0; r < static_cast<int>(minsnap::StandardRoute::Unsupported); ++r)
+      if (std::strcmp(name, minsnap::standard_route_name(static_cast<minsnap::StandardRoute>(r))) == 0)
+        a.forced = static_cast<minsnap::StandardRoute>(r);
+    if (!a.forced) return MINSNAP_ERR_ARG;
+  }
+  const cudaError_t e = minsnap::launch_solve_standard(a, as_stream(stream));
+  if (e == cudaErrorNotSupported && a.forced) return MINSNAP_ERR_UNSUPPORTED;
+  CU(e);
   return MINSNAP_OK;
 }
 
@@ -792,13 +803,9 @@ int minsnap_solve_standard_host(long B, int K, int D, int N, int derivative, con
 #define TRY(x) do { cudaError_t e__ = (x); if (e__ != cudaSuccess) { rc = cuda_fail(e__, #x); goto done; } } while (0)
   const int h = N / 2;
   const int n_free = (K - 1) * (h - 1);
-  // chunk = unit of the copy/solve/copy pipeline (MINSNAP_TUNE_HOST_CHUNK overrides for measurements)
-  long chunk_pref = 4096;   // measured on B200 + PCIe Gen5: 4096-8192 is best (D2H stays busy, small pipeline fill)
-  if (const char* v = std::getenv("MINSNAP_TUNE_HOST_CHUNK")) {
-    const long want = std::atol(v);
-    if (want >= 16) chunk_pref = want;
-  }
-  const long chunk = std::min<long>(B, chunk_pref);
+  // chunk = unit of the copy/solve/copy pipeline; measured on B200 + PCIe Gen5: 4096-8192 is best (D2H stays busy,
+  // small pipeline fill)
+  const long chunk = std::min<long>(B, 4096);
   // Stage layout: one device block per pipeline stage, carved into the per-chunk arrays.
   const size_t nc = (size_t)chunk;
   size_t off = 0;

@@ -12,6 +12,8 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include <type_traits>
+
 // __constant__: kernels that index the tables with compile-time constants get c[bank][offset]
 // operands straight into DFMA/DMUL (no loads, no immediate moves)
 #define MINSNAP_TABLE_QUAL static __constant__
@@ -124,6 +126,30 @@ __device__ inline double warp_sum(double v) {
 #pragma unroll
   for (int off = 16; off > 0; off >>= 1) v += __shfl_xor_sync(0xffffffffu, v, off);
   return v;
+}
+
+// Stream-ordered scratch memory, freed on `stream` when it goes out of scope (after the work enqueued so far).
+struct AsyncBuffer {
+  void* ptr = nullptr;
+  cudaStream_t stream = nullptr;
+  cudaError_t alloc(size_t bytes, cudaStream_t s) {
+    stream = s;
+    return cudaMallocAsync(&ptr, bytes ? bytes : 16, s);
+  }
+  ~AsyncBuffer() {
+    if (ptr) cudaFreeAsync(ptr, stream);
+  }
+};
+
+// f(std::integral_constant<int, D>) for the dimension counts D = 1..3 the standard-mask kernels are compiled for.
+template <class F>
+inline cudaError_t with_dim(int D, F&& f) {
+  switch (D) {
+    case 1: return f(std::integral_constant<int, 1>{});
+    case 2: return f(std::integral_constant<int, 2>{});
+    case 3: return f(std::integral_constant<int, 3>{});
+    default: return cudaErrorInvalidValue;
+  }
 }
 
 }  // namespace minsnap

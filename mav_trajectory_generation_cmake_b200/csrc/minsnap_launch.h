@@ -5,6 +5,8 @@
 #include <stddef.h>
 #include <stdint.h>
 
+#include <optional>
+
 namespace minsnap {
 
 // Largest dynamic shared memory a CTA may request on sm_100 (227 KB).
@@ -67,6 +69,15 @@ cudaError_t launch_time_select(long B, int S, int K, const double* d_cand, const
                                double* d_times, double* d_incumbent, double* d_history_row, cudaStream_t stream);
 
 // ---- minsnap_standard.cu ---------------------------------------------------------------
+// The kernels behind minsnap_solve_standard; choose_standard_route (minsnap_standard_route.cuh) picks one.
+enum class StandardRoute { Tm, Pair, PairLong, Bcr, Chunked, General, Unsupported };
+
+// The names MINSNAP_STANDARD_ROUTE takes.
+inline const char* standard_route_name(StandardRoute r) {
+  static const char* const names[] = {"tm", "pair", "pair_long", "bcr", "chunked", "general", "unsupported"};
+  return names[static_cast<int>(r)];
+}
+
 struct StandardSolveArgs {
   long B;
   int K, D, N, derivative;
@@ -79,6 +90,7 @@ struct StandardSolveArgs {
   double* d_free_out;              // optional [B][n_free][D]
   double* d_cost;                  // optional
   int32_t* d_status;               // optional
+  std::optional<StandardRoute> forced;  // this route or cudaErrorNotSupported, never a fallback
 };
 bool standard_supported(int K, int D, int N, int derivative);
 cudaError_t launch_solve_standard(const StandardSolveArgs& a, cudaStream_t stream);

@@ -2,19 +2,11 @@
 // src/vertex.cpp:59,71-76) -- end vertices fix derivatives 0..h-1, interior vertices fix
 // position only.  n_fixed = K + 2h - 1, n_free = (K-1)(h-1).
 //
-// Two routes, both on the GPU:
-//   * fast route (minsnap_standard_fast.cuh): N = 10, snap, a thread pair per trajectory;
-//   * generic route: pack the inputs into the general layout and run the general kernels
-//     (any N, K, D, derivative the general path supports).
+// N = 10, snap, D <= 3 runs one of the standard-mask kernels (minsnap_standard_route.cuh picks it); every other
+// shape packs its inputs into the general layout and runs the general kernels.
 #include "minsnap_device.cuh"
 #include "minsnap_launch.h"
-#include <cstdlib>
-#include <cstring>
-
-#include "minsnap_standard_fast.cuh"
-#include "minsnap_standard_bcr.cuh"
-#include "minsnap_standard_tm.cuh"
-#include "minsnap_standard_chunked.cuh"
+#include "minsnap_standard_route.cuh"
 
 namespace minsnap {
 
@@ -47,18 +39,6 @@ __global__ void pack_standard_kernel(long B, int K, int D, int h, const double* 
     fixed_values[e] = val;
   }
 }
-
-struct AsyncBuffer {
-  void* ptr = nullptr;
-  cudaStream_t stream = nullptr;
-  cudaError_t alloc(size_t bytes, cudaStream_t s) {
-    stream = s;
-    return cudaMallocAsync(&ptr, bytes ? bytes : 16, s);
-  }
-  ~AsyncBuffer() {
-    if (ptr) cudaFreeAsync(ptr, stream);
-  }
-};
 
 static cudaError_t generic_route(long B, int S, int K, int D, int N, int derivative, const double* d_positions,
                                  const double* d_end_derivatives, const double* d_times, double* d_coeffs,
@@ -96,153 +76,98 @@ static cudaError_t generic_route(long B, int S, int K, int D, int N, int derivat
 }
 
 bool standard_supported(int K, int D, int N, int derivative) {
-  return fast::supported(K, D, N, derivative) ||
-         (N == 10 && derivative == 4 && D >= 1 && D <= 3 && K > fast::kMaxK && bcr::supported(K, D));
+  return choose_standard_route({1, K, D, N, derivative, sm_count(), true, true, {}}) != StandardRoute::General;
 }
 
-// Kernel choice for the fast route with coefficients: the second-generation kernel (block storage in
-// tensor memory, coefficients out through the TMA; minsnap_standard_tm.cuh) where it applies -- K = 2 or 4 <= K
-// up to 12 and a 16-byte aligned coefficient array -- else the first-generation two-lane kernel.
-// MINSNAP_STANDARD_KERNEL=pair forces the first generation (A/B measurements).
-static bool use_tm_kernel(const fast::FastParams& p, int D, int N, int derivative) {
-  if (!tm::supported(p.K, D, N, derivative) || p.sweep_S > 0 || !p.coeffs) return false;
-  if (reinterpret_cast<uintptr_t>(p.coeffs) % 16 != 0) return false;
-  const char* v = std::getenv("MINSNAP_STANDARD_KERNEL");
-  return !(v && std::strcmp(v, "pair") == 0);
+static bool aligned16(const void* ptr) { return reinterpret_cast<uintptr_t>(ptr) % 16 == 0; }
+
+// The parameters of the standard-mask kernels common to a solve and a cost sweep.
+static fast::FastParams fast_params(long B, int K, const double* positions, const double* end_derivatives,
+                                    const double* times, double* cost, int32_t* status) {
+  fast::FastParams p{};
+  p.B = B; p.K = K; p.positions = positions; p.end_derivatives = end_derivatives; p.times = times;
+  p.cost = cost; p.status = status;
+  return p;
 }
 
-static cudaError_t launch_fast_route(const fast::FastParams& p, int D, bool coeffs, bool tm_kernel, cudaStream_t stream) {
-  if (coeffs && tm_kernel) {
-    const cudaError_t e = tm::launch(p, D, stream);
-    if (e != cudaErrorNotSupported) return e;   // no tensor map: the first-generation kernel takes over
+static cudaError_t run_route(StandardRoute route, const StandardSolveArgs& a, const StandardRouteQuery& q,
+                             cudaStream_t stream) {
+  fast::FastParams p = fast_params(a.B, a.K, a.d_positions, a.d_end_derivatives, a.d_times, a.d_cost, a.d_status);
+  p.v_max = a.v_max; p.a_max = a.a_max; p.magic = a.magic; p.times_out = a.d_times_out;
+  p.coeffs = a.d_coeffs; p.free_out = a.d_free_out;
+  p.aligned16 = q.inputs_aligned16 && q.coeffs_aligned16;
+  // Without given times, Tm and Pair compute them in registers.  Chunked and General read them from memory: they are
+  // estimated first.  Bcr and PairLong compute them too, into a scratch times_out where a later pass reads them
+  // (Bcr's cost, PairLong's recovery).
+  AsyncBuffer times_scratch, free_scratch;
+  const bool estimate = route == StandardRoute::Chunked || route == StandardRoute::General;
+  const bool times_later = (route == StandardRoute::Bcr && p.cost) || route == StandardRoute::PairLong;
+  cudaError_t e;
+  if (!p.times && !p.times_out && (estimate || times_later)) {
+    if ((e = times_scratch.alloc(sizeof(double) * (size_t)a.B * a.K, stream)) != cudaSuccess) return e;
+    p.times_out = static_cast<double*>(times_scratch.ptr);
   }
-#define MINSNAP_FAST_CASE(D_) \
-  case D_:                    \
-    return coeffs ? fast::launch_d<D_, true>(p, stream) : fast::launch_d<D_, false>(p, stream);
-  switch (D) {
-    MINSNAP_FAST_CASE(1)
-    MINSNAP_FAST_CASE(2)
-    MINSNAP_FAST_CASE(3)
-    default: return cudaErrorInvalidValue;
+  if (!p.times && estimate) {
+    if ((e = launch_estimate_times(a.B, a.K, a.D, a.d_positions, a.v_max, a.a_max, a.magic, p.times_out, stream)) !=
+        cudaSuccess)
+      return e;
+    p.times = p.times_out;
   }
-#undef MINSNAP_FAST_CASE
+  const double* times = p.times ? p.times : p.times_out;
+  if (route == StandardRoute::General)
+    return generic_route(a.B, 1, a.K, a.D, a.N, a.derivative, a.d_positions, a.d_end_derivatives, times, a.d_coeffs,
+                         a.d_free_out, a.d_cost, a.d_status, stream);
+  // Bcr, Chunked and PairLong leave the cost to a pass over the coefficients (ref computeCost, LIN.i:113-130)
+  double* cost = nullptr;
+  if (route == StandardRoute::Bcr || route == StandardRoute::Chunked || route == StandardRoute::PairLong)
+    std::swap(cost, p.cost);
+  if (route == StandardRoute::PairLong && !p.free_out) {
+    if ((e = free_scratch.alloc(sizeof(double) * (size_t)a.B * (a.K - 1) * fast::kF * a.D, stream)) != cudaSuccess)
+      return e;
+    p.free_out = static_cast<double*>(free_scratch.ptr);
+  }
+  e = with_dim(a.D, [&](auto dim) {
+    constexpr int D = decltype(dim)::value;
+    switch (route) {
+      case StandardRoute::Tm: return tm::launch_d<D>(p, stream);
+      case StandardRoute::Pair: return fast::launch_d<D, true>(p, stream);
+      case StandardRoute::Bcr: return bcr::launch_d<D>(p, stream);
+      case StandardRoute::Chunked: return chunked::launch_d<D>(p, stream);
+      case StandardRoute::PairLong: {
+        // the two-lane kernel in long-chain mode: forward and backward sweeps only (free derivatives out), then the
+        // coefficients as a pass of their own with one thread per segment
+        const cudaError_t r = fast::launch_d<D, false>(p, stream);
+        return r != cudaSuccess ? r : bcr::launch_recover<D>(p, p.free_out, times, stream);
+      }
+      default: return cudaErrorInvalidValue;
+    }
+  });
+  if (e != cudaSuccess || !cost) return e;
+  return launch_cost(a.B, a.K, a.D, a.N, a.derivative, a.d_coeffs, times, cost, stream);
 }
 
 cudaError_t launch_solve_standard(const StandardSolveArgs& a, cudaStream_t stream) {
   if (a.B == 0) return cudaSuccess;
-  AsyncBuffer times_scratch;
-  const double* times = a.d_times;
-  cudaError_t e;
-  const bool fast_ok = fast::supported(a.K, a.D, a.N, a.derivative);
-  // the reduction kernel covers long chains whose staged inputs no longer fit the two-lane kernel
-  const bool bcr_ok = a.N == 10 && a.derivative == 4 && a.D >= 1 && a.D <= 3 && a.K > fast::kMaxK &&
-                      bcr::supported(a.K, a.D);
-  if (!times && !fast_ok && !bcr_ok) {
-    // the generic route needs the times in memory; the fast kernel computes them in-register
-    double* dst = a.d_times_out;
-    if (!dst) {
-      if ((e = times_scratch.alloc(sizeof(double) * (size_t)a.B * a.K, stream)) != cudaSuccess) return e;
-      dst = static_cast<double*>(times_scratch.ptr);
-    }
-    if ((e = launch_estimate_times(a.B, a.K, a.D, a.d_positions, a.v_max, a.a_max, a.magic, dst, stream)) !=
-        cudaSuccess)
-      return e;
-    times = dst;
-  }
-  if (fast_ok || bcr_ok) {
-    fast::FastParams p;
-    p.B = a.B; p.K = a.K; p.positions = a.d_positions; p.end_derivatives = a.d_end_derivatives;
-    p.times = a.d_times; p.v_max = a.v_max; p.a_max = a.a_max; p.magic = a.magic; p.times_out = a.d_times_out;
-    p.coeffs = a.d_coeffs; p.free_out = a.d_free_out; p.cost = a.d_cost; p.status = a.d_status; p.sweep_S = 0;
-    p.aligned16 = (reinterpret_cast<uintptr_t>(a.d_positions) % 16 == 0) &&
-                  (reinterpret_cast<uintptr_t>(a.d_times) % 16 == 0) &&
-                  (reinterpret_cast<uintptr_t>(a.d_coeffs) % 16 == 0);
-    // Long chains: block cyclic reduction, one CTA per trajectory (minsnap_standard_bcr.cuh), while
-    // the batch is too small to fill the machine with two-lane warps.  Measured at K = 256: a
-    // trajectory takes ~25 us through the reduction and two CTAs fit an SM, so B trajectories cost
-    // ceil(B / 296) x 25 us (64 -> 0.023 ms, 512 -> 0.052 ms, 4,096 -> 0.35 ms); the two-lane kernel
-    // (sweeps, then the separate recovery pass below) needs 0.17 ms however small the batch and
-    // 0.48 ms for 4,096, and keeps that time up to ~19,000 trajectories (16 per warp, 8 warps per
-    // SM).  MINSNAP_LONG_CHAIN_KERNEL=pair|bcr forces one.
-    const char* which = a.K > fast::kMaxK ? std::getenv("MINSNAP_LONG_CHAIN_KERNEL") : nullptr;
-    const int forced = !which ? 0 : std::strcmp(which, "pair") == 0 ? 1 : std::strcmp(which, "bcr") == 0 ? 2
-                                  : std::strcmp(which, "chunked") == 0 ? 3 : 0;
-    const bool small_batch = a.B <= sm_count() * 2 * 19;
-    // Partitioned route (minsnap_standard_chunked.cuh): chunk Schur complements, separator solve, then every chunk
-    // through the headline kernel.  Its four launches cost ~70 us however small the batch; the reduction kernel's
-    // ceil(B / 296) x 25 us is below that up to four waves (K = 256: 1,024 -> 0.100 against 0.107 ms, 4,096 ->
-    // 0.348 against 0.267 ms, 16,384 -> 1.35 against 0.93 ms).  MINSNAP_LONG_CHAIN_KERNEL=chunked forces it.
-    const bool chunk_ok = chunked::supported(a.K, a.D, a.N, a.derivative) && p.aligned16 &&
-                          reinterpret_cast<uintptr_t>(a.d_coeffs) % 16 == 0;
-    if (chunk_ok && (forced == 3 || (forced == 0 && a.B > sm_count() * 2 * 4))) {
-      double* cost = p.cost;
-      p.cost = nullptr;
-      if (!p.times) {
-        double* dst = p.times_out;
-        if (!dst) {
-          if ((e = times_scratch.alloc(sizeof(double) * (size_t)a.B * a.K, stream)) != cudaSuccess) return e;
-          dst = static_cast<double*>(times_scratch.ptr);
-        }
-        if ((e = launch_estimate_times(a.B, a.K, a.D, a.d_positions, a.v_max, a.a_max, a.magic, dst, stream)) != cudaSuccess)
-          return e;
-        p.times = dst;
-      }
-      e = chunked::launch(p, a.D, stream);
-      if (e == cudaSuccess && cost) return launch_cost(a.B, a.K, a.D, a.N, a.derivative, a.d_coeffs, p.times, cost, stream);
-      if (e != cudaErrorNotSupported) return e;
-      p.cost = cost;   // no tensor map: the older routes below
-      p.times = a.d_times;
-    }
-    if (bcr_ok && (!fast_ok || (forced != 1 && (small_batch || forced == 2)))) {
-      double* cost = p.cost;
-      p.cost = nullptr;
-      if (cost && !p.times && !p.times_out) {
-        // the cost pass below reads the segment times the kernel computes
-        if ((e = times_scratch.alloc(sizeof(double) * (size_t)a.B * a.K, stream)) != cudaSuccess) return e;
-        p.times_out = static_cast<double*>(times_scratch.ptr);
-      }
-      if ((e = bcr::launch(p, a.D, stream)) != cudaSuccess) return e;
-      // a16 from the coefficients (ref computeCost, LIN.i:113-130)
-      if (cost)
-        return launch_cost(a.B, a.K, a.D, a.N, a.derivative, a.d_coeffs, p.times ? p.times : p.times_out, cost, stream);
-      return cudaSuccess;
-    }
-    if (a.K > fast::kMaxK) {
-      // Two-lane kernel, long-chain mode: forward and backward sweeps only (free derivatives out), then
-      // the coefficients as a pass of their own with one thread per segment, then the cost from them.
-      AsyncBuffer free_scratch;
-      double* cost = p.cost;
-      p.cost = nullptr;
-      if (!p.free_out) {
-        if ((e = free_scratch.alloc(sizeof(double) * (size_t)a.B * (a.K - 1) * fast::kF * a.D, stream)) != cudaSuccess)
-          return e;
-        p.free_out = static_cast<double*>(free_scratch.ptr);
-      }
-      if (!p.times && !p.times_out) {
-        if ((e = times_scratch.alloc(sizeof(double) * (size_t)a.B * a.K, stream)) != cudaSuccess) return e;
-        p.times_out = static_cast<double*>(times_scratch.ptr);
-      }
-      if ((e = launch_fast_route(p, a.D, false, false, stream)) != cudaSuccess) return e;
-      const double* t = p.times ? p.times : p.times_out;
-      if ((e = bcr::launch_recover(p, a.D, p.free_out, t, stream)) != cudaSuccess) return e;
-      if (cost) return launch_cost(a.B, a.K, a.D, a.N, a.derivative, a.d_coeffs, t, cost, stream);
-      return cudaSuccess;
-    }
-    return launch_fast_route(p, a.D, true, use_tm_kernel(p, a.D, a.N, a.derivative), stream);
-  }
-  return generic_route(a.B, 1, a.K, a.D, a.N, a.derivative, a.d_positions, a.d_end_derivatives, times, a.d_coeffs,
-                       a.d_free_out, a.d_cost, a.d_status, stream);
+  const StandardRouteQuery q{a.B, a.K, a.D, a.N, a.derivative, sm_count(), aligned16(a.d_coeffs),
+                             aligned16(a.d_positions) && aligned16(a.d_times), a.forced};
+  const StandardRoute route = choose_standard_route(q);
+  if (route == StandardRoute::Unsupported) return cudaErrorNotSupported;
+  const cudaError_t e = run_route(route, a, q, stream);
+  // cudaErrorNotSupported: the headline kernel could not be set up (no tensor map).  Unforced, Tm falls back to the
+  // first-generation kernel and Chunked to the default decision without it.
+  if (e != cudaErrorNotSupported || q.forced) return e;
+  if (route == StandardRoute::Tm) return run_route(StandardRoute::Pair, a, q, stream);
+  if (route == StandardRoute::Chunked) return run_route(route_after_chunked(q), a, q, stream);
+  return e;
 }
 
 cudaError_t launch_cost_sweep(const SweepArgs& a, cudaStream_t stream) {
   if (a.B == 0) return cudaSuccess;
-  if (fast::sweep_supported(a.K, a.D, a.N, a.derivative)) {
-    fast::FastParams p;
-    p.B = a.B; p.K = a.K; p.positions = a.d_positions; p.end_derivatives = a.d_end_derivatives;
-    p.times = a.d_times; p.v_max = 0; p.a_max = 0; p.magic = 0; p.times_out = nullptr;
-    p.coeffs = nullptr; p.free_out = nullptr; p.cost = a.d_cost; p.status = a.d_status; p.sweep_S = a.S;
-    p.aligned16 = reinterpret_cast<uintptr_t>(a.d_times) % 16 == 0;
-    return launch_fast_route(p, a.D, false, false, stream);
+  if (fast::supported(a.K, a.D, a.N, a.derivative)) {
+    fast::FastParams p = fast_params(a.B, a.K, a.d_positions, a.d_end_derivatives, a.d_times, a.d_cost, a.d_status);
+    p.sweep_S = a.S;
+    p.aligned16 = aligned16(a.d_times);
+    return with_dim(a.D, [&](auto dim) { return fast::launch_d<decltype(dim)::value, false>(p, stream); });
   }
   return generic_route(a.B, a.S, a.K, a.D, a.N, a.derivative, a.d_positions, a.d_end_derivatives, a.d_times, nullptr,
                        nullptr, a.d_cost, a.d_status, stream);

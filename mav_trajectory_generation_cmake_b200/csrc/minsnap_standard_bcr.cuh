@@ -562,26 +562,11 @@ inline cudaError_t launch_d(const FastParams& p, cudaStream_t stream) {
   return cudaGetLastError();
 }
 
-inline cudaError_t launch_recover(const FastParams& p, int D, const double* free_values, const double* times,
-                                  cudaStream_t stream) {
+template <int D>
+inline cudaError_t launch_recover(const FastParams& p, const double* free_values, const double* times, cudaStream_t stream) {
   const long n = p.B * p.K;
-  const unsigned grid = (unsigned)((n + 127) / 128);
-  switch (D) {
-    case 1: recover_standard_kernel<1><<<grid, 128, 0, stream>>>(p, free_values, times); break;
-    case 2: recover_standard_kernel<2><<<grid, 128, 0, stream>>>(p, free_values, times); break;
-    case 3: recover_standard_kernel<3><<<grid, 128, 0, stream>>>(p, free_values, times); break;
-    default: return cudaErrorInvalidValue;
-  }
+  recover_standard_kernel<D><<<(unsigned)((n + 127) / 128), 128, 0, stream>>>(p, free_values, times);
   return cudaGetLastError();
-}
-
-inline cudaError_t launch(const FastParams& p, int D, cudaStream_t stream) {
-  switch (D) {
-    case 1: return launch_d<1>(p, stream);
-    case 2: return launch_d<2>(p, stream);
-    case 3: return launch_d<3>(p, stream);
-    default: return cudaErrorInvalidValue;
-  }
 }
 
 #undef H1T

@@ -630,25 +630,13 @@ __global__ void fold_chunk_status_kernel(long B, int J, const int32_t* __restric
   status[b] = s;
 }
 
-struct Scratch {
-  void* ptr = nullptr;
-  cudaStream_t stream = nullptr;
-  cudaError_t alloc(size_t bytes, cudaStream_t s) {
-    stream = s;
-    return cudaMallocAsync(&ptr, bytes ? bytes : 16, s);
-  }
-  ~Scratch() {
-    if (ptr) cudaFreeAsync(ptr, stream);
-  }
-};
-
 // Two internal streams per host thread and device (created once, never destroyed before the thread ends): the
 // sub-batches of a call run their kernel chains side by side, so that the latency-bound separator solve of one --
 // a 31-block chain on one warp per 16 trajectories -- overlaps the throughput-bound kernels of the other.  The fork
 // and the join are events on the caller's stream: stream order as the caller sees it is unchanged, and the whole
 // thing is capturable into a CUDA graph.
 struct SideStreams {
-  static constexpr int kN = 4;
+  static constexpr int kN = 2;
   int device = -1;
   cudaStream_t s[kN] = {};
   cudaEvent_t fork = nullptr, join[kN] = {};
@@ -714,7 +702,7 @@ inline cudaError_t run_range(const FastParams& p, const RangeScratch<D>& w, cuda
   // the chunks' interior free derivatives land in [B J][m-1][4][D]; the trajectory's array interleaves the
   // separators, so a caller asking for them gets them through the scatter below
   q.free_out = p.free_out ? w.chunk_free : nullptr;
-  if ((e = tm::launch(q, D, s)) != cudaSuccess) return e;
+  if ((e = tm::launch_d<D>(q, s)) != cudaSuccess) return e;
   if (p.free_out) {
     const long total = n_ch * (m - 1) * kVec;
     long grid = (total + 255) / 256;
@@ -742,16 +730,12 @@ inline cudaError_t launch_d(const FastParams& p, cudaStream_t stream) {
   // Sub-batches: two from 2,048 trajectories on (each still fills the machine in its Schur and chunk kernels); the
   // ranges are multiples of 16 trajectories so that every array of a range keeps its alignment.  Measured at
   // K = 256: 4,096 trajectories 247 -> 232 us, 16,384 848 -> 805 us; three and four sub-batches 237 / 812 us.
-  // MINSNAP_CHUNKED_LANES=1 switches the side streams off, 3 or 4 ask for more (A/B measurements).
-  static const int want_lanes = [] { const char* v = std::getenv("MINSNAP_CHUNKED_LANES"); return v ? std::atoi(v) : 2; }();
-  int lanes = 1;
-  if (want_lanes > 1 && p.B >= 2048 && side_streams().ready()) lanes = want_lanes < SideStreams::kN ? want_lanes : SideStreams::kN;
-  while (lanes > 1 && p.B / lanes < 1024) --lanes;
+  const int lanes = p.B >= 2048 && side_streams().ready() ? SideStreams::kN : 1;
   long first[SideStreams::kN + 1];
   for (int i = 0; i <= lanes; ++i) first[i] = i == lanes ? p.B : ((p.B * i / lanes) + 15) / 16 * 16;
 
   cudaError_t e;
-  Scratch rec, ends, st_chunk, st_extra, slots, sep_blocks, sep_edge, sep_middle, free_scratch;
+  AsyncBuffer rec, ends, st_chunk, st_extra, slots, sep_blocks, sep_edge, sep_middle, free_scratch;
   const long n_ch = p.B * J;
   const long warps16 = (p.B + 15) / 16 + lanes;   // every range rounds its warp count up
   if ((e = rec.alloc(sizeof(double) * (size_t)Fields<D>::kCount * n_ch, stream)) != cudaSuccess) return e;
@@ -800,15 +784,6 @@ inline cudaError_t launch_d(const FastParams& p, cudaStream_t stream) {
     if (e != cudaSuccess) { result = e; break; }
   }
   return result;
-}
-
-inline cudaError_t launch(const FastParams& p, int D, cudaStream_t stream) {
-  switch (D) {
-    case 1: return launch_d<1>(p, stream);
-    case 2: return launch_d<2>(p, stream);
-    case 3: return launch_d<3>(p, stream);
-    default: return cudaErrorInvalidValue;
-  }
 }
 
 #undef H1T

@@ -32,8 +32,6 @@
 #pragma once
 #include <cuda_pipeline.h>
 
-#include <cstdlib>
-
 #include "minsnap_device.cuh"
 #include "minsnap_launch.h"
 
@@ -49,30 +47,10 @@ constexpr int kMaxK = 24;
 
 #define H1T(r, s) (minsnap_tables::kH1_N10_d4[(r) * 10 + (s)])
 #define A1T(i, r) (minsnap_tables::kA1inv_N10[(i) * 10 + (r)])
-// coefficient store policy (measurement knob): 0 streaming (evict-first), 1 plain, 2 .cg, 3 .wt
 // 256-bit streaming store (PTX 8.8, sm_100+: STG.E.EF.ENL2.256); ptr must be 32-byte aligned.
 __device__ __forceinline__ void store_cs_v4(double* ptr, double a, double b, double c, double d) {
-#if defined(MINSNAP_STORE_POLICY) && MINSNAP_STORE_POLICY == 9
-  if (a == 1.2345678e300)
-#endif
   asm volatile("st.global.cs.v4.f64 [%0], {%1, %2, %3, %4};" ::"l"(ptr), "d"(a), "d"(b), "d"(c), "d"(d) : "memory");
 }
-
-#ifndef MINSNAP_STORE_POLICY
-#define MINSNAP_STORE_POLICY 0
-#endif
-#if MINSNAP_STORE_POLICY == 1
-#define MINSNAP_STORE2(ptr, val) (*(ptr) = (val))
-#elif MINSNAP_STORE_POLICY == 2
-#define MINSNAP_STORE2(ptr, val) __stcg(ptr, val)
-#elif MINSNAP_STORE_POLICY == 3
-#define MINSNAP_STORE2(ptr, val) __stwt(ptr, val)
-#elif MINSNAP_STORE_POLICY == 9
-// measurement only: the arithmetic stays, the store (practically) never executes
-#define MINSNAP_STORE2(ptr, val) do { if ((val).x == 1.2345678e300) __stcs(ptr, val); } while (0)
-#else
-#define MINSNAP_STORE2(ptr, val) __stcs(ptr, val)
-#endif
 
 // 1/x for a positive normal double: hardware seed (~20 bits) + two Newton steps.
 __device__ __forceinline__ double fast_rcp(double x) {
@@ -812,14 +790,14 @@ __global__ void __launch_bounds__(128) solve_standard_pair_kernel(FastParams p) 
               for (int e = 0; e + 4 <= n; e += 4)
                 store_cs_v4(dst + e, MINSNAP_CF(e), MINSNAP_CF(e + 1), MINSNAP_CF(e + 2), MINSNAP_CF(e + 3));
               if (n % 4 == 2)
-                MINSNAP_STORE2(reinterpret_cast<double2*>(dst + n - 2), make_double2(MINSNAP_CF(n - 2), MINSNAP_CF(n - 1)));
+                __stcs(reinterpret_cast<double2*>(dst + n - 2), make_double2(MINSNAP_CF(n - 2), MINSNAP_CF(n - 1)));
             } else {
-              MINSNAP_STORE2(reinterpret_cast<double2*>(dst), make_double2(MINSNAP_CF(0), MINSNAP_CF(1)));
+              __stcs(reinterpret_cast<double2*>(dst), make_double2(MINSNAP_CF(0), MINSNAP_CF(1)));
 #pragma unroll
               for (int e = 2; e + 4 <= n; e += 4)
                 store_cs_v4(dst + e, MINSNAP_CF(e), MINSNAP_CF(e + 1), MINSNAP_CF(e + 2), MINSNAP_CF(e + 3));
               if ((n - 2) % 4 == 2)
-                MINSNAP_STORE2(reinterpret_cast<double2*>(dst + n - 2), make_double2(MINSNAP_CF(n - 2), MINSNAP_CF(n - 1)));
+                __stcs(reinterpret_cast<double2*>(dst + n - 2), make_double2(MINSNAP_CF(n - 2), MINSNAP_CF(n - 1)));
             }
 #undef MINSNAP_CF
           } else {
@@ -879,7 +857,6 @@ inline bool supported(int K, int D, int N, int derivative) {
   if (K <= kMaxK) return true;
   return D == 1 ? inputs_fit<1>(K) : D == 2 ? inputs_fit<2>(K) : inputs_fit<3>(K);
 }
-inline bool sweep_supported(int K, int D, int N, int derivative) { return supported(K, D, N, derivative); }
 
 template <int D, bool kCoeffs, bool kGlobalSlots, bool kDirect = false>
 inline cudaError_t launch_mode(FastParams p, cudaStream_t stream) {
@@ -891,25 +868,13 @@ inline cudaError_t launch_mode(FastParams p, cudaStream_t stream) {
     const size_t cta = per_warp * w + 1024;
     if (per_warp * w > kMaxDynamicSmem) break;
     int resident = (int)((228 * 1024) / cta) * w;
-    if (resident > 8) resident = 8;             // 255 registers per thread: at most 8 warps per SM
+    // 255 registers per thread: at most 8 warps per SM.  Measured on B200 (65,536 x K=10) with the 32-byte
+    // coefficient stores: 6 warps 61.7 us, 7 warps 58.3 us, 8 warps 56.3 us; the cost-only kernel scales the same way.
+    if (resident > 8) resident = 8;
     if (resident > best) { best = resident; warps = w; }
   }
   if (per_warp * warps > kMaxDynamicSmem) return cudaErrorInvalidConfiguration;
-  size_t smem = per_warp * warps;
-  // Resident warps per SM.  Measured on B200 (65,536 x K=10) with the 32-byte coefficient stores:
-  // 6 warps 61.7 us, 7 warps 58.3 us, 8 warps (the register-file limit) 56.3 us; the cost-only
-  // kernel scales the same way.  MINSNAP_TUNE_MAX_WARPS overrides for measurements.
-  int cap = 8;
-  if (const char* v = std::getenv("MINSNAP_TUNE_MAX_WARPS")) {
-    const int want = std::atoi(v);
-    if (want >= 1) cap = want;
-  }
-  if (warps == 1 && cap < 8) {
-    // shared memory is carved in 256-byte units (ncu: padding to a multiple of 16 bytes that "fits" 7
-    // CTAs on paper leaves 6 resident)
-    const size_t need = ((228 * 1024) / (size_t)cap - 1024) & ~(size_t)255;
-    if (need > smem && need <= kMaxDynamicSmem && (228 * 1024) / (need + 1024) == (size_t)cap) smem = need;
-  }
+  const size_t smem = per_warp * warps;
   // the cost path is compiled out when no cost is requested (smaller hot loop, fewer registers)
   void (*kernel)(FastParams) = p.cost ? solve_standard_pair_kernel<D, kCoeffs, kGlobalSlots, true, kDirect>
                                       : solve_standard_pair_kernel<D, kCoeffs, kGlobalSlots, false, kDirect>;
@@ -945,43 +910,11 @@ inline cudaError_t launch_mode(FastParams p, cudaStream_t stream) {
 template <int D, bool kCoeffs>
 inline cudaError_t launch_d(const FastParams& p, cudaStream_t stream) {
   if (p.K <= kMaxK) {
-    // MINSNAP_TUNE_DIRECT=0/1 overrides the measured default (direct for the cost sweep only)
-    static const int tune = [] { const char* v = std::getenv("MINSNAP_TUNE_DIRECT"); return v ? std::atoi(v) : -1; }();
-    const bool direct = tune >= 0 ? tune == 1 : (!kCoeffs && p.sweep_S > 0);
-    if (direct && p.times) return launch_mode<D, kCoeffs, false, true>(p, stream);
+    // direct reads for the cost sweep only (measured: see kDirect above)
+    if (!kCoeffs && p.sweep_S > 0 && p.times) return launch_mode<D, kCoeffs, false, true>(p, stream);
     return launch_mode<D, kCoeffs, false>(p, stream);
   }
   return launch_mode<D, kCoeffs, true>(p, stream);
-}
-
-inline cudaError_t launch(const StandardSolveArgs& a, cudaStream_t stream) {
-  FastParams p;
-  p.B = a.B; p.K = a.K; p.positions = a.d_positions; p.end_derivatives = a.d_end_derivatives;
-  p.times = a.d_times; p.v_max = a.v_max; p.a_max = a.a_max; p.magic = a.magic; p.times_out = a.d_times_out;
-  p.coeffs = a.d_coeffs; p.free_out = a.d_free_out; p.cost = a.d_cost; p.status = a.d_status; p.sweep_S = 0;
-  p.aligned16 = (reinterpret_cast<uintptr_t>(a.d_positions) % 16 == 0) &&
-                (reinterpret_cast<uintptr_t>(a.d_times) % 16 == 0) &&
-                (reinterpret_cast<uintptr_t>(a.d_coeffs) % 16 == 0);
-  switch (a.D) {
-    case 1: return launch_d<1, true>(p, stream);
-    case 2: return launch_d<2, true>(p, stream);
-    case 3: return launch_d<3, true>(p, stream);
-    default: return cudaErrorInvalidValue;
-  }
-}
-
-inline cudaError_t launch_sweep(const SweepArgs& a, cudaStream_t stream) {
-  FastParams p;
-  p.B = a.B; p.K = a.K; p.positions = a.d_positions; p.end_derivatives = a.d_end_derivatives;
-  p.times = a.d_times; p.v_max = 0; p.a_max = 0; p.magic = 0; p.times_out = nullptr;
-  p.coeffs = nullptr; p.free_out = nullptr; p.cost = a.d_cost; p.status = a.d_status; p.sweep_S = a.S;
-  p.aligned16 = reinterpret_cast<uintptr_t>(a.d_times) % 16 == 0;
-  switch (a.D) {
-    case 1: return launch_d<1, false>(p, stream);
-    case 2: return launch_d<2, false>(p, stream);
-    case 3: return launch_d<3, false>(p, stream);
-    default: return cudaErrorInvalidValue;
-  }
 }
 
 }  // namespace fast

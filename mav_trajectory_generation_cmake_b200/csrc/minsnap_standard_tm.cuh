@@ -32,7 +32,6 @@
 #pragma once
 #include <cuda.h>
 #include <algorithm>
-#include <cstdio>
 #include <cstdlib>
 
 #include "minsnap_standard_fast.cuh"
@@ -870,23 +869,22 @@ inline cudaError_t launch_d(FastParams p, cudaStream_t stream) {
     }
     if (ctas < 1) ctas = 1;
   }
-  // Above two waves of CTAs a warp takes batches_per_warp batches (the second arrives in the other input
+  // Above two waves of CTAs a warp takes kBatchesPerWarp batches (the second arrives in the other input
   // buffer during the first; allocation, table, barrier and the final drain are paid once), and the grid stays a
   // whole number of waves so that every resident slot ends up with the same number of batches, give or take
   // one, as under one-batch CTAs: 65,536 solves, grid 1,024 -> 592: 43.2 -> 42.2 us.  (Grids that are not a
   // multiple of the slots lose to quantisation: 512 CTAs 47.3 us, 342 CTAs 55.8 us.)
+  constexpr long kBatchesPerWarp = 2;
   const long slots = (long)sms * ctas;
-  static const long batches_per_warp = [] { const char* v = std::getenv("MINSNAP_TM_BATCHES"); return v ? std::atol(v) : 2L; }();
   long grid = need;
-  if (batches_per_warp > 1 && need > 2 * slots) {
+  if (need > 2 * slots) {
     const long waves = (need + slots - 1) / slots;
-    grid = slots * ((waves + batches_per_warp - 1) / batches_per_warp);
+    grid = slots * ((waves + kBatchesPerWarp - 1) / kBatchesPerWarp);
     if (grid > need) grid = need;
   }
-  // MINSNAP_TM_PDL=0 switches programmatic dependent launch off (A/B measurements)
+  // MINSNAP_TM_PDL=0 switches programmatic dependent launch off: back-to-back launches may deadlock under it while
+  // launch_dependents precedes tcgen05.alloc (dependent CTAs can take the tensor memory a predecessor CTA waits for)
   static const int pdl = [] { const char* v = std::getenv("MINSNAP_TM_PDL"); return v ? std::atoi(v) : 1; }();
-  if (std::getenv("MINSNAP_TM_DEBUG"))
-    std::fprintf(stderr, "tm grid %ld need %ld slots %ld ctas %d sms %d smem %zu cols %d\n", grid, need, slots, ctas, sms, smem, cols);
   cudaLaunchConfig_t cfg = {};
   cfg.gridDim = dim3((unsigned)grid);
   cfg.blockDim = dim3(kWarpsPerCta * 32);
@@ -898,15 +896,6 @@ inline cudaError_t launch_d(FastParams p, cudaStream_t stream) {
   cfg.attrs = attr;
   cfg.numAttrs = pdl ? 1 : 0;
   return cudaLaunchKernelEx(&cfg, kernel, p, cols, sms * ctas * kWarpsPerCta, map, pdl);
-}
-
-inline cudaError_t launch(const FastParams& p, int D, cudaStream_t stream) {
-  switch (D) {
-    case 1: return launch_d<1>(p, stream);
-    case 2: return launch_d<2>(p, stream);
-    case 3: return launch_d<3>(p, stream);
-    default: return cudaErrorInvalidValue;
-  }
 }
 
 }  // namespace tm

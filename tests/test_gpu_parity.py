@@ -25,6 +25,13 @@ def batch_values(pos, N_=N):
     return np.stack([vertex_values(p, N_) for p in pos])
 
 
+def solve_on_route(ms, monkeypatch, route, *args, **kwargs):
+    """ms.solve_standard through the kernel MINSNAP_STANDARD_ROUTE names: that kernel or an error, never another."""
+    with monkeypatch.context() as m:
+        m.setenv("MINSNAP_STANDARD_ROUTE", route)
+        return ms.solve_standard(*args, **kwargs)
+
+
 # ------------------------------------------------------------------------------------------
 # a10 reordering: bit-exact
 # ------------------------------------------------------------------------------------------
@@ -286,18 +293,16 @@ def test_long_chain_kernels_agree(ms, oracle, torch_cuda, monkeypatch, D):
         pos = np.cumsum(rng.uniform(0.3, 2.0, (B, K + 1, D)) * rng.choice([-1.0, 1.0], (B, K + 1, D)), axis=1)
         ends = rng.normal(size=(B, 2, 4, D))
         outs = {}
-        for which in ("bcr", "pair"):
-            monkeypatch.setenv("MINSNAP_LONG_CHAIN_KERNEL", which)
-            outs[which] = ms.solve_standard(dev(torch, pos), None, end_derivatives=dev(torch, ends), v_max=3.0,
-                                            a_max=5.0, want_free=True, want_cost=True, want_times=True)
-        a, b = outs["bcr"], outs["pair"]
+        for which in ("bcr", "pair_long"):
+            outs[which] = solve_on_route(ms, monkeypatch, which, dev(torch, pos), None, end_derivatives=dev(torch, ends),
+                                         v_max=3.0, a_max=5.0, want_free=True, want_cost=True, want_times=True)
+        a, b = outs["bcr"], outs["pair_long"]
         assert (a["status"] == 0).all() and (b["status"] == 0).all()
         assert torch.equal(a["times"], b["times"])
         assert coeff_rel_err(a["coeffs"].cpu().numpy(), b["coeffs"].cpu().numpy()) <= 1e-9, K
         scale = b["free_values"].abs().amax(dim=(1, 2), keepdim=True)
         assert float(((a["free_values"] - b["free_values"]).abs() / scale).max()) <= 1e-9, K
         assert float((a["cost"] / b["cost"] - 1.0).abs().max()) <= 1e-9, K
-    monkeypatch.delenv("MINSNAP_LONG_CHAIN_KERNEL")
     if D == 3:
         # the reduction reaches K = 513 at D = 3 (the two-lane kernel does not): checked against the oracle
         K = 513
@@ -329,9 +334,8 @@ def test_long_chain_partitioned_route(ms, oracle, torch_cuda, monkeypatch, D):
         ends = rng.normal(size=(B, 2, 4, D))
         outs = {}
         for which in ("bcr", "chunked"):
-            monkeypatch.setenv("MINSNAP_LONG_CHAIN_KERNEL", which)
-            outs[which] = ms.solve_standard(dev(torch, pos), None, end_derivatives=dev(torch, ends), v_max=3.0,
-                                            a_max=5.0, want_free=True, want_cost=True, want_times=True)
+            outs[which] = solve_on_route(ms, monkeypatch, which, dev(torch, pos), None, end_derivatives=dev(torch, ends),
+                                         v_max=3.0, a_max=5.0, want_free=True, want_cost=True, want_times=True)
         a, b = outs["bcr"], outs["chunked"]
         assert (a["status"] == 0).all() and (b["status"] == 0).all(), K
         # the partitioned route runs the stand-alone estimateSegmentTimes kernel, the reduction kernel its own copy
@@ -341,10 +345,9 @@ def test_long_chain_partitioned_route(ms, oracle, torch_cuda, monkeypatch, D):
         assert float(((a["free_values"] - b["free_values"]).abs() / scale).max()) <= 1e-9, K
         assert float((a["cost"] / b["cost"] - 1.0).abs().max()) <= 1e-9, K
     # against the oracle, rest-to-rest, given times, K = 256 (BASELINE config 4's shape)
-    monkeypatch.setenv("MINSNAP_LONG_CHAIN_KERNEL", "chunked")
     K = 256
     pos, times = random_batch(oracle, 2, K, D=D)
-    out = ms.solve_standard(dev(torch, pos), dev(torch, times), want_cost=True)
+    out = solve_on_route(ms, monkeypatch, "chunked", dev(torch, pos), dev(torch, times), want_cost=True)
     ref = oracle_solve_batch(oracle, standard_mask(K), batch_values(pos), times)
     assert (out["status"] == 0).all()
     assert coeff_rel_err(out["coeffs"].cpu().numpy(), ref["coeffs"]) <= COEFF_TOL
@@ -352,10 +355,9 @@ def test_long_chain_partitioned_route(ms, oracle, torch_cuda, monkeypatch, D):
     # a non-positive segment time inside a chunk is reported for its trajectory only
     bad = times.copy()
     bad[1, 100] = -1.0
-    out = ms.solve_standard(dev(torch, pos), dev(torch, bad))
+    out = solve_on_route(ms, monkeypatch, "chunked", dev(torch, pos), dev(torch, bad))
     st = out["status"].cpu().numpy()
     assert st[0] == 0 and (st[1] & 2)
-    monkeypatch.delenv("MINSNAP_LONG_CHAIN_KERNEL")
 
 
 def test_long_chain_status_bits(ms, oracle, torch_cuda):
@@ -670,12 +672,9 @@ def test_two_kernel_generations_agree(ms, oracle, torch_cuda, monkeypatch, K, D)
     pos_d, end_d = dev(torch, pos), dev(torch, end)
     results = {}
     for name in ("tm", "pair"):
-        if name == "pair":
-            monkeypatch.setenv("MINSNAP_STANDARD_KERNEL", "pair")
-        results[name] = ms.solve_standard(pos_d, None, end_derivatives=end_d, v_max=3.0, a_max=5.0, want_cost=True,
-                                          want_free=True, want_times=True)
+        results[name] = solve_on_route(ms, monkeypatch, name, pos_d, None, end_derivatives=end_d, v_max=3.0, a_max=5.0,
+                                       want_cost=True, want_free=True, want_times=True)
         torch.cuda.synchronize()
-    monkeypatch.delenv("MINSNAP_STANDARD_KERNEL")
     a, b = results["tm"], results["pair"]
     assert int((a["status"] != 0).sum()) == 0 and int((b["status"] != 0).sum()) == 0
     assert np.array_equal(a["times"].cpu().numpy(), b["times"].cpu().numpy())
@@ -710,12 +709,9 @@ def test_two_batches_per_warp(ms, oracle, torch_cuda, monkeypatch, K, D):
     pos_d, end_d = dev(torch, pos), dev(torch, end)
     results = {}
     for name in ("tm", "pair"):
-        if name == "pair":
-            monkeypatch.setenv("MINSNAP_STANDARD_KERNEL", "pair")
-        results[name] = ms.solve_standard(pos_d, None, end_derivatives=end_d, v_max=3.0, a_max=5.0, want_cost=True,
-                                          want_free=True, want_times=True)
+        results[name] = solve_on_route(ms, monkeypatch, name, pos_d, None, end_derivatives=end_d, v_max=3.0, a_max=5.0,
+                                       want_cost=True, want_free=True, want_times=True)
         torch.cuda.synchronize()
-    monkeypatch.delenv("MINSNAP_STANDARD_KERNEL")
     a, b = results["tm"], results["pair"]
     assert int((a["status"] != 0).sum()) == 0 and int((b["status"] != 0).sum()) == 0
     assert torch.equal(a["times"], b["times"])
@@ -747,16 +743,29 @@ def test_partitioned_route_two_batches_per_warp(ms, torch_cuda, monkeypatch):
     ends = rng.normal(size=(B, 2, 4, D))
     outs = {}
     for which in ("bcr", "chunked"):
-        monkeypatch.setenv("MINSNAP_LONG_CHAIN_KERNEL", which)
-        outs[which] = ms.solve_standard(dev(torch, pos), None, end_derivatives=dev(torch, ends), v_max=3.0, a_max=5.0,
-                                        want_cost=True)
+        outs[which] = solve_on_route(ms, monkeypatch, which, dev(torch, pos), None, end_derivatives=dev(torch, ends),
+                                     v_max=3.0, a_max=5.0, want_cost=True)
         torch.cuda.synchronize()
-    monkeypatch.delenv("MINSNAP_LONG_CHAIN_KERNEL")
     a, b = outs["bcr"], outs["chunked"]
     assert (a["status"] == 0).all() and (b["status"] == 0).all()
     scale = a["coeffs"].abs().amax(dim=3, keepdim=True).clamp_min(1e-300)
     assert float(((a["coeffs"] - b["coeffs"]).abs() / scale).max()) <= 1e-9
     assert float((a["cost"] / b["cost"] - 1.0).abs().max()) <= 1e-9
+
+
+def test_forced_route_never_falls_back(ms, oracle, torch_cuda, monkeypatch):
+    """A route forced through MINSNAP_STANDARD_ROUTE that cannot take the call is an error, not another kernel; so
+    is a name that is no route."""
+    torch = torch_cuda
+    for route, K in (("tm", 3), ("chunked", 50)):
+        pos, times = random_batch(oracle, 4, K)
+        with pytest.raises(ms.MinsnapError) as err:
+            solve_on_route(ms, monkeypatch, route, dev(torch, pos), dev(torch, times))
+        assert err.value.code == ms.capi.ERR_UNSUPPORTED, route
+    pos, times = random_batch(oracle, 4, 10)
+    with pytest.raises(ms.MinsnapError) as err:
+        solve_on_route(ms, monkeypatch, "no_such_route", dev(torch, pos), dev(torch, times))
+    assert err.value.code == ms.capi.ERR_ARG
 
 
 def test_second_generation_status_bits(ms, torch_cuda):

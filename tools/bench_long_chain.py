@@ -6,8 +6,8 @@ for B in (296, 512, 1024, 4096, 16384):
     pos = torch.from_numpy(ms.random_positions_host(B, K, [-10.0, -20.0, -10.0], [10.0, 20.0, 10.0], 12345)).cuda()
     times = ms.estimate_segment_times(pos, 3.0, 5.0)
     coeffs = torch.empty((B, K, 3, 10), dtype=torch.float64, device="cuda")
-    for which in ("bcr", "pair", "chunked"):
-        os.environ["MINSNAP_LONG_CHAIN_KERNEL"] = which
+    for which in ("bcr", "pair_long", "chunked"):
+        os.environ["MINSNAP_STANDARD_ROUTE"] = which
         for _ in range(3): ms.solve_standard(pos, times, coeffs=coeffs, want_status=False)
         torch.cuda.synchronize()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)

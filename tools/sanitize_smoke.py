@@ -18,13 +18,13 @@ for K, B in ((10, 40), (9, 37), (5, 20), (3, 5), (33, 6), (64, 3), (100, 2)):
     out = ms.solve_standard(pos, times, end_derivatives=ends, want_free=True, want_cost=True)
     assert int((out["status"] != 0).sum()) == 0
     if K > 24:
-        for which in ("pair", "bcr", "chunked"):
+        for which in ("pair_long", "bcr", "chunked"):
             if which == "chunked" and K not in (64,):
                 continue
-            os.environ["MINSNAP_LONG_CHAIN_KERNEL"] = which
+            os.environ["MINSNAP_STANDARD_ROUTE"] = which
             o2 = ms.solve_standard(pos, None, v_max=3.0, a_max=5.0, want_times=True)
             assert torch.isfinite(o2["coeffs"]).all()
-        del os.environ["MINSNAP_LONG_CHAIN_KERNEL"]
+        del os.environ["MINSNAP_STANDARD_ROUTE"]
     s = ms.sample_uniform(out["coeffs"], times, 50, 5)
     e = ms.extrema(out["coeffs"], times, 1, mode=1, want_roots=True)
     g = ms.time_gradient(out["coeffs"], times)
