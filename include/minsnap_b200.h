@@ -299,6 +299,74 @@ MINSNAP_API int minsnap_collision_gradient(long B, int K, int D, int N, const do
                                            double* d_cost, double* d_grad_free, int32_t* d_is_collision,
                                            int32_t* d_charged, minsnap_stream_t stream);
 
+/* ---- the free derivatives (and segment times) against the collision cost ---------------------
+ * J = w_d J_d + w_c J_c + w_t sum(T), the objective of the reference's nonlinear optimiser over d_p (and T):
+ *   J_d = sum_dim d^T R d with d = [d_f; d_p]  (ref getCostAndGradientDerivative, NL.i:1452-1521) -- this is
+ *         2 computeCost, NOT computeCost;
+ *   J_c = the collision cost of minsnap_collision_cost  (ref getCostAndGradientCollision, NL.i:1523-1709);
+ *   w_t sum(T), whose time gradient is the w_t of minsnap_time_gradient  (ref getCostAndGradientTime,
+ *         NL.i:2155-2243).
+ * h_fixed_mask is a HOST pointer as in minsnap_solve; it reaches the device in a kernel's parameters, not by a copy.
+ *
+ * minsnap_derivative_gradient: at the given (d_f, d_p, T), any mask, any supported N and D:
+ *   d_cost_Jd [B]            J_d = d^T R d (2 computeCost);
+ *   d_grad_free [B][n_free][D] dJ_d/dd_p = 2 (R_pf d_f + R_pp d_p), in the layout of free_values;
+ *   d_diag_free [B][n_free]  (optional) diag(R_pp);
+ *   d_coeffs [B][K][D][N]    (optional) the coefficients, bit-identical to minsnap_coeffs_from_constraints.
+ * Deterministic: no atomics, the same bits on every run.  d_workspace: minsnap_solve_workspace_bytes(N, K) bytes. */
+MINSNAP_API int minsnap_derivative_gradient(long B, int K, int D, int N, int derivative,
+                                            const uint8_t* h_fixed_mask, const double* d_fixed_values,
+                                            const double* d_free_values, const double* d_times,
+                                            double* d_coeffs, double* d_cost_Jd, double* d_grad_free,
+                                            double* d_diag_free, void* d_workspace, size_t workspace_bytes,
+                                            minsnap_stream_t stream);
+
+/* minsnap_free_objective: J for S candidates per trajectory.  d_fixed_values [B][n_fixed][D] is shared by the S
+ * candidates of trajectory b; d_free_values [B][S][n_free][D], d_times [B][S][K] -> d_objective [B][S]; optional
+ * d_Jd, d_Jc [B][S] (the two terms before weighting) and d_is_collision [B][S].  The map and walk parameters are
+ * those of minsnap_collision_cost; D must be 3 and N 10 (MINSNAP_ERR_UNSUPPORTED otherwise).  Temporary device
+ * memory is allocated stream-ordered (cudaMallocAsync). */
+MINSNAP_API int minsnap_free_objective(long B, int S, int K, int D, int N, int derivative,
+                                       const uint8_t* h_fixed_mask, const double* d_fixed_values,
+                                       const double* d_free_values, const double* d_times, double w_d,
+                                       double w_c, double w_t, const double* d_sdf, const int32_t* h_dims,
+                                       const double* h_origin, double resolution, double oob_value,
+                                       const double* h_min_bound, const double* h_max_bound,
+                                       int use_continuous_distance, double dt, double map_resolution,
+                                       double epsilon, double robot_radius, double coll_pot_multiplier,
+                                       double* d_objective, double* d_Jd, double* d_Jc,
+                                       int32_t* d_is_collision, minsnap_stream_t stream);
+
+/* minsnap_optimize_free_constraints: an additive batched driver (NLopt, which the reference uses, is absent, so no
+ * parity is claimed for the optimiser -- only for the objective and the gradients it is built from).  Every
+ * trajectory descends J over its free derivatives d_p (d_free_values [B][n_free][D], in/out) and, with
+ * optimize_times != 0, its segment times (d_times [B][K], in/out).  Per iteration, at the incumbent: J_d, its
+ * gradient g_d and diag(R_pp) (minsnap_derivative_gradient), J_c and g_c (minsnap_collision_gradient), with
+ * optimize_times the time gradient w_d dJ_d/dT + w_t (minsnap_time_gradient, increment gradient_increment).  Then
+ * n_steps candidates, s = 0 .. n_steps-1, move both blocks with the same ladder index:
+ *   d_p - 2^-s (w_d g_d + w_c g_c) / (2 w_d diag(R_pp))   (at s = 0 and w_c = 0: the Jacobi step on J_d);
+ *   T   as minsnap_optimize_segment_times moves it without a penalty: T - (max_relative_step / 2^s) scale g_T,
+ *       scale = min_k T_k / |g_T,k|, clamped at min_time; the times stay when optimize_times == 0.
+ * minsnap_free_objective evaluates the candidates; the first minimum among the finite ones is accepted when it is
+ * strictly below the incumbent.  w_d > 0.  All launches are on `stream`, the workspace is one cudaMallocAsync and
+ * nothing returns to the host: the call can be captured into a CUDA graph once it has run eagerly on the thread.
+ * d_history (optional) [iterations + 1][B]: the incumbent J, first at the initial state; d_is_collision (optional)
+ * [B]: the collision flag at the returned state.  D must be 3 and N 10. */
+MINSNAP_API int minsnap_optimize_free_constraints(long B, int K, int D, int N, int derivative,
+                                                  const uint8_t* h_fixed_mask, const double* d_fixed_values,
+                                                  double* d_free_values, double* d_times, int optimize_times,
+                                                  double w_d, double w_c, double w_t, const double* d_sdf,
+                                                  const int32_t* h_dims, const double* h_origin,
+                                                  double resolution, double oob_value,
+                                                  const double* h_min_bound, const double* h_max_bound,
+                                                  int use_continuous_distance, double dt,
+                                                  double map_resolution, double epsilon,
+                                                  double robot_radius, double coll_pot_multiplier,
+                                                  int iterations, int n_steps, double max_relative_step,
+                                                  double min_time, double gradient_increment,
+                                                  double* d_history, int32_t* d_is_collision,
+                                                  minsnap_stream_t stream);
+
 /* ---- host-buffer entry points (synchronous; copies inside) -------------------------------
  * The calls a host program makes when its data lives in host memory.  Work is cut into
  * chunks that are copied and solved on alternating streams so that PCIe and the SMs overlap.
@@ -338,6 +406,12 @@ MINSNAP_API int minsnap_coeffs_from_constraints_host(long B, int K, int D, int N
                                                      const double* h_fixed_values,
                                                      const double* h_free_values,
                                                      const double* h_times, double* h_coeffs);
+MINSNAP_API int minsnap_derivative_gradient_host(long B, int K, int D, int N, int derivative,
+                                                 const uint8_t* h_fixed_mask,
+                                                 const double* h_fixed_values,
+                                                 const double* h_free_values, const double* h_times,
+                                                 double* h_coeffs, double* h_cost_Jd,
+                                                 double* h_grad_free, double* h_diag_free);
 MINSNAP_API int minsnap_cost_host(long B, int K, int D, int N, int derivative,
                                   const double* h_coeffs, const double* h_times, double* h_cost);
 

@@ -403,6 +403,155 @@ def collision_gradient(coeffs, times, sdf, origin, resolution, min_bound, max_bo
     return dict(cost=cost_t, gradient=grad, is_collision=hit, charged=charged)
 
 
+# ---- the free derivatives (and times) against w_d J_d + w_c J_c + w_t sum(T) ---------------------------------------
+def derivative_gradient(mask, fixed_values, free_values, times, N=10, derivative=SNAP, want_coeffs=False,
+                        want_diag=False):
+    """J_d = d^T R d (= 2 computeCost; ref getCostAndGradientDerivative, NL.i:1452-1521) and its gradient
+    2 (R_pf d_f + R_pp d_p) in the free derivatives, at the given constraints.  mask: host uint8 [(K+1)][h];
+    fixed_values [B][n_fixed][D], free_values [B][n_free][D], times [B][K] (CUDA tensors) -> dict(Jd [B],
+    gradient [B][n_free][D], diag [B][n_free] = diag(R_pp) or None, coeffs [B][K][D][N] or None)."""
+    torch = _torch()
+    mask = np.ascontiguousarray(mask, np.uint8)
+    K = mask.shape[0] - 1
+    B, _, D = fixed_values.shape
+    _, n_free = mask_counts(mask)
+    dev = times.device
+    jd = torch.empty((B,), dtype=torch.float64, device=dev)
+    grad = torch.empty((B, n_free, D), dtype=torch.float64, device=dev)
+    diag = torch.empty((B, n_free), dtype=torch.float64, device=dev) if want_diag else None
+    coeffs = torch.empty((B, K, D, N), dtype=torch.float64, device=dev) if want_coeffs else None
+    ws_bytes = _lib().minsnap_solve_workspace_bytes(N, K)
+    ws = torch.empty((ws_bytes,), dtype=torch.uint8, device=dev)
+    capi.check(_lib().minsnap_derivative_gradient(B, K, D, N, derivative, _hptr(mask), _dptr(fixed_values, torch.float64),
+                                                  _dptr(free_values, torch.float64), _dptr(times, torch.float64),
+                                                  _dptr(coeffs), _dptr(jd), _dptr(grad), _dptr(diag), _dptr(ws), ws_bytes,
+                                                  _stream()), "minsnap_derivative_gradient")
+    return dict(Jd=jd, gradient=grad, diag=diag, coeffs=coeffs)
+
+
+def _collision_map(sdf, origin, resolution, min_bound, max_bound, dt, map_resolution, epsilon, robot_radius,
+                   coll_pot_multiplier, use_continuous_distance, oob_value):
+    """The map and walk arguments of minsnap_collision_cost, in its order, and the host arrays they point into
+    (which must outlive the call)."""
+    torch = _torch()
+    if map_resolution is None:
+        map_resolution = resolution
+    host = (np.asarray(sdf.shape, np.int32), _np(origin, np.float64), _np(min_bound, np.float64),
+            _np(max_bound, np.float64))
+    dims, org, lo, hi = host
+    args = (_dptr(sdf, torch.float64), _hptr(dims), _hptr(org), float(resolution), float(oob_value), _hptr(lo), _hptr(hi),
+            int(bool(use_continuous_distance)), float(dt), float(map_resolution), float(epsilon), float(robot_radius),
+            float(coll_pot_multiplier))
+    return host, args
+
+
+def free_objective(mask, fixed_values, free_values, times, sdf, origin, resolution, min_bound, max_bound, w_c, w_d=0.1,
+                   w_t=1.0, dt=0.1, map_resolution=None, epsilon=0.5, robot_radius=0.5, coll_pot_multiplier=1.0,
+                   use_continuous_distance=True, oob_value=0.0, N=10, derivative=SNAP, want_terms=False):
+    """J = w_d J_d + w_c J_c + w_t sum(T) for S candidates per trajectory (minsnap_free_objective).  fixed_values
+    [B][n_fixed][3] is shared by the candidates of a trajectory; free_values [B][S][n_free][3], times [B][S][K] ->
+    objective [B][S] (with want_terms also dict(Jd, Jc, is_collision), each [B][S]).  The map arguments are those of
+    collision_cost.  w_d and w_t default to the reference's cost weights; w_c has no default."""
+    torch = _torch()
+    mask = np.ascontiguousarray(mask, np.uint8)
+    K = mask.shape[0] - 1
+    B, S = times.shape[0], times.shape[1]
+    D = fixed_values.shape[2]
+    dev = times.device
+    obj = torch.empty((B, S), dtype=torch.float64, device=dev)
+    terms = dict(Jd=torch.empty((B, S), dtype=torch.float64, device=dev),
+                 Jc=torch.empty((B, S), dtype=torch.float64, device=dev),
+                 is_collision=torch.empty((B, S), dtype=torch.int32, device=dev)) if want_terms else {}
+    host, margs = _collision_map(sdf, origin, resolution, min_bound, max_bound, dt, map_resolution, epsilon, robot_radius,
+                                 coll_pot_multiplier, use_continuous_distance, oob_value)
+    capi.check(_lib().minsnap_free_objective(B, S, K, D, N, derivative, _hptr(mask), _dptr(fixed_values, torch.float64),
+                                             _dptr(free_values, torch.float64), _dptr(times, torch.float64), float(w_d),
+                                             float(w_c), float(w_t), *margs, _dptr(obj), _dptr(terms.get("Jd")),
+                                             _dptr(terms.get("Jc")), _dptr(terms.get("is_collision")), _stream()),
+               "minsnap_free_objective")
+    return (obj, terms) if want_terms else obj
+
+
+def optimize_free_constraints(mask, fixed_values, free_values, times, sdf, origin, resolution, min_bound, max_bound, w_c,
+                              w_d=0.1, w_t=1.0, optimize_times=False, iterations=20, n_steps=8, max_relative_step=0.5,
+                              min_time=0.1, gradient_increment=1e-3, dt=0.1, map_resolution=None, epsilon=0.5,
+                              robot_radius=0.5, coll_pot_multiplier=1.0, use_continuous_distance=True, oob_value=0.0,
+                              N=10, derivative=SNAP):
+    """Additive batched driver for the reference's nonlinear problem over the free derivatives (and, with
+    optimize_times, the segment times): every trajectory descends J = w_d J_d + w_c J_c + w_t sum(T) along a
+    Jacobi-scaled step, the line search is one evaluation of n_steps candidates.  One C-ABI call
+    (minsnap_optimize_free_constraints): the whole loop is enqueued on the current stream.  The reference runs one
+    NLopt instance per trajectory on the host.  Returns (free_values, times, objective history [iterations + 1][B],
+    is_collision [B] at the returned state)."""
+    torch = _torch()
+    mask = np.ascontiguousarray(mask, np.uint8)
+    K = mask.shape[0] - 1
+    B, _, D = fixed_values.shape
+    free_values = free_values.clone().contiguous()
+    times = times.clone().contiguous()
+    history = torch.empty((iterations + 1, B), dtype=torch.float64, device=times.device)
+    hit = torch.empty((B,), dtype=torch.int32, device=times.device)
+    host, margs = _collision_map(sdf, origin, resolution, min_bound, max_bound, dt, map_resolution, epsilon, robot_radius,
+                                 coll_pot_multiplier, use_continuous_distance, oob_value)
+    capi.check(_lib().minsnap_optimize_free_constraints(B, K, D, N, derivative, _hptr(mask),
+                                                        _dptr(fixed_values, torch.float64), _dptr(free_values),
+                                                        _dptr(times), int(bool(optimize_times)), float(w_d), float(w_c),
+                                                        float(w_t), *margs, int(iterations), int(n_steps),
+                                                        float(max_relative_step), float(min_time),
+                                                        float(gradient_increment), _dptr(history), _dptr(hit), _stream()),
+               "minsnap_optimize_free_constraints")
+    return free_values, times, history, hit
+
+
+def optimize_free_constraints_reference_glue(mask, fixed_values, free_values, times, sdf, origin, resolution, min_bound,
+                                             max_bound, w_c, w_d=0.1, w_t=1.0, optimize_times=False, iterations=20,
+                                             n_steps=8, max_relative_step=0.5, min_time=0.1, gradient_increment=1e-3,
+                                             N=10, derivative=SNAP, **map_kw):
+    """The descent of optimize_free_constraints with its glue written in elementwise torch operations around the
+    C-ABI calls (derivative_gradient, collision_gradient, time_gradient, free_objective): kept as the checker of
+    minsnap_optimize_free_constraints in the tests."""
+    torch = _torch()
+    mask = np.ascontiguousarray(mask, np.uint8)
+    K = mask.shape[0] - 1
+    B, n_fixed, D = fixed_values.shape
+    dev = times.device
+    col, counts = reorder(torch.from_numpy(mask.reshape(1, -1)).to(dev), N, K)
+    n_free = int(counts[0, 1])
+    free, times = free_values.clone(), times.clone()
+    S = n_steps
+
+    def objective(f, t):
+        return free_objective(mask, fixed_values, f.contiguous(), t.contiguous(), sdf, origin, resolution, min_bound,
+                              max_bound, w_c, w_d=w_d, w_t=w_t, N=N, derivative=derivative, want_terms=True, **map_kw)
+
+    obj0, terms0 = objective(free[:, None], times[:, None])
+    history, hit = [obj0[:, 0]], terms0["is_collision"][:, 0]
+    ladder = 0.5 ** torch.arange(S, dtype=torch.float64, device=dev)
+    rows = torch.arange(B, device=dev)
+    for _ in range(iterations):
+        dg = derivative_gradient(mask, fixed_values, free, times, N=N, derivative=derivative, want_coeffs=True,
+                                 want_diag=True)
+        cg = collision_gradient(dg["coeffs"], times, sdf, origin, resolution, min_bound, max_bound, col_of_row=col[0],
+                                n_fixed=n_fixed, n_free=n_free, **map_kw)
+        step = (w_d * dg["gradient"] + w_c * cg["gradient"]) / ((2.0 * w_d) * dg["diag"][:, :, None])
+        cand_free = free[:, None] - ladder[None, :, None, None] * step[:, None]
+        if optimize_times:
+            g = time_gradient(dg["coeffs"], times, increment=gradient_increment, w_d=w_d, w_t=w_t, derivative=derivative)
+            scale = (times / g.abs().clamp_min(1e-300)).min(1, keepdim=True).values
+            cand_t = times[:, None, :] - ((max_relative_step * ladder)[None, :, None] * scale[:, :, None]) * g[:, None, :]
+            cand_t = cand_t.clamp_min(min_time)
+        else:
+            cand_t = times[:, None, :].expand(B, S, K)
+        obj, terms = objective(cand_free, cand_t)
+        best, arg = torch.where(torch.isfinite(obj), obj, torch.full_like(obj, float("inf"))).min(1)
+        improved = torch.isfinite(best) & (best < history[-1])
+        free = torch.where(improved[:, None, None], cand_free[rows, arg], free)
+        times = torch.where(improved[:, None], cand_t[rows, arg], times)
+        hit = torch.where(improved, terms["is_collision"][rows, arg], hit)
+        history.append(torch.where(improved, best, history[-1]))
+    return free, times, torch.stack(history), hit
+
+
 EXTREMA_OPTIMIZATION = 0   # PolynomialOptimization::computeMaximumOfMagnitude (ref LIN.i:470-503)
 EXTREMA_TRAJECTORY = 1     # Trajectory::computeMinMaxMagnitude (ref src/trajectory.cpp:181-217)
 EXTREMA_KEEP_SMALL_COEFFICIENTS = 16   # OR into mode: do not truncate coefficients below 2.2e-16
@@ -593,6 +742,22 @@ def coeffs_from_constraints_host(mask, fixed_values, free_values, times, N=10):
                                                            _hptr(free_values), _hptr(times), _hptr(coeffs)),
                "minsnap_coeffs_from_constraints_host")
     return coeffs
+
+
+def derivative_gradient_host(mask, fixed_values, free_values, times, N=10, derivative=SNAP):
+    """numpy variant of derivative_gradient(): dict(Jd, gradient, diag, coeffs)."""
+    mask = np.ascontiguousarray(mask, np.uint8)
+    K = mask.shape[0] - 1
+    fixed_values, free_values, times = _np(fixed_values, np.float64), _np(free_values, np.float64), _np(times, np.float64)
+    B, _, D = fixed_values.shape
+    _, n_free = mask_counts(mask)
+    out = dict(Jd=np.empty((B,), np.float64), gradient=np.empty((B, n_free, D), np.float64),
+               diag=np.empty((B, n_free), np.float64), coeffs=np.empty((B, K, D, N), np.float64))
+    capi.check(_lib().minsnap_derivative_gradient_host(B, K, D, N, derivative, _hptr(mask), _hptr(fixed_values),
+                                                       _hptr(free_values), _hptr(times), _hptr(out["coeffs"]),
+                                                       _hptr(out["Jd"]), _hptr(out["gradient"]), _hptr(out["diag"])),
+               "minsnap_derivative_gradient_host")
+    return out
 
 
 def cost_host(coeffs, times, derivative=SNAP):

@@ -578,6 +578,16 @@ int minsnap_optimize_segment_times(long B, int K, int D, int N, int derivative, 
 }
 
 // SURVEY 8(f)3: collision cost and its gradient against a dense distance grid (ref NL.i:1523-1709)
+static int collision_args_check(long B, int K, int D, int N, const int32_t* h_dims, const double* h_origin,
+                                double resolution, const double* h_min_bound, const double* h_max_bound, double dt,
+                                double map_resolution, double epsilon) {
+  if (B < 0 || K < 1 || !h_dims || !h_origin || !h_min_bound || !h_max_bound || !(resolution > 0.0) || !(dt > 0.0) ||
+      !(map_resolution > 0.0) || !(epsilon > 0.0) || h_dims[0] < 1 || h_dims[1] < 1 || h_dims[2] < 1)
+    return MINSNAP_ERR_ARG;
+  if (D != 3 || N != 10) return MINSNAP_ERR_UNSUPPORTED;
+  return MINSNAP_OK;
+}
+
 static int collision_call(long B, int K, int D, int N, const double* d_coeffs, const double* d_times,
                           const double* d_sdf, const int32_t* h_dims, const double* h_origin, double resolution,
                           double oob_value, const double* h_min_bound, const double* h_max_bound,
@@ -585,10 +595,9 @@ static int collision_call(long B, int K, int D, int N, const double* d_coeffs, c
                           double robot_radius, double coll_pot_multiplier, bool want_gradient,
                           const int32_t* d_col_of_row, int n_fixed, int n_free, double* d_cost, double* d_grad_free,
                           int32_t* d_is_collision, int32_t* d_charged, minsnap_stream_t stream) {
-  if (B < 0 || K < 1 || !h_dims || !h_origin || !h_min_bound || !h_max_bound || !(resolution > 0.0) || !(dt > 0.0) ||
-      !(map_resolution > 0.0) || !(epsilon > 0.0) || h_dims[0] < 1 || h_dims[1] < 1 || h_dims[2] < 1)
-    return MINSNAP_ERR_ARG;
-  if (D != 3 || N != 10) return MINSNAP_ERR_UNSUPPORTED;
+  const int rc = collision_args_check(B, K, D, N, h_dims, h_origin, resolution, h_min_bound, h_max_bound, dt,
+                                      map_resolution, epsilon);
+  if (rc != MINSNAP_OK) return rc;
   if (want_gradient) {
     if (n_free < 0 || n_fixed < 0) return MINSNAP_ERR_ARG;
     if (!d_col_of_row && n_free != (K - 1) * (N / 2 - 1)) return MINSNAP_ERR_ARG;   // the standard mask's count
@@ -638,6 +647,219 @@ int minsnap_collision_gradient(long B, int K, int D, int N, const double* d_coef
                         h_max_bound, use_continuous_distance, dt, map_resolution, epsilon, robot_radius,
                         coll_pot_multiplier, true, d_col_of_row, n_fixed, n_free, d_cost, d_grad_free, d_is_collision,
                         d_charged, stream);
+}
+
+// ---------------------------------------------------------------------------------------
+// The free derivatives (and segment times) against J = w_d J_d + w_c J_c + w_t sum(T)
+// (ref getCostAndGradientDerivative NL.i:1452-1521, getCostAndGradientCollision NL.i:1523-1709,
+//  getCostAndGradientTime NL.i:2155-2243)
+// ---------------------------------------------------------------------------------------
+namespace {
+
+// The distance grid and the walk's parameters of minsnap_collision_cost, carried as one value.
+struct CollisionMap {
+  const double* sdf;
+  const int32_t* dims;
+  const double* origin;
+  double resolution, oob_value;
+  const double* min_bound;
+  const double* max_bound;
+  int use_continuous_distance;
+  double dt, map_resolution, epsilon, robot_radius, coll_pot_multiplier;
+
+  int check(long B, int K, int D, int N) const {
+    return collision_args_check(B, K, D, N, dims, origin, resolution, min_bound, max_bound, dt, map_resolution,
+                                epsilon);
+  }
+  int cost(long B, int K, const double* coeffs, const double* times, double* out, int32_t* hit,
+           cudaStream_t st) const {
+    return minsnap_collision_cost(B, K, 3, 10, coeffs, times, sdf, dims, origin, resolution, oob_value, min_bound,
+                                  max_bound, use_continuous_distance, dt, map_resolution, epsilon, robot_radius,
+                                  coll_pot_multiplier, out, hit, nullptr, st);
+  }
+  int gradient(long B, int K, const double* coeffs, const double* times, const int32_t* col_of_row, int n_fixed,
+               int n_free, double* out, double* grad, cudaStream_t st) const {
+    return minsnap_collision_gradient(B, K, 3, 10, coeffs, times, sdf, dims, origin, resolution, oob_value, min_bound,
+                                      max_bound, use_continuous_distance, dt, map_resolution, epsilon, robot_radius,
+                                      coll_pot_multiplier, col_of_row, n_fixed, n_free, out, grad, nullptr, nullptr,
+                                      st);
+  }
+};
+
+minsnap::GeneralSolveArgs recovery_args(long B, int K, int D, int N, int derivative, int n_fixed, int n_free,
+                                        const int32_t* d_col_of_row, const double* d_fixed_values,
+                                        const double* d_free_values, const double* d_times) {
+  minsnap::GeneralSolveArgs a;
+  a.B = B; a.K = K; a.D = D; a.N = N; a.derivative = derivative; a.n_fixed = n_fixed; a.n_free = n_free;
+  a.d_col_of_row = d_col_of_row; a.d_fixed_values = d_fixed_values; a.d_free_in = d_free_values;
+  a.d_times = d_times; a.d_coeffs = nullptr; a.d_free_out = nullptr; a.d_cost = nullptr; a.d_status = nullptr;
+  return a;
+}
+
+// minsnap_free_objective on the device, the index map already built: recovery of the B*S candidates (fixed values
+// shared by the S candidates of a trajectory), the collision walk, the combine kernel.  Scratch: coeffs
+// [B*S][K][D][N], cost and jc [B*S].
+int free_objective_device(long B, int S, int K, int D, int N, int derivative, int n_fixed, int n_free,
+                          const int32_t* d_col_of_row, const double* d_fixed_values, const double* d_free_values,
+                          const double* d_times, double w_d, double w_c, double w_t, const CollisionMap& map,
+                          double* d_objective, double* d_Jd, double* d_jc, int32_t* d_is_collision, double* coeffs,
+                          double* cost, cudaStream_t st) {
+  const long n = B * S;
+  minsnap::GeneralSolveArgs a =
+      recovery_args(n, K, D, N, derivative, n_fixed, n_free, d_col_of_row, d_fixed_values, d_free_values, d_times);
+  a.fixed_div = S;
+  a.d_coeffs = coeffs;
+  a.d_cost = cost;
+  CU(minsnap::launch_coeffs_from_constraints(a, st));
+  const int rc = map.cost(n, K, coeffs, d_times, d_jc, d_is_collision, st);
+  if (rc != MINSNAP_OK) return rc;
+  CU(minsnap::launch_free_combine(n, K, cost, d_jc, d_times, w_d, w_c, w_t, d_objective, d_Jd, st));
+  return MINSNAP_OK;
+}
+
+}  // namespace
+
+int minsnap_derivative_gradient(long B, int K, int D, int N, int derivative, const uint8_t* h_fixed_mask,
+                                const double* d_fixed_values, const double* d_free_values, const double* d_times,
+                                double* d_coeffs, double* d_cost_Jd, double* d_grad_free, double* d_diag_free,
+                                void* d_workspace, size_t workspace_bytes, minsnap_stream_t stream) {
+  if (!shape_ok(B, K, D, N, derivative) || !h_fixed_mask) return MINSNAP_ERR_ARG;
+  if (!d_workspace || workspace_bytes < SolveWorkspace::bytes(N, K)) return MINSNAP_ERR_WORKSPACE;
+  int n_fixed, n_free;
+  count_mask(h_fixed_mask, N, K, &n_fixed, &n_free);
+  if (B == 0) return MINSNAP_OK;
+  if (!d_times || !d_cost_Jd || (n_fixed > 0 && !d_fixed_values) || (n_free > 0 && (!d_free_values || !d_grad_free)))
+    return MINSNAP_ERR_ARG;
+  cudaStream_t st = as_stream(stream);
+  SolveWorkspace ws(d_workspace, N, K);
+  CU(minsnap::launch_reorder_host_mask(N, K, h_fixed_mask, ws.mask, ws.col_of_row, ws.counts, st));
+  minsnap::GeneralSolveArgs a =
+      recovery_args(B, K, D, N, derivative, n_fixed, n_free, ws.col_of_row, d_fixed_values, d_free_values, d_times);
+  a.d_coeffs = d_coeffs; a.d_cost = d_cost_Jd; a.d_grad_free = d_grad_free; a.d_diag_free = d_diag_free;
+  CU(minsnap::launch_derivative_gradient(a, st));
+  return MINSNAP_OK;
+}
+
+int minsnap_free_objective(long B, int S, int K, int D, int N, int derivative, const uint8_t* h_fixed_mask,
+                           const double* d_fixed_values, const double* d_free_values, const double* d_times, double w_d,
+                           double w_c, double w_t, const double* d_sdf, const int32_t* h_dims, const double* h_origin,
+                           double resolution, double oob_value, const double* h_min_bound, const double* h_max_bound,
+                           int use_continuous_distance, double dt, double map_resolution, double epsilon,
+                           double robot_radius, double coll_pot_multiplier, double* d_objective, double* d_Jd,
+                           double* d_Jc, int32_t* d_is_collision, minsnap_stream_t stream) {
+  if (!shape_ok(B, K, D, N, derivative) || S < 1 || !h_fixed_mask) return MINSNAP_ERR_ARG;
+  const CollisionMap map{d_sdf, h_dims, h_origin, resolution, oob_value, h_min_bound, h_max_bound,
+                         use_continuous_distance, dt, map_resolution, epsilon, robot_radius, coll_pot_multiplier};
+  int rc = map.check(B, K, D, N);
+  if (rc != MINSNAP_OK) return rc;
+  int n_fixed, n_free;
+  count_mask(h_fixed_mask, N, K, &n_fixed, &n_free);
+  if (B == 0) return MINSNAP_OK;
+  if (!d_times || !d_sdf || !d_objective || (n_fixed > 0 && !d_fixed_values) || (n_free > 0 && !d_free_values))
+    return MINSNAP_ERR_ARG;
+  cudaStream_t st = as_stream(stream);
+  const size_t n = (size_t)B * S;
+  const size_t ws_head = align_up(SolveWorkspace::bytes(N, K), 256);
+  char* ws = nullptr;
+  retain_pool_memory();
+  CU(cudaMallocAsync(reinterpret_cast<void**>(&ws), ws_head + sizeof(double) * n * ((size_t)K * D * N + 2), st));
+  SolveWorkspace sw(ws, N, K);
+  double* coeffs = reinterpret_cast<double*>(ws + ws_head);
+  double* cost = coeffs + n * K * D * N;
+  double* jc = cost + n;
+  const cudaError_t e = minsnap::launch_reorder_host_mask(N, K, h_fixed_mask, sw.mask, sw.col_of_row, sw.counts, st);
+  if (e != cudaSuccess) rc = cuda_fail(e, "launch_reorder_host_mask");
+  if (rc == MINSNAP_OK)
+    rc = free_objective_device(B, S, K, D, N, derivative, n_fixed, n_free, sw.col_of_row, d_fixed_values,
+                               d_free_values, d_times, w_d, w_c, w_t, map, d_objective, d_Jd, jc, d_is_collision,
+                               coeffs, cost, st);
+  if (rc == MINSNAP_OK && d_Jc && cudaMemcpyAsync(d_Jc, jc, sizeof(double) * n, cudaMemcpyDeviceToDevice, st) != cudaSuccess)
+    rc = MINSNAP_ERR_CUDA;
+  cudaFreeAsync(ws, st);
+  return rc;
+}
+
+// A batched descent on the free derivatives (and optionally the segment times) that never leaves the device: every
+// iteration is launches on `stream` only (recovery with the gradient of J_d, collision gradient, [time gradient,
+// time ladder,] candidate ladder, recovery + walk + combine of the candidates, select); the workspace is one
+// stream-ordered allocation and the mask reaches the device by value, so the call can be captured into a CUDA graph.
+int minsnap_optimize_free_constraints(long B, int K, int D, int N, int derivative, const uint8_t* h_fixed_mask,
+                                      const double* d_fixed_values, double* d_free_values, double* d_times,
+                                      int optimize_times, double w_d, double w_c, double w_t, const double* d_sdf,
+                                      const int32_t* h_dims, const double* h_origin, double resolution,
+                                      double oob_value, const double* h_min_bound, const double* h_max_bound,
+                                      int use_continuous_distance, double dt, double map_resolution, double epsilon,
+                                      double robot_radius, double coll_pot_multiplier, int iterations, int n_steps,
+                                      double max_relative_step, double min_time, double gradient_increment,
+                                      double* d_history, int32_t* d_is_collision, minsnap_stream_t stream) {
+  if (!shape_ok(B, K, D, N, derivative) || !h_fixed_mask || iterations < 0 || n_steps < 1 || !(w_d > 0.0) ||
+      !(max_relative_step > 0.0) || !(min_time > 0.0) || !(gradient_increment > 0.0))
+    return MINSNAP_ERR_ARG;
+  const CollisionMap map{d_sdf, h_dims, h_origin, resolution, oob_value, h_min_bound, h_max_bound,
+                         use_continuous_distance, dt, map_resolution, epsilon, robot_radius, coll_pot_multiplier};
+  int rc = map.check(B, K, D, N);
+  if (rc != MINSNAP_OK) return rc;
+  int n_fixed, n_free;
+  count_mask(h_fixed_mask, N, K, &n_fixed, &n_free);
+  if (B == 0) return MINSNAP_OK;
+  if (!d_times || !d_sdf || (n_fixed > 0 && !d_fixed_values) || (n_free > 0 && !d_free_values)) return MINSNAP_ERR_ARG;
+  cudaStream_t st = as_stream(stream);
+  const size_t nb = (size_t)B, S = (size_t)n_steps, nfd = (size_t)n_free * D, nc = (size_t)K * D * N;
+  const size_t ws_head = align_up(SolveWorkspace::bytes(N, K), 256);
+  const size_t n_doubles = nb * (nc + 2 * nfd + n_free + K + 3) + nb * S * (nfd + K + nc + 3);
+  char* ws = nullptr;
+  retain_pool_memory();
+  CU(cudaMallocAsync(reinterpret_cast<void**>(&ws), ws_head + sizeof(double) * n_doubles + sizeof(int32_t) * nb * (S + 1), st));
+  SolveWorkspace sw(ws, N, K);
+  double* coeffs = reinterpret_cast<double*>(ws + ws_head);   // the incumbent's
+  double* grad_d = coeffs + nb * nc;
+  double* grad_c = grad_d + nb * nfd;
+  double* diag = grad_c + nb * nfd;
+  double* grad_t = diag + nb * n_free;
+  double* jd = grad_t + nb * K;
+  double* jc = jd + nb;
+  double* incumbent = jc + nb;
+  double* cand_free = incumbent + nb;
+  double* cand_times = cand_free + nb * S * nfd;
+  double* cand_coeffs = cand_times + nb * S * K;
+  double* cand_cost = cand_coeffs + nb * S * nc;
+  double* cand_jc = cand_cost + nb * S;
+  double* cand_obj = cand_jc + nb * S;
+  int32_t* cand_hit = reinterpret_cast<int32_t*>(cand_obj + nb * S);
+  int32_t* hit = d_is_collision ? d_is_collision : cand_hit + nb * S;
+  cudaError_t e = minsnap::launch_reorder_host_mask(N, K, h_fixed_mask, sw.mask, sw.col_of_row, sw.counts, st);
+  if (e != cudaSuccess) rc = cuda_fail(e, "launch_reorder_host_mask");
+  // the incumbent objective at the initial state: the candidate pipeline with one candidate per trajectory
+  if (rc == MINSNAP_OK)
+    rc = free_objective_device(B, 1, K, D, N, derivative, n_fixed, n_free, sw.col_of_row, d_fixed_values, d_free_values,
+                               d_times, w_d, w_c, w_t, map, incumbent, nullptr, cand_jc, hit, cand_coeffs, cand_cost, st);
+  if (rc == MINSNAP_OK && d_history)
+    if (cudaMemcpyAsync(d_history, incumbent, sizeof(double) * nb, cudaMemcpyDeviceToDevice, st) != cudaSuccess) rc = MINSNAP_ERR_CUDA;
+  for (int it = 0; it < iterations && rc == MINSNAP_OK; ++it) {
+    minsnap::GeneralSolveArgs a =
+        recovery_args(B, K, D, N, derivative, n_fixed, n_free, sw.col_of_row, d_fixed_values, d_free_values, d_times);
+    a.d_coeffs = coeffs; a.d_cost = jd; a.d_grad_free = grad_d; a.d_diag_free = diag;
+    e = minsnap::launch_derivative_gradient(a, st);
+    if (e == cudaSuccess) rc = map.gradient(B, K, coeffs, d_times, sw.col_of_row, n_fixed, n_free, jc, grad_c, st);
+    if (e == cudaSuccess && rc == MINSNAP_OK && optimize_times) {
+      rc = minsnap_time_gradient(B, K, D, N, derivative, coeffs, d_times, gradient_increment, w_d, w_t, grad_t, nullptr, st);
+      if (rc == MINSNAP_OK)
+        e = minsnap::launch_time_candidates(B, n_steps, K, d_times, grad_t, 0.0, max_relative_step, min_time, cand_times, st);
+    }
+    if (e == cudaSuccess && rc == MINSNAP_OK)
+      e = minsnap::launch_free_candidates(B, n_steps, n_free, D, K, d_free_values, grad_d, grad_c, diag, w_d, w_c, d_times,
+                                          cand_free, optimize_times ? nullptr : cand_times, st);
+    if (e == cudaSuccess && rc == MINSNAP_OK)
+      rc = free_objective_device(B, n_steps, K, D, N, derivative, n_fixed, n_free, sw.col_of_row, d_fixed_values,
+                                 cand_free, cand_times, w_d, w_c, w_t, map, cand_obj, nullptr, cand_jc, cand_hit,
+                                 cand_coeffs, cand_cost, st);
+    if (e == cudaSuccess && rc == MINSNAP_OK)
+      e = minsnap::launch_free_select(B, n_steps, (int)nfd, K, cand_obj, cand_free, cand_times, cand_hit, d_free_values,
+                                      d_times, incumbent, hit, d_history ? d_history + (size_t)(it + 1) * nb : nullptr, st);
+    if (rc == MINSNAP_OK && e != cudaSuccess) rc = cuda_fail(e, "free-constraint descent");
+  }
+  cudaFreeAsync(ws, st);
+  return rc;
 }
 
 // ---------------------------------------------------------------------------------------
@@ -715,6 +937,34 @@ int minsnap_coeffs_from_constraints_host(long B, int K, int D, int N, const uint
     return minsnap_coeffs_from_constraints(B, K, D, N, h_fixed_mask, hc.dev<double>(i_fixed), hc.dev<double>(i_free),
                                            hc.dev<double>(i_times), hc.dev<double>(o_coeffs), hc.dev<char>(t_ws),
                                            SolveWorkspace::bytes(N, K), st);
+  });
+}
+
+int minsnap_derivative_gradient_host(long B, int K, int D, int N, int derivative, const uint8_t* h_fixed_mask,
+                                     const double* h_fixed_values, const double* h_free_values, const double* h_times,
+                                     double* h_coeffs, double* h_cost_Jd, double* h_grad_free, double* h_diag_free) {
+  if (!shape_ok(B, K, D, N, derivative) || !h_fixed_mask) return MINSNAP_ERR_ARG;
+  int n_fixed, n_free;
+  count_mask(h_fixed_mask, N, K, &n_fixed, &n_free);
+  if (B == 0) return MINSNAP_OK;
+  if (!h_times || !h_cost_Jd || (n_fixed > 0 && !h_fixed_values) || (n_free > 0 && (!h_free_values || !h_grad_free)))
+    return MINSNAP_ERR_ARG;
+  HostCall hc;
+  const size_t nb = (size_t)B;
+  const int i_fixed = hc.in(h_fixed_values, sizeof(double) * nb * n_fixed * D);
+  const int i_free = hc.in(h_free_values, sizeof(double) * nb * n_free * D);
+  const int i_times = hc.in(h_times, sizeof(double) * nb * K);
+  const int o_coeffs = hc.out(h_coeffs, h_coeffs ? sizeof(double) * nb * K * D * N : 0);
+  const int o_cost = hc.out(h_cost_Jd, sizeof(double) * nb);
+  const int o_grad = hc.out(h_grad_free, sizeof(double) * nb * n_free * D);
+  const int o_diag = hc.out(h_diag_free, h_diag_free ? sizeof(double) * nb * n_free : 0);
+  const int t_ws = hc.scratch(SolveWorkspace::bytes(N, K));
+  return hc.run([&](cudaStream_t st) {
+    return minsnap_derivative_gradient(B, K, D, N, derivative, h_fixed_mask, hc.dev<double>(i_fixed),
+                                       hc.dev<double>(i_free), hc.dev<double>(i_times),
+                                       hc.dev_if<double>(o_coeffs, h_coeffs), hc.dev<double>(o_cost),
+                                       hc.dev<double>(o_grad), hc.dev_if<double>(o_diag, h_diag_free),
+                                       hc.dev<char>(t_ws), SolveWorkspace::bytes(N, K), st);
   });
 }
 

@@ -212,6 +212,9 @@ struct GeneralKernelParams {
   double* free_out;
   double* cost;
   int32_t* status;
+  // kGrad only (appended so that the other instantiations see the same parameter offsets)
+  double* grad_free;  // [B][n_free][D]: dJ_d/dd_p = 2 (R_pf d_f + R_pp d_p)
+  double* diag_free;  // [B][n_free]: diag(R_pp), optional
 };
 
 // d value of end-point row r of segment seg in dimension dim.
@@ -221,8 +224,9 @@ __device__ inline double dvalue(const int32_t* col, const double* df, const doub
   return c < n_fixed ? df[c * D + dim] : dp[(c - n_fixed) * D + dim];
 }
 
-// Coefficient recovery (a13) and optional cost (a16) for one trajectory held in shared memory.
-template <int N>
+// Coefficient recovery (a13) and optional cost (a16) for one trajectory held in shared memory.  kGrad adds the
+// gradient of J_d = d^T R d in the free derivatives and diag(R_pp), and writes J_d (not 0.5 J_d) to p.cost.
+template <int N, bool kGrad>
 __device__ inline void recover_coefficients(const GeneralKernelParams& p, long b, int lane, const double* H1s,
                                             const double* A1s, const int32_t* col, const double* tpow,
                                             const double* df, const double* dp, int& nonfinite) {
@@ -258,11 +262,39 @@ __device__ inline void recover_coefficients(const GeneralKernelParams& p, long b
   }
   if (p.cost) {
     cost_acc = warp_sum(cost_acc);
-    if (lane == 0) p.cost[b] = 0.5 * cost_acc;
+    if (lane == 0) p.cost[b] = kGrad ? cost_acc : 0.5 * cost_acc;
+  }
+  if (kGrad) {
+    // Free column c is the constraint (vertex v, derivative k).  Two rows map to it: row h+k of segment v-1 (its
+    // end) and row k of segment v (its start), so (R d)_c = (H_{v-1} d_{v-1})_{h+k} + (H_v d_v)_k and
+    // R_pp[c][c] = H_{v-1}[h+k][h+k] + H_v[k][k].  One lane owns each (v, k, dim) and adds the two rows in that
+    // order: every output has one writer and a fixed summation order, so the result is bitwise reproducible.
+    const int n_vk = (p.K + 1) * h;
+    for (int t = lane; t < n_vk * p.D; t += kWarp) {
+      const int dim = t % p.D;
+      const int v = t / (p.D * h), k = (t / p.D) % h;
+      const int c = (v < p.K ? col[v * N + k] : col[(v - 1) * N + h + k]) - p.n_fixed;
+      if (c < 0) continue;
+      double g = 0.0, diag = 0.0;
+#pragma unroll
+      for (int side = 0; side < 2; ++side) {   // 0: end of segment v-1, 1: start of segment v
+        const int seg = v - 1 + side, n = side ? k : h + k;
+        if (seg < 0 || seg >= p.K) continue;
+        const double* tp = tpow + seg * PW + (N - 1) + 1 - 2 * p.delta;
+        double row = 0.0;
+#pragma unroll
+        for (int s = 0; s < N; ++s)
+          row += H1s[n * N + s] * tp[k + (s % h)] * dvalue(col, df, dp, p.n_fixed, p.D, seg * N + s, dim);
+        g += row;
+        diag += H1s[n * N + n] * tp[2 * k];
+      }
+      p.grad_free[(b * p.n_free + c) * p.D + dim] = 2.0 * g;
+      if (p.diag_free && dim == 0) p.diag_free[b * p.n_free + c] = diag;
+    }
   }
 }
 
-template <int N, bool kSolve>
+template <int N, bool kSolve, bool kGrad = false>
 __global__ void __launch_bounds__(256) solve_general_kernel(GeneralKernelParams p) {
   constexpr int h = N / 2;
   constexpr int PW = 2 * N - 1;
@@ -395,7 +427,7 @@ __global__ void __launch_bounds__(256) solve_general_kernel(GeneralKernelParams 
 
     // ---- a13 (+a16): coefficients, cost ---------------------------------------------------
     int nonfinite = 0;
-    recover_coefficients<N>(p, b, lane, H1s, A1s, col, tpow, df, rhs, nonfinite);
+    recover_coefficients<N, kGrad>(p, b, lane, H1s, A1s, col, tpow, df, rhs, nonfinite);
     if (nonfinite) status |= 4;
     status = __reduce_or_sync(0xffffffffu, status);
     if (p.status && lane == 0) p.status[b] = status;
@@ -403,14 +435,14 @@ __global__ void __launch_bounds__(256) solve_general_kernel(GeneralKernelParams 
   }
 }
 
-template <int N, bool kSolve>
+template <int N, bool kSolve, bool kGrad = false>
 static cudaError_t launch_general_n(const GeneralSolveArgs& a, cudaStream_t stream) {
   if (a.B == 0) return cudaSuccess;
   int warps = 8;
   while (warps > 1 && GeneralLayout<N>::cta_bytes(warps, a.K, a.D, a.n_fixed, a.n_free) > 100 * 1024) warps >>= 1;
   size_t smem = GeneralLayout<N>::cta_bytes(warps, a.K, a.D, a.n_fixed, a.n_free);
   if (smem > kMaxDynamicSmem) return cudaErrorInvalidConfiguration;
-  auto kernel = solve_general_kernel<N, kSolve>;
+  auto kernel = solve_general_kernel<N, kSolve, kGrad>;
   cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   if (e != cudaSuccess) return e;
   GeneralKernelParams p;
@@ -420,6 +452,7 @@ static cudaError_t launch_general_n(const GeneralSolveArgs& a, cudaStream_t stre
   p.col_of_row = a.d_col_of_row; p.fixed_values = a.d_fixed_values; p.free_in = a.d_free_in;
   p.times = a.d_times; p.coeffs = a.d_coeffs; p.free_out = a.d_free_out; p.cost = a.d_cost;
   p.status = a.d_status;
+  p.grad_free = a.d_grad_free; p.diag_free = a.d_diag_free;
   long grid = (a.B + warps - 1) / warps;
   const long max_grid = sm_count() * 32;
   if (grid > max_grid) grid = max_grid;
@@ -435,6 +468,31 @@ cudaError_t launch_solve_general(const GeneralSolveArgs& a, cudaStream_t stream)
 cudaError_t launch_coeffs_from_constraints(const GeneralSolveArgs& a, cudaStream_t stream) {
   MINSNAP_DISPATCH_N(a.N, return (launch_general_n<kN, false>(a, stream)));
   return cudaSuccess;
+}
+
+cudaError_t launch_derivative_gradient(const GeneralSolveArgs& a, cudaStream_t stream) {
+  if (!a.d_cost || (a.n_free > 0 && !a.d_grad_free)) return cudaErrorInvalidValue;
+  MINSNAP_DISPATCH_N(a.N, return (launch_general_n<kN, false, true>(a, stream)));
+  return cudaSuccess;
+}
+
+// The mask travels by value in the kernel's parameters, so that a caller can capture the whole call into a CUDA
+// graph: a copy from pageable host memory cannot be captured.
+__global__ void unpack_mask_kernel(MaskBits bits, int n, uint8_t* __restrict__ mask) {
+  for (int i = threadIdx.x; i < n; i += blockDim.x) mask[i] = (bits.words[i >> 5] >> (i & 31)) & 1u;
+}
+
+cudaError_t launch_reorder_host_mask(int N, int K, const uint8_t* h_mask, uint8_t* d_mask, int32_t* d_col_of_row,
+                                     int32_t* d_counts, cudaStream_t stream) {
+  const int n = (K + 1) * (N / 2);
+  if (n > 32 * MaskBits::kWords) return cudaErrorInvalidConfiguration;
+  MaskBits bits = {};
+  for (int i = 0; i < n; ++i)
+    if (h_mask[i]) bits.words[i >> 5] |= 1u << (i & 31);
+  unpack_mask_kernel<<<1, 256, 0, stream>>>(bits, n, d_mask);
+  cudaError_t e = cudaGetLastError();
+  if (e != cudaSuccess) return e;
+  return launch_reorder(N, K, 1, d_mask, d_col_of_row, d_counts, stream);
 }
 
 // =========================================================================================
@@ -659,6 +717,119 @@ cudaError_t launch_time_select(long B, int S, int K, const double* d_cand, const
   if (B == 0) return cudaSuccess;
   time_select_kernel<<<(unsigned)((B + 127) / 128), 128, 0, stream>>>(B, S, K, d_cand, d_cost, time_penalty, d_times,
                                                                      d_incumbent, d_history_row);
+  return cudaGetLastError();
+}
+
+// =========================================================================================
+// The glue of the batched descent on the free derivatives (and optionally the segment times) against
+// J = w_d J_d + w_c J_c + w_t sum(T), on the device.  See minsnap_optimize_free_constraints.
+// =========================================================================================
+// cand_free[b][s][j] = d_p[b][j] - 2^-s (w_d g_d[b][j] + w_c g_c[b][j]) / (2 w_d diag[b][j / D]): a Jacobi-scaled
+// step, in the units of each free derivative.  Every operation is rounded on its own (no contraction), the sequence
+// an elementwise torch version of the step performs.  cand_times (optional) [b][s] = times[b]: the times stay.
+__global__ void __launch_bounds__(256) free_candidates_kernel(long B, int S, int n_fd, int D, int K,
+                                                              const double* __restrict__ free_values,
+                                                              const double* __restrict__ grad_d,
+                                                              const double* __restrict__ grad_c,
+                                                              const double* __restrict__ diag, double w_d, double w_c,
+                                                              const double* __restrict__ times,
+                                                              double* __restrict__ cand_free,
+                                                              double* __restrict__ cand_times) {
+  const long n_free_total = B * S * n_fd;
+  const long total = n_free_total + (cand_times ? B * S * K : 0);
+  for (long idx = (long)blockIdx.x * blockDim.x + threadIdx.x; idx < total; idx += (long)gridDim.x * blockDim.x) {
+    if (idx < n_free_total) {
+      const long bs = idx / n_fd;
+      const int j = (int)(idx - bs * n_fd);
+      const long b = bs / S;
+      const int s = (int)(bs - b * S);
+      const long g = b * n_fd + j;
+      const double num = __dadd_rn(__dmul_rn(w_d, grad_d[g]), __dmul_rn(w_c, grad_c[g]));
+      const double step = __ddiv_rn(num, __dmul_rn(2.0 * w_d, diag[b * (n_fd / D) + j / D]));
+      cand_free[idx] = __dsub_rn(free_values[g], __dmul_rn(ldexp(1.0, -s), step));
+    } else {
+      const long i = idx - n_free_total;
+      const long bs = i / K;
+      cand_times[i] = times[(bs / S) * K + (i - bs * K)];
+    }
+  }
+}
+
+// objective[i] = w_d J_d + w_c J_c + w_t sum_k times[i][k], J_d = 2 computeCost (the sum left to right, as
+// computeTotalTrajectoryTime).  Jd (optional) receives J_d.
+__global__ void __launch_bounds__(256) free_combine_kernel(long n, int K, const double* __restrict__ cost,
+                                                           const double* __restrict__ jc,
+                                                           const double* __restrict__ times, double w_d, double w_c,
+                                                           double w_t, double* __restrict__ objective,
+                                                           double* __restrict__ jd) {
+  const long i = (long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  double total = 0.0;
+  for (int k = 0; k < K; ++k) total += times[i * K + k];
+  const double j_d = 2.0 * cost[i];
+  objective[i] = w_d * j_d + w_c * jc[i] + w_t * total;
+  if (jd) jd[i] = j_d;
+}
+
+// The first minimum over the finite candidate objectives replaces the incumbent (free values, times, collision
+// flag, objective) only when it is strictly smaller; history_row (optional) receives the incumbent.
+__global__ void __launch_bounds__(128) free_select_kernel(long B, int S, int n_fd, int K,
+                                                          const double* __restrict__ cand_obj,
+                                                          const double* __restrict__ cand_free,
+                                                          const double* __restrict__ cand_times,
+                                                          const int32_t* __restrict__ cand_hit,
+                                                          double* __restrict__ free_values, double* __restrict__ times,
+                                                          double* __restrict__ incumbent, int32_t* __restrict__ hit,
+                                                          double* __restrict__ history_row) {
+  const long b = (long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (b >= B) return;
+  double best = 0.0;
+  int arg = -1;
+  for (int s = 0; s < S; ++s) {
+    const double obj = cand_obj[b * S + s];
+    if (isfinite(obj) && (arg < 0 || obj < best)) { best = obj; arg = s; }
+  }
+  double cur = incumbent[b];
+  if (arg >= 0 && best < cur) {
+    const long c = b * S + arg;
+    for (int j = 0; j < n_fd; ++j) free_values[b * n_fd + j] = cand_free[c * n_fd + j];
+    for (int k = 0; k < K; ++k) times[b * K + k] = cand_times[c * K + k];
+    if (hit) hit[b] = cand_hit[c];
+    cur = best;
+    incumbent[b] = cur;
+  }
+  if (history_row) history_row[b] = cur;
+}
+
+cudaError_t launch_free_candidates(long B, int S, int n_free, int D, int K, const double* d_free, const double* d_grad_d,
+                                   const double* d_grad_c, const double* d_diag, double w_d, double w_c,
+                                   const double* d_times, double* d_cand_free, double* d_cand_times,
+                                   cudaStream_t stream) {
+  const long total = B * S * ((long)n_free * D + (d_cand_times ? K : 0));
+  if (total == 0) return cudaSuccess;
+  long grid = (total + 255) / 256;
+  if (grid > sm_count() * 32) grid = sm_count() * 32;
+  free_candidates_kernel<<<(int)grid, 256, 0, stream>>>(B, S, n_free * D, D, K, d_free, d_grad_d, d_grad_c, d_diag, w_d,
+                                                        w_c, d_times, d_cand_free, d_cand_times);
+  return cudaGetLastError();
+}
+
+cudaError_t launch_free_combine(long n, int K, const double* d_cost, const double* d_jc, const double* d_times,
+                                double w_d, double w_c, double w_t, double* d_objective, double* d_jd,
+                                cudaStream_t stream) {
+  if (n == 0) return cudaSuccess;
+  free_combine_kernel<<<(unsigned)((n + 255) / 256), 256, 0, stream>>>(n, K, d_cost, d_jc, d_times, w_d, w_c, w_t,
+                                                                       d_objective, d_jd);
+  return cudaGetLastError();
+}
+
+cudaError_t launch_free_select(long B, int S, int n_fd, int K, const double* d_cand_obj, const double* d_cand_free,
+                               const double* d_cand_times, const int32_t* d_cand_hit, double* d_free, double* d_times,
+                               double* d_incumbent, int32_t* d_hit, double* d_history_row, cudaStream_t stream) {
+  if (B == 0) return cudaSuccess;
+  free_select_kernel<<<(unsigned)((B + 127) / 128), 128, 0, stream>>>(B, S, n_fd, K, d_cand_obj, d_cand_free,
+                                                                     d_cand_times, d_cand_hit, d_free, d_times,
+                                                                     d_incumbent, d_hit, d_history_row);
   return cudaGetLastError();
 }
 

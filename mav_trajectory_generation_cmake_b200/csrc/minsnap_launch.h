@@ -45,12 +45,26 @@ struct GeneralSolveArgs {
   const double* d_times;        // [B][K]
   double* d_coeffs;             // [B][K][D][N] (optional for cost-only runs)
   double* d_free_out;           // optional
-  double* d_cost;               // optional
+  double* d_cost;               // optional; J_d = d^T R d instead of computeCost in launch_derivative_gradient
   int32_t* d_status;            // optional
+  double* d_grad_free = nullptr;  // [B][n_free][D], launch_derivative_gradient only: dJ_d/dd_p
+  double* d_diag_free = nullptr;  // [B][n_free], launch_derivative_gradient only (optional): diag(R_pp)
 };
 // Returns cudaErrorInvalidConfiguration when one problem does not fit shared memory.
 cudaError_t launch_solve_general(const GeneralSolveArgs& a, cudaStream_t stream);
 cudaError_t launch_coeffs_from_constraints(const GeneralSolveArgs& a, cudaStream_t stream);
+// coefficient recovery plus J_d, its gradient in d_p and diag(R_pp) (d_grad_free and d_cost required)
+cudaError_t launch_derivative_gradient(const GeneralSolveArgs& a, cudaStream_t stream);
+
+// A (K+1) x h mask packed into bits, passed by value to the kernel that unpacks it on the device.
+struct MaskBits {
+  static constexpr int kWords = 512;   // 16,384 constraints, beyond what the general kernel's shared memory takes
+  uint32_t words[kWords];
+};
+// launch_reorder of one HOST mask, without a host-to-device copy (capturable into a CUDA graph); d_mask receives the
+// unpacked mask.  cudaErrorInvalidConfiguration when the mask has more than 32 * MaskBits::kWords entries.
+cudaError_t launch_reorder_host_mask(int N, int K, const uint8_t* h_mask, uint8_t* d_mask, int32_t* d_col_of_row,
+                                     int32_t* d_counts, cudaStream_t stream);
 cudaError_t launch_cost(long B, int K, int D, int N, int derivative, const double* d_coeffs,
                         const double* d_times, double* d_cost, cudaStream_t stream);
 
@@ -67,6 +81,18 @@ cudaError_t launch_time_candidates(long B, int S, int K, const double* d_times, 
                                    cudaStream_t stream);
 cudaError_t launch_time_select(long B, int S, int K, const double* d_cand, const double* d_cost, double time_penalty,
                                double* d_times, double* d_incumbent, double* d_history_row, cudaStream_t stream);
+
+// device-side glue of the batched descent on the free derivatives (minsnap_optimize_free_constraints)
+cudaError_t launch_free_candidates(long B, int S, int n_free, int D, int K, const double* d_free, const double* d_grad_d,
+                                   const double* d_grad_c, const double* d_diag, double w_d, double w_c,
+                                   const double* d_times, double* d_cand_free, double* d_cand_times,
+                                   cudaStream_t stream);
+cudaError_t launch_free_combine(long n, int K, const double* d_cost, const double* d_jc, const double* d_times,
+                                double w_d, double w_c, double w_t, double* d_objective, double* d_jd,
+                                cudaStream_t stream);
+cudaError_t launch_free_select(long B, int S, int n_fd, int K, const double* d_cand_obj, const double* d_cand_free,
+                               const double* d_cand_times, const int32_t* d_cand_hit, double* d_free, double* d_times,
+                               double* d_incumbent, int32_t* d_hit, double* d_history_row, cudaStream_t stream);
 
 // ---- minsnap_standard.cu ---------------------------------------------------------------
 // The kernels behind minsnap_solve_standard; choose_standard_route (minsnap_standard_route.cuh) picks one.
