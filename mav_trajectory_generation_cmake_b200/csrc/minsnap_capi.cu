@@ -445,9 +445,10 @@ int minsnap_sample_at(long B, int K, int D, int N, const double* d_coeffs, const
 int minsnap_evaluate_range(long B, int K, int D, int N, const double* d_coeffs, const double* d_times,
                            double t_start, double t_end, double dt, int derivative, int max_samples,
                            double* d_out, double* d_t_out, int32_t* d_count, minsnap_stream_t stream) {
-  if (B < 0 || K < 1 || D < 1 || !minsnap::supported_n(N) || !(dt > 0.0) || derivative < 0 || max_samples < 0 ||
-      !d_coeffs || !d_times || !d_out)
+  if (B < 0 || K < 1 || D < 1 || !minsnap::supported_n(N) || !(dt > 0.0) || derivative < 0 || max_samples < 0)
     return MINSNAP_ERR_ARG;
+  if (B == 0) return MINSNAP_OK;   // empty batch: nothing to read or write
+  if (!d_coeffs || !d_times || !d_out) return MINSNAP_ERR_ARG;
   CU(minsnap::launch_evaluate_range(B, K, D, N, d_coeffs, d_times, t_start, t_end, dt, derivative, max_samples,
                                     d_out, d_t_out, d_count, as_stream(stream)));
   return MINSNAP_OK;

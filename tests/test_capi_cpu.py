@@ -61,6 +61,17 @@ def test_argument_errors_are_codes_not_crashes(ms):
     assert lib.minsnap_fp64_peak(0, None) == capi.ERR_ARG
 
 
+def test_evaluate_range_empty_batch_is_a_no_op(ms):
+    """B = 0 reads no pointer, like every other batched entry; the shape is still checked."""
+    lib = ms.load()
+    from mav_trajectory_generation_cmake_b200 import capi
+    args = (0.0, 1.0, 0.1, 0, 16, None, None, None, None)
+    assert lib.minsnap_evaluate_range(0, 10, 3, 10, None, None, *args) == capi.OK
+    assert lib.minsnap_evaluate_range(1, 10, 3, 10, None, None, *args) == capi.ERR_ARG
+    assert lib.minsnap_evaluate_range(0, 10, 3, 7, None, None, *args) == capi.ERR_ARG
+    assert lib.minsnap_evaluate_range(-1, 10, 3, 10, None, None, *args) == capi.ERR_ARG
+
+
 def test_random_positions_match_oracle_generator(ms, oracle):
     lo, hi = [-10.0, -20.0, -10.0], [10.0, 20.0, 10.0]
     got = ms.random_positions_host(33, 10, lo, hi, 12345)
