@@ -1,8 +1,15 @@
 """Every launch variant of the sampling, evaluate_range, cost and cost-sweep launchers has a case in
 tests/test_gpu_kernel_variants.py.  The variant of each case comes from that file's restatement of the launcher's
 choice, so a threshold moved in a .cu file (and mirrored there) that leaves some variant without a case fails here,
-on a machine without a GPU."""
+on a machine without a GPU.  The same holds for the collision walk and the gradient instantiation of the general
+kernel in tests/test_gpu_collision_walk.py, whose hand-built and map cases are also checked here to reach the edges
+they are built for."""
+import numpy as np
+
+import test_gpu_collision_walk as W
 import test_gpu_kernel_variants as V
+from oracle import oracle_py
+from test_collision_cost import field
 
 SMS = V.B200_SMS
 
@@ -51,3 +58,99 @@ def test_grid_stride_cases_loop():
     assert V.sweep_variant(V.SWEEP_LOOP_K, V.SWEEP_LOOP_D) == "direct"
     assert V.sweep_loops(V.SWEEP_LOOP_B * V.SWEEP_LOOP_S, V.SWEEP_LOOP_K, V.SWEEP_LOOP_D, SMS)
     assert not V.evaluate_range_loops(64 * SMS, SMS) and not V.cost_loops(128 * SMS, SMS)
+
+
+# ---- the collision walk and the gradient kernel (tests/test_gpu_collision_walk.py) ----------------------------------
+def test_gradient_kernel_warp_steps_have_cases():
+    """Every warps-per-CTA step of the general kernel's gradient instantiation has a case at its first and its last
+    K for both masks, the first refused K has a case, and D = 1 has one past its last step."""
+    steps, refused = W.warp_steps(3, "standard")
+    assert steps == {8: (1, 21), 4: (22, 42), 2: (43, 82), 1: (83, 365)} and refused == 366
+    steps_d1, refused_d1 = W.warp_steps(1, "standard")
+    assert [steps_d1[w][0] for w in (4, 2, 1)] == [25, 49, 96] and refused_d1 == 419
+    for kind in ("standard", "general"):
+        steps, refused = W.warp_steps(3, kind)
+        have = {args[0]: tag for args, tag in W.GRADIENT_CASES if args[1:] == (3, kind)}
+        assert set(steps) == {8, 4, 2, 1}
+        for warps, (first, last) in steps.items():
+            assert have.get(first) == warps and have.get(last) == warps, (kind, warps, first, last)
+        assert (refused, 3, kind) in W.ERROR_CASES
+    for K, D, kind in W.ERROR_CASES:
+        assert W.gradient_variant(K, D, kind) is None and W.gradient_variant(K - 1, D, kind) == 1
+    assert any(args[1] == 1 and args[0] > steps_d1[1][0] and tag == 1 for args, tag in W.GRADIENT_CASES)
+    assert any(args[0] == 1 for args, _ in W.GRADIENT_CASES) and 1 in W.WALK_K_CASES
+
+
+def test_collision_walk_and_gradient_loop_cases_loop():
+    """The batch of every grid-stride case loops on 148 SMs, and the chunks it is compared with do not."""
+    assert W.walk_loops(W.WALK_LOOP_B, SMS) and not W.walk_loops(W.WALK_CHUNK, SMS)
+    looped = set()
+    for K, B, chunk in W.GRADIENT_LOOP_CASES:
+        warps = W.gradient_variant(K, 3, "standard")
+        assert W.general_loops(B, warps, SMS) and not W.general_loops(chunk, warps, SMS)
+        looped.add(warps)
+    assert looped == {8, 1}
+    n, warps = W.FREE_B * W.FREE_S, W.gradient_variant(W.FREE_K, 3, "standard")
+    assert W.general_loops(n, warps, SMS) and W.walk_loops(n, SMS)
+    chunk = W.FREE_CHUNK * W.FREE_S
+    assert not W.general_loops(chunk, warps, SMS) and not W.walk_loops(chunk, SMS)
+
+
+def test_walk_boundary_cases_reach_their_edges():
+    """The hand-built walks do what they are built for, on a Python replay of the walk that agrees with the oracle
+    on the number of charged samples."""
+    g = field("sphere")
+    for name, (rows, row_times, dt, limit, _) in W.BOUNDARY_CASES.items():
+        kw = dict(W.MAP1, dt=dt, map_resolution=limit, use_continuous_distance=True)
+        for c, times in zip(rows, row_times):
+            charged, entry, counts, margin = W.replay_walk(c, times, dt, limit)
+            assert oracle_py.collision_cost(c, times, g, **kw)[2] == len(charged), name
+            assert margin > 1e-6 and max(counts) < 1e5, (name, margin)
+        charged, entry, counts, margin = W.replay_walk(rows[0], row_times[0], dt, limit)
+        times = row_times[0]
+        cost, hit, _ = oracle_py.collision_cost(rows[0], times, g, **kw)
+        assert cost > 0.1 and hit, name                        # the walk crosses the obstacle
+        if name == "lane31":     # on and one ulp below 32 dt: a full chunk, then one with no valid sample; one ulp
+            assert times[0] == W.repeated(dt, 32) and times[1] < times[0] < times[2]     # above: a 33rd sample
+            assert counts == [32, 32, 33, 64]
+        elif name == "short_and_zero":
+            assert counts[1] == 0 and counts[3] == 1 and times[3] < dt
+            assert 0.0 <= entry[1] < dt and entry[2] < 0.0     # the zero-length segment leaves time_sum negative
+        elif name == "many_chunks":
+            assert counts[0] > 60 * 32
+        else:
+            slow = [s for s in charged if s[0] == 1 and s[1] == 0.0]
+            assert len(slow) == 1 and np.linalg.norm(slow[0][4]) < 1e-6 and slow[0][2] > 0.5
+            cost, _, hit = oracle_py.collision_potential(slow[0][3], g, **W.potential_kw(kw))
+            assert hit and cost > 1.0
+
+
+def test_walk_map_cases_reach_their_edges(oracle):
+    """The charged samples of the map cases reach all three branches of cost_potential and cells outside the grid,
+    and in continuous mode a centre whose eight-cell stencil falls off the grid (the discrete fallback)."""
+    g = W.grid2_field()
+    assert g.shape == W.GRID2_DIMS and len(set(W.GRID2_DIMS)) == 3 and len(set(W.GRID2_ORIGIN)) == 3
+    for case in W.MAP_CASES:
+        for continuous in (True, False):
+            coeffs, times, kw = W.map_case(oracle, case, continuous)
+            seen = W.map_edges(coeffs, times, g, kw)
+            assert min(seen["collision"], seen["band"], seen["free"], seen["outside"]) > 0, (case, seen)
+            assert seen["stencil_off"] > 0 or not continuous, (case, seen)
+    mr = {W.walk_kw(dict(resolution=W.GRID2_RES, **kw))["map_resolution"] for kw in W.MAP_CASES.values()}
+    assert min(mr) < W.GRID2_RES < max(mr)
+    assert {kw.get("robot_radius", 0.5) for kw in W.MAP_CASES.values()} >= {0.0}
+    assert {kw["oob_value"] < 0.5 for kw in W.MAP_CASES.values()} == {True, False}
+
+
+def test_walk_chain_cases_reach_the_last_free_vertex(oracle):
+    """At every K > 1 the oracle's gradient is non-zero in the columns of vertex K - 1, the last free one."""
+    g = field(W.CHAIN_FIELD)
+    kw = W.chain_kw()
+    for K in W.WALK_K_CASES:
+        if K == 1:
+            continue
+        coeffs, times = W.chain_case(oracle, K)
+        col, n_fixed, n_free = oracle.reorder(10, K, W.standard_mask(K))
+        last = max(np.abs(oracle_py.collision_cost_gradient(coeffs[b], times[b], col, n_fixed, n_free, sdf=g, **kw)[1]
+                          [-4:]).max() for b in range(len(times)))
+        assert last > 0, K
