@@ -135,6 +135,7 @@ MINSNAP_API int minsnap_cost(long B, int K, int D, int N, int derivative, const 
  * d_end_derivatives [B][2][h-1][D] (start then end vertex, derivatives 1..h-1) or NULL = zeros.
  * d_times NULL => times are computed on the device from (v_max, a_max, magic) exactly as
  * minsnap_estimate_segment_times does and, when d_times_out != NULL, written there.
+ * A shape no kernel takes (MINSNAP_ERR_UNSUPPORTED) writes no output, d_times_out included.
  * The environment variable MINSNAP_STANDARD_ROUTE=tm|pair|pair_long|bcr|chunked|general (read on every call) runs
  * the named kernel instead of the one the shape and batch size select, for tests that compare two kernels:
  * MINSNAP_ERR_UNSUPPORTED when that kernel cannot take the call, MINSNAP_ERR_ARG for any other name. */

@@ -465,6 +465,12 @@ cudaError_t launch_solve_general(const GeneralSolveArgs& a, cudaStream_t stream)
   return cudaSuccess;
 }
 
+cudaError_t general_fits(int N, int K, int D, int n_fixed, int n_free) {
+  MINSNAP_DISPATCH_N(N, return GeneralLayout<kN>::cta_bytes(1, K, D, n_fixed, n_free) <= kMaxDynamicSmem
+                                   ? cudaSuccess : cudaErrorInvalidConfiguration);
+  return cudaSuccess;
+}
+
 cudaError_t launch_coeffs_from_constraints(const GeneralSolveArgs& a, cudaStream_t stream) {
   MINSNAP_DISPATCH_N(a.N, return (launch_general_n<kN, false>(a, stream)));
   return cudaSuccess;

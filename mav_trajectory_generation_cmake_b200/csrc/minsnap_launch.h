@@ -52,6 +52,8 @@ struct GeneralSolveArgs {
 };
 // Returns cudaErrorInvalidConfiguration when one problem does not fit shared memory.
 cudaError_t launch_solve_general(const GeneralSolveArgs& a, cudaStream_t stream);
+// cudaErrorInvalidConfiguration where launch_solve_general would refuse the shape, without launching anything
+cudaError_t general_fits(int N, int K, int D, int n_fixed, int n_free);
 cudaError_t launch_coeffs_from_constraints(const GeneralSolveArgs& a, cudaStream_t stream);
 // coefficient recovery plus J_d, its gradient in d_p and diag(R_pp) (d_grad_free and d_cost required)
 cudaError_t launch_derivative_gradient(const GeneralSolveArgs& a, cudaStream_t stream);

@@ -103,6 +103,10 @@ static cudaError_t run_route(StandardRoute route, const StandardSolveArgs& a, co
   const bool estimate = route == StandardRoute::Chunked || route == StandardRoute::General;
   const bool times_later = (route == StandardRoute::Bcr && p.cost) || route == StandardRoute::PairLong;
   cudaError_t e;
+  // a shape the general kernel refuses is refused before the estimate below writes times_out
+  if (route == StandardRoute::General &&
+      (e = general_fits(a.N, a.K, a.D, a.K + a.N - 1, (a.K - 1) * (a.N / 2 - 1))) != cudaSuccess)
+    return e;
   if (!p.times && !p.times_out && (estimate || times_later)) {
     if ((e = times_scratch.alloc(sizeof(double) * (size_t)a.B * a.K, stream)) != cudaSuccess) return e;
     p.times_out = static_cast<double*>(times_scratch.ptr);

@@ -130,3 +130,46 @@ def oracle_gradient(oracle, pos, times, increment, w_d, w_t):
         bigger[n] = 0.1 if bigger[n] <= 0.1 else bigger[n] + increment
         grad[n] = w_d * (J_d(bigger) - J_d(smaller)) / (2.0 * increment) + w_t
     return grad, J_d(times)
+
+
+def banded_ld_solve(oracle_ld, N, derivative, mask, values, times):
+    """The linear solve of one trajectory in long double, in O(K): R_pp d_p = -R_pf d_f by banded elimination.
+
+    R is assembled from oracle_ld.segment_hessian and the column map of oracle.reorder exactly as the dense oracle
+    assembles it (R[col[i N + r]][col[i N + s]] += H_i[r][s]).  Free columns are ordered by (vertex, derivative), so
+    two free columns that share a segment are at most N - 1 apart: R_pp has half bandwidth N - 1.  The reference's
+    A^-T Q A^-1 is symmetric only to ~1e-14 relative, so both halves of the band are kept (an LDL^T of the lower half
+    would differ from the dense oracle by that asymmetry times the condition number, 1e-10 at K = 64).
+    mask[(K+1)][h], values[(K+1)][h][D], times[K] -> coeffs [K][D][N], d_free [n_free][D], cost (long double)."""
+    mask = np.asarray(mask, bool)
+    K, D = mask.shape[0] - 1, values.shape[-1]
+    col, nf, npf = oracle_ld.reorder(N, K, mask)
+    col = col.reshape(K, N)
+    ld, w = np.longdouble, N - 1
+    d = np.zeros((nf + npf, D), ld)
+    d[:nf] = np.asarray(values, ld)[mask]              # fixed columns in (vertex, derivative) order
+    band = np.zeros((npf + w, 2 * w + 1), ld)          # band[c][w + j] = R_pp[c][c + j]
+    rhs = np.zeros((npf + w, D), ld)                   # -R_pf d_f
+    for i in range(K):
+        H = oracle_ld.segment_hessian(N, derivative, times[i])
+        for r in range(N):
+            cr = col[i, r]
+            if cr < nf:
+                continue
+            for s in range(N):
+                cs = col[i, s]
+                if cs < nf:
+                    rhs[cr - nf] -= H[r, s] * d[cs]
+                else:
+                    band[cr - nf, w + cs - cr] += H[r, s]
+    for c in range(npf):                               # elimination without pivoting, forward substitution
+        for j in range(1, w + 1):
+            f = band[c + j, w - j] / band[c, w]
+            band[c + j, w - j : 2 * w + 1 - j] -= f * band[c, w:]
+            rhs[c + j] -= f * rhs[c]
+    x = np.zeros((npf + w, D), ld)
+    for c in range(npf - 1, -1, -1):
+        x[c] = (rhs[c] - band[c, w + 1 :] @ x[c + 1 : c + w + 1]) / band[c, w]
+    d[nf:] = x[:npf]
+    coeffs = oracle_ld.coeffs_from_constraints(N, K, D, col.ravel(), np.ascontiguousarray(d.T), times)
+    return coeffs, d[nf:].copy(), oracle_ld.compute_cost(N, K, D, derivative, coeffs, times)

@@ -52,23 +52,23 @@ def walk_loops(B, sms=B200_SMS):
     return B > sms * 32 * 4
 
 
-def general_per_warp_doubles(K, D, n_fixed, n_free):
+def general_per_warp_doubles(K, D, n_fixed, n_free, N=N):
     """GeneralLayout<N>::per_warp_doubles, minsnap_general.cu:194-196."""
     return K * (2 * N - 1) + n_free * N + n_free * D + n_fixed * D + N
 
 
-def general_cta_bytes(warps, K, D, n_fixed, n_free):
+def general_cta_bytes(warps, K, D, n_fixed, n_free, N=N):
     """GeneralLayout<N>::cta_bytes, minsnap_general.cu:197-200."""
-    return (2 * N * N + warps * general_per_warp_doubles(K, D, n_fixed, n_free)) * 8 + 4 * N * K
+    return (2 * N * N + warps * general_per_warp_doubles(K, D, n_fixed, n_free, N)) * 8 + 4 * N * K
 
 
-def general_warps(K, D, n_fixed, n_free):
+def general_warps(K, D, n_fixed, n_free, N=N):
     """launch_general_n, minsnap_general.cu:441-444: warps per CTA halved from 8 while the CTA needs more than
     100 KiB, None (cudaErrorInvalidConfiguration, MINSNAP_ERR_UNSUPPORTED) above kMaxDynamicSmem."""
     warps = 8
-    while warps > 1 and general_cta_bytes(warps, K, D, n_fixed, n_free) > 100 * 1024:
+    while warps > 1 and general_cta_bytes(warps, K, D, n_fixed, n_free, N) > 100 * 1024:
         warps >>= 1
-    return warps if general_cta_bytes(warps, K, D, n_fixed, n_free) <= MAX_DYNAMIC_SMEM else None
+    return warps if general_cta_bytes(warps, K, D, n_fixed, n_free, N) <= MAX_DYNAMIC_SMEM else None
 
 
 def general_loops(B, warps, sms=B200_SMS):

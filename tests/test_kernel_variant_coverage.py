@@ -3,11 +3,12 @@ tests/test_gpu_kernel_variants.py.  The variant of each case comes from that fil
 choice, so a threshold moved in a .cu file (and mirrored there) that leaves some variant without a case fails here,
 on a machine without a GPU.  The same holds for the collision walk and the gradient instantiation of the general
 kernel in tests/test_gpu_collision_walk.py, whose hand-built and map cases are also checked here to reach the edges
-they are built for."""
+they are built for, and for the kernels behind minsnap_solve_standard in tests/test_gpu_standard_variants.py."""
 import numpy as np
 
 import test_gpu_collision_walk as W
 import test_gpu_kernel_variants as V
+import test_gpu_standard_variants as S
 from oracle import oracle_py
 from test_collision_cost import field
 
@@ -154,3 +155,68 @@ def test_walk_chain_cases_reach_the_last_free_vertex(oracle):
         last = max(np.abs(oracle_py.collision_cost_gradient(coeffs[b], times[b], col, n_fixed, n_free, sdf=g, **kw)[1]
                           [-4:]).max() for b in range(len(times)))
         assert last > 0, K
+
+
+# ---- minsnap_solve_standard (tests/test_gpu_standard_variants.py) ------------------------------------------------
+def _standard_variants():
+    routes = S.routes_of(S.STD_CASES)
+    return [(c, r, S.variant(c, r)) for c, r in zip(S.STD_CASES, routes)]
+
+
+def test_every_standard_route_variant_has_a_case():
+    """Each case reaches the route it is written for (the route binary), and every variant has a case: the 24 tm
+    instantiations through solve_standard, every tm grid mode for each D, pair (D, kCost) and its grid-stride loop,
+    both pair_long scratch branches, every bcr thread step at D = 3 and a looping bcr case for each D, every chunk
+    length for each D on one and on two ranges, and the general route at N != 10, derivative != 4 and D >= 4."""
+    cases = _standard_variants()
+    for c, r, _ in cases:
+        assert r == (c.forced or r) and r != "unsupported", (c, r)
+    tags = {}
+    for c, r, v in cases:
+        tags.setdefault(r, set()).add(v)
+    assert all(r == "tm" for c, r, _ in cases if c in S.TM_CASES)
+    assert {v[:4] for v in tags["tm"]} == {(D, cost, ex, odd) for D in (1, 2, 3) for cost in (False, True)
+                                           for ex in (False, True) for odd in (False, True)}
+    for inst in {v[:4] for v in tags["tm"]}:     # two time modes for every instantiation
+        assert len({c.times for c, r, v in cases if r == "tm" and v[:4] == inst}) >= 2, inst
+    modes = ("one batch per warp", "two batches, even waves", "two batches, odd waves")
+    assert {(v[0], v[4]) for v in tags["tm"]} == {(D, m) for D in (1, 2, 3) for m in modes}
+    assert any(r == "tm" and v[0] == 1 and v[4] != modes[0] and S.tm_ctas(c.K, 1, False, False) == 3
+               for c, r, v in cases)
+    assert {v[:2] for v in tags["pair"]} == {(D, cost) for D in (1, 2, 3) for cost in (False, True)}
+    assert any(v[2] for v in tags["pair"])
+    assert {v[1:] for v in tags["pair_long"]} >= {(f, t) for f in ("free scratch", "free out")
+                                                  for t in ("given", "times scratch", "est_out")}
+    assert {v[1] for v in tags["bcr"] if v[0] == 3} == {64, 96, 128, 160, 192, 224, 256}
+    assert {v[0] for v in tags["bcr"] if v[3]} == {1, 2, 3} and any(v[4] for v in tags["bcr"])
+    assert {(v[0], v[2]) for v in tags["bcr"]} == {(D, n) for D in (1, 2, 3) for n in (1, 2)}
+    assert {v for v in tags["chunked"]} == {(D, m, n) for D in (1, 2, 3) for m in (4, 6, 8, 10, 12) for n in (1, 2)}
+    general = tags["general"]
+    assert {v[0] for v in general} >= {4, 6, 8, 12} and {v[1] for v in general if v[0] == 10} >= {2, 3}
+    assert {v[2] for v in general} >= {4, 5}
+
+
+def test_standard_loop_and_edge_cases():
+    """Grid-stride and capacity cases are where they are meant to be at 148 SMs."""
+    assert S.pair_loops(S.PAIR_LOOP.B, 3, 1, SMS) and not S.pair_loops(S.PAIR_LOOP.B // 2, 3, 1, SMS)
+    for c in S.BCR_CASES:
+        if c.K == 40:
+            assert c.B > SMS * S.bcr_resident(40, c.D)
+    for D, K in ((1, 907), (2, 604), (3, 453)):
+        c = S.Case(K, D, 3, "given", False, False, False, "pair_long")
+        assert c in [x._replace(times="given", ends=False, free=False, cost=False) for x in S.PAIR_LONG_CASES]
+        assert S.routes_of([c, c._replace(K=K + 1)]) == ["pair_long", "unsupported"]
+    N, K, D, B = S.SOLVE_LOOP
+    assert W.general_loops(B, S.general_solve_warps(N, K, D), SMS)
+    steps, refused = S.general_solve_steps(10, 3)
+    assert (steps, refused) == W.warp_steps(3, "standard")
+    assert {K for N, K, _, _ in S.SOLVE_CASES if N == 10} >= {k for lo_hi in steps.values() for k in lo_hi}
+    steps12, _ = S.general_solve_steps(12, 3)
+    assert {S.general_solve_warps(12, K, 3) for N, K, _, _ in S.SOLVE_CASES if N == 12} == set(steps12)
+    # past the standard-mask kernels (K = 513 / 604 / 907 at D = 3 / 2 / 1) the general route refuses every K, and
+    # each first refused K has a case
+    for D, K in S.REFUSED.items():
+        c = S.Case(K, D, 2, "given", False, False, False)
+        assert S.routes_of([c, c._replace(K=K - 1)]) == ["general", "bcr" if D == 3 else "pair_long"]
+        assert S.general_solve_warps(10, K, D) is None
+    assert S.REFUSED == {3: 514, 2: 605, 1: 908}

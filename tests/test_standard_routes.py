@@ -29,21 +29,22 @@ TABLE = [
 ]
 
 
-@pytest.fixture(scope="module")
-def routes():
+def run_routes(queries):
+    """The route of each query: (B, K, D, N, derivative, sms, coeffs_aligned16, inputs_aligned16, forced or None).
+    Builds the binary when a header is newer (tests/test_gpu_standard_variants.py tags its cases with it too)."""
     deps = [SRC] + [os.path.join(CSRC, f) for f in os.listdir(CSRC) if f.endswith((".cuh", ".h"))]
     if not os.path.exists(BIN) or any(os.path.getmtime(d) > os.path.getmtime(BIN) for d in deps):
         os.makedirs(os.path.dirname(BIN), exist_ok=True)
         subprocess.check_call(["nvcc", "-gencode", "arch=compute_100a,code=sm_100a", "-std=c++17", SRC, "-o", BIN])
+    text = "".join("%d %d %d %d %d %d %d %d %s\n" % (*q[:6], int(q[6]), int(q[7]), q[8] or "-") for q in queries)
+    out = subprocess.run([BIN], input=text, capture_output=True, text=True, check=True).stdout.split()
+    assert len(out) == len(queries)
+    return out
 
-    def run(queries):
-        """queries: (B, K, D, N, derivative, sms, coeffs_aligned16, inputs_aligned16, forced or None)"""
-        text = "".join("%d %d %d %d %d %d %d %d %s\n" % (*q[:6], int(q[6]), int(q[7]), q[8] or "-") for q in queries)
-        out = subprocess.run([BIN], input=text, capture_output=True, text=True, check=True).stdout.split()
-        assert len(out) == len(queries)
-        return out
 
-    return run
+@pytest.fixture(scope="module")
+def routes():
+    return run_routes
 
 
 def check(routes, cases):
