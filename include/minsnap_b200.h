@@ -218,7 +218,8 @@ MINSNAP_API int minsnap_extrema(long B, int K, int D, int N, const double* d_coe
 
 /* ---- SURVEY 8(f)2: the time-only objective and its numeric gradient ------------------------
  * minsnap_time_objective (ref objectiveFunctionTime, NL.i:765-832, without the collision and
- * soft-constraint terms): for every trajectory b and candidate time allocation s
+ * soft-constraint terms; minsnap_time_objective_soft below adds the soft terms): for every trajectory b and
+ * candidate time allocation s
  *   objective[b][s] = computeCost(solveLinear(times[b][s])) + time_penalty * (sum_k times[b][s][k])^2.
  * Standard mask (as minsnap_cost_sweep, which it runs); d_cost [B][S] optional.
  * minsnap_time_gradient (ref getCostAndGradientTime, NL.i:2155-2243): central differences of
@@ -253,6 +254,66 @@ MINSNAP_API int minsnap_optimize_segment_times(long B, int K, int D, int N, int 
                                                double max_relative_step, double min_time,
                                                double gradient_increment, double* d_history,
                                                minsnap_stream_t stream);
+
+/* ---- the time-only objective with the reference's soft limits on max |p^(k)| ------------------
+ * ref: objectiveFunctionTime with use_soft_constraints (NL.i:765-832), evaluateMaximumMagnitudeAsSoftConstraint
+ *      (NL.i:2396-2426) over evaluateMaximumMagnitudeConstraint (NL.i:2346-2392), i.e. computeMaximumOfMagnitude.
+ * Constraint c (1 <= n_constraints <= 4) limits derivative h_derivatives[c] (0 .. N-2) over all dimensions to
+ * h_limits[c] > 0; its term is
+ *   term_c = min(maximum_cost, exp((max_c - limit_c) / limit_c * weight))     (std::min: a NaN exponent gives
+ *            maximum_cost, as in the reference),
+ * max_c bit-identical to minsnap_extrema(..., MINSNAP_EXTREMA_OPTIMIZATION | extrema_flags)'s max_value.  The soft
+ * cost is the sum of the terms from 0 in constraint order.  weight and maximum_cost are positive and finite;
+ * extrema_flags is 0 (the reference's coefficient truncation) or MINSNAP_EXTREMA_KEEP_SMALL_COEFFICIENTS.  The host
+ * arrays reach the device in kernel parameters, not by a copy, so every call can be captured into a CUDA graph once
+ * it has run eagerly on the thread.  Temporary device memory is allocated stream-ordered (cudaMallocAsync).
+ *
+ * minsnap_soft_constraint_cost: solved trajectories d_coeffs [B][K][D][N], d_times [B][K] (D <= 32) -> d_cost [B];
+ * optional d_terms [B][n_constraints] (term_c) and d_max_value [B][n_constraints] (max_c). */
+MINSNAP_API int minsnap_soft_constraint_cost(long B, int K, int D, int N, const double* d_coeffs,
+                                             const double* d_times, int n_constraints,
+                                             const int32_t* h_derivatives, const double* h_limits,
+                                             double weight, double maximum_cost, int extrema_flags,
+                                             double* d_cost, double* d_terms, double* d_max_value,
+                                             minsnap_stream_t stream);
+
+/* minsnap_time_objective_soft: for every trajectory b and candidate allocation s (standard mask, the shapes
+ * minsnap_solve_standard takes; MINSNAP_ERR_UNSUPPORTED otherwise, before any device work)
+ *   objective[b][s] = computeCost + time_penalty * (sum_k times[b][s][k])^2 + soft cost,
+ * the time sum left to right and the three parts added in that order (cost_trajectory + cost_time +
+ * cost_constraints).  A solve with a non-zero status (e.g. a time <= 0) gives a NaN objective.  d_positions
+ * [B][K+1][D], d_end_derivatives as in minsnap_solve_standard or NULL, d_times [B][S][K] -> d_objective [B][S];
+ * optional d_cost [B][S] (computeCost), d_soft [B][S] (soft cost), d_terms [B][S][n_constraints]. */
+MINSNAP_API int minsnap_time_objective_soft(long B, int S, int K, int D, int N, int derivative,
+                                            const double* d_positions, const double* d_end_derivatives,
+                                            const double* d_times, double time_penalty, int n_constraints,
+                                            const int32_t* h_derivatives, const double* h_limits,
+                                            double weight, double maximum_cost, int extrema_flags,
+                                            double* d_objective, double* d_cost, double* d_soft,
+                                            double* d_terms, minsnap_stream_t stream);
+
+/* minsnap_optimize_segment_times_soft: minsnap_optimize_segment_times on the objective above (no parity is claimed
+ * for the optimiser, NLopt being absent; only for the objective and its pieces).  Per iteration, at the incumbent:
+ * solve, minsnap_time_gradient (w_d = 0.5, w_t = 0); the 2K allocations T -/+ gradient_increment e_n of every
+ * trajectory (a time <= 0.1 moved to 0.1 on both sides) are re-solved and their soft cost's central difference is
+ * added to the gradient; the step ladder of minsnap_optimize_segment_times (which adds the penalty's gradient);
+ * minsnap_time_objective_soft over the n_steps candidates; the first minimum among the finite objectives is accepted
+ * when strictly below the incumbent.  All launches are on `stream` and nothing returns to the host.  The workspace is
+ * one cudaMallocAsync of, with R = max(2K, n_steps), h = N/2 and n_c = n_constraints,
+ *   8 B (R ((K+1) D + 2 (h-1) D [only with end derivatives] + K D N + K + 3) + K + 1) + 4 B R + 32 B R K n_c bytes
+ * (plus alignment): 4.47 GB at B = 65,536, K = 10, n_steps = 16, D = 3, N = 10, n_c = 2 (computed from the shapes).
+ * d_times [B][K] in/out; d_history (optional) [iterations + 1][B]: the incumbent objective, first at the initial
+ * times; d_max_value (optional) [B][n_constraints]: the maxima at the returned times. */
+MINSNAP_API int minsnap_optimize_segment_times_soft(long B, int K, int D, int N, int derivative,
+                                                    const double* d_positions,
+                                                    const double* d_end_derivatives, double* d_times,
+                                                    int iterations, double time_penalty, int n_steps,
+                                                    double max_relative_step, double min_time,
+                                                    double gradient_increment, int n_constraints,
+                                                    const int32_t* h_derivatives, const double* h_limits,
+                                                    double weight, double maximum_cost, int extrema_flags,
+                                                    double* d_history, double* d_max_value,
+                                                    minsnap_stream_t stream);
 
 /* ---- SURVEY 8(f)3: collision cost of solved trajectories against a signed-distance grid ------
  * ref: PolynomialOptimizationNonLinear::getCostAndGradientCollision (NL.i:1523-1709, cost and collision flag),

@@ -1,9 +1,10 @@
 """Python plumbing over the C ABI: torch tensors for device memory and streams, numpy arrays
 for the host-buffer entry points.  Every function is a thin argument marshaller around one
-C-ABI call -- there is no arithmetic and no fallback here.  The two additive drivers of the
-time-only problem (optimize_segment_times, time_objective_with_soft_constraints) are the
-exception: they chain several C-ABI calls on the device and glue them with elementwise torch
-operations (step ladders, exp / clamp of the soft-constraint terms).
+C-ABI call -- there is no arithmetic and no fallback here.  The exceptions are the torch-glue
+versions kept as the tests' checkers (time_objective_with_soft_constraints and the *_reference_glue
+drivers), which chain several C-ABI calls on the device and glue them with elementwise torch
+operations (step ladders, exp / clamp of the soft-constraint terms), and the cost_time term that
+time_objective_soft reports with want_terms.
 
 Layouts are those of include/minsnap_b200.h (h = N/2):
   fixed_values [B][n_fixed][D], free_values [B][n_free][D], positions [B][K+1][D],
@@ -345,6 +346,139 @@ def optimize_segment_times_reference_glue(positions, times, iterations=20, time_
         improved = best < history[-1]
         chosen = cand[torch.arange(B, device=cand.device), arg]
         times = torch.where(improved[:, None], chosen, times)
+        history.append(torch.where(improved, best, history[-1]))
+    return times, torch.stack(history)
+
+
+# ---- the time-only objective with the reference's soft limits on max |p^(k)| ------------------------------------
+def _soft_args(constraints, soft_constraint_weight, maximum_cost, keep_small):
+    """The constraint arguments of the soft-constraint entries, in their order, and the host arrays they point into
+    (which must outlive the call)."""
+    ks = np.asarray([int(k) for k, _ in constraints], np.int32)
+    limits = np.asarray([float(v) for _, v in constraints], np.float64)
+    args = (len(ks), _hptr(ks), _hptr(limits), float(soft_constraint_weight), float(maximum_cost),
+            EXTREMA_KEEP_SMALL_COEFFICIENTS if keep_small else 0)
+    return (ks, limits), args
+
+
+def soft_constraint_cost(coeffs, times, constraints, soft_constraint_weight=100.0, maximum_cost=1.0e12,
+                         keep_small=False, want_terms=False):
+    """Soft cost of solved trajectories (ref evaluateMaximumMagnitudeAsSoftConstraint, NL.i:2396-2426):
+    sum over constraints (k, limit) of min(maximum_cost, exp((max |p^(k)| - limit) / limit * weight)), the maximum
+    that of extrema(..., mode=EXTREMA_OPTIMIZATION) bit for bit.  coeffs [B][K][D][N], times [B][K] -> cost [B]
+    (with want_terms also dict(terms, max_value), each [B][n_constraints]).  One C-ABI call
+    (minsnap_soft_constraint_cost)."""
+    torch = _torch()
+    B, K, D, N = coeffs.shape
+    n_c = len(constraints)
+    dev = coeffs.device
+    cost_t = torch.empty((B,), dtype=torch.float64, device=dev)
+    terms = torch.empty((B, n_c), dtype=torch.float64, device=dev) if want_terms else None
+    peak = torch.empty((B, n_c), dtype=torch.float64, device=dev) if want_terms else None
+    host, sargs = _soft_args(constraints, soft_constraint_weight, maximum_cost, keep_small)
+    capi.check(_lib().minsnap_soft_constraint_cost(B, K, D, N, _dptr(coeffs, torch.float64), _dptr(times, torch.float64),
+                                                   *sargs, _dptr(cost_t), _dptr(terms), _dptr(peak), _stream()),
+               "minsnap_soft_constraint_cost")
+    return (cost_t, dict(terms=terms, max_value=peak)) if want_terms else cost_t
+
+
+def time_objective_soft(positions, times, time_penalty, constraints, soft_constraint_weight=100.0, maximum_cost=1.0e12,
+                        end_derivatives=None, keep_small=False, N=10, derivative=SNAP, want_terms=False):
+    """The objective of time_objective_with_soft_constraints in one C-ABI call (minsnap_time_objective_soft):
+    computeCost + time_penalty * total_time^2 + soft cost, NaN where the solve fails.  positions [B][K+1][D], times
+    [B][S][K] -> objective [B][S]; with want_terms also dict(cost_trajectory, cost_time, cost_constraints) as
+    time_objective_with_soft_constraints gives them (cost_constraints: one [B][S] tensor per constraint)."""
+    torch = _torch()
+    B, K1, D = positions.shape
+    S = times.shape[1]
+    n_c = len(constraints)
+    dev = positions.device
+    obj = torch.empty((B, S), dtype=torch.float64, device=dev)
+    cost_t = torch.empty((B, S), dtype=torch.float64, device=dev) if want_terms else None
+    terms = torch.empty((B, S, n_c), dtype=torch.float64, device=dev) if want_terms else None
+    host, sargs = _soft_args(constraints, soft_constraint_weight, maximum_cost, keep_small)
+    capi.check(_lib().minsnap_time_objective_soft(B, S, K1 - 1, D, N, derivative, _dptr(positions, torch.float64),
+                                                  _dptr(end_derivatives), _dptr(times, torch.float64), float(time_penalty),
+                                                  *sargs, _dptr(obj), _dptr(cost_t), None, _dptr(terms), _stream()),
+               "minsnap_time_objective_soft")
+    if not want_terms:
+        return obj
+    total = times[..., 0]
+    for k in range(1, K1 - 1):       # left to right, as the objective sums it
+        total = total + times[..., k]
+    return obj, dict(cost_trajectory=cost_t, cost_time=total * total * time_penalty,
+                     cost_constraints=[terms[..., j] for j in range(n_c)])
+
+
+def optimize_segment_times_soft(positions, times, constraints, iterations=20, time_penalty=500.0, n_steps=16,
+                                max_relative_step=0.5, min_time=0.1, end_derivatives=None, gradient_increment=1e-3,
+                                soft_constraint_weight=100.0, maximum_cost=1.0e12, keep_small=False, N=10,
+                                derivative=SNAP):
+    """optimize_segment_times on the objective of time_objective_soft: the gradient adds the central difference of
+    the soft cost over re-solved allocations T -/+ gradient_increment e_n.  One C-ABI call
+    (minsnap_optimize_segment_times_soft): the whole loop is enqueued on the current stream.  Returns (times,
+    objective history [iterations + 1][B], max_value [B][n_constraints] at the returned times)."""
+    torch = _torch()
+    B, K1, D = positions.shape
+    times = times.clone().contiguous()
+    history = torch.empty((iterations + 1, B), dtype=torch.float64, device=positions.device)
+    peak = torch.empty((B, len(constraints)), dtype=torch.float64, device=positions.device)
+    host, sargs = _soft_args(constraints, soft_constraint_weight, maximum_cost, keep_small)
+    capi.check(_lib().minsnap_optimize_segment_times_soft(B, K1 - 1, D, N, derivative, _dptr(positions, torch.float64),
+                                                          _dptr(end_derivatives), _dptr(times, torch.float64),
+                                                          int(iterations), float(time_penalty), int(n_steps),
+                                                          float(max_relative_step), float(min_time),
+                                                          float(gradient_increment), *sargs, _dptr(history), _dptr(peak),
+                                                          _stream()), "minsnap_optimize_segment_times_soft")
+    return times, history, peak
+
+
+def optimize_segment_times_soft_reference_glue(positions, times, constraints, iterations=20, time_penalty=500.0,
+                                               n_steps=16, max_relative_step=0.5, min_time=0.1, end_derivatives=None,
+                                               gradient_increment=1e-3, soft_constraint_weight=100.0,
+                                               maximum_cost=1.0e12, keep_small=False):
+    """The descent of optimize_segment_times_soft with its glue written in elementwise torch operations around the
+    C-ABI calls (solve_standard, time_gradient, soft_constraint_cost, time_objective_soft): kept as the checker of
+    minsnap_optimize_segment_times_soft in the tests."""
+    torch = _torch()
+    B, K1, D = positions.shape
+    K = K1 - 1
+    dev = positions.device
+    soft_kw = dict(soft_constraint_weight=soft_constraint_weight, maximum_cost=maximum_cost, keep_small=keep_small)
+
+    def objective(t):
+        return time_objective_soft(positions, t.contiguous(), time_penalty, constraints, end_derivatives=end_derivatives,
+                                   **soft_kw)
+
+    times = times.clone()
+    history = [objective(times[:, None, :])[:, 0]]
+    ladder = max_relative_step * 0.5 ** torch.arange(n_steps, dtype=torch.float64, device=dev)
+    eye = torch.eye(K, dtype=torch.bool, device=dev)
+    rep_p = positions.repeat_interleave(2 * K, dim=0).contiguous()
+    rep_e = None if end_derivatives is None else end_derivatives.repeat_interleave(2 * K, dim=0).contiguous()
+    rows = torch.arange(B, device=dev)
+    h = gradient_increment
+    for _ in range(iterations):
+        coeffs = solve_standard(positions, times, end_derivatives=end_derivatives, want_status=False)["coeffs"]
+        g = time_gradient(coeffs, times, increment=h, w_d=0.5, w_t=0.0)
+        short = times <= 0.1
+        t_minus = torch.where(short, torch.full_like(times, 0.1), times - h)
+        t_plus = torch.where(short, torch.full_like(times, 0.1), times + h)
+        base = times[:, None, :].expand(B, K, K)
+        moved = torch.stack([torch.where(eye[None], t_minus[:, None, :], base),
+                             torch.where(eye[None], t_plus[:, None, :], base)], 2)     # [B][n][-/+][K]
+        flat = moved.reshape(B * 2 * K, K).contiguous()
+        c2 = solve_standard(rep_p, flat, end_derivatives=rep_e, want_status=False)["coeffs"]
+        soft = soft_constraint_cost(c2, flat, constraints, **soft_kw).reshape(B, K, 2)
+        g = g + (soft[..., 1] - soft[..., 0]) / (2.0 * h)
+        g = g + 2.0 * time_penalty * times.sum(1, keepdim=True)
+        scale = (times / g.abs().clamp_min(1e-300)).min(1, keepdim=True).values
+        cand = times[:, None, :] - (ladder[None, :, None] * scale[:, :, None]) * g[:, None, :]
+        cand = cand.clamp_min(min_time).contiguous()
+        obj = objective(cand)
+        best, arg = torch.where(torch.isfinite(obj), obj, torch.full_like(obj, float("inf"))).min(1)
+        improved = torch.isfinite(best) & (best < history[-1])
+        times = torch.where(improved[:, None], cand[rows, arg], times)
         history.append(torch.where(improved, best, history[-1]))
     return times, torch.stack(history)
 

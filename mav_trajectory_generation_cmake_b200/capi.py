@@ -48,6 +48,11 @@ SIGNATURES = {
     "minsnap_time_objective": (_i, [_l, _i, _i, _i, _i, _i, _vp, _vp, _vp, _d, _vp, _vp, _vp, _vp]),
     "minsnap_time_gradient": (_i, [_l, _i, _i, _i, _i, _vp, _vp, _d, _d, _d, _vp, _vp, _vp]),
     "minsnap_optimize_segment_times": (_i, [_l, _i, _i, _i, _i, _vp, _vp, _vp, _i, _d, _i, _d, _d, _d, _vp, _vp]),
+    "minsnap_soft_constraint_cost": (_i, [_l, _i, _i, _i, _vp, _vp, _i, _vp, _vp, _d, _d, _i, _vp, _vp, _vp, _vp]),
+    "minsnap_time_objective_soft": (_i, [_l, _i, _i, _i, _i, _i, _vp, _vp, _vp, _d, _i, _vp, _vp, _d, _d, _i, _vp, _vp, _vp,
+                                         _vp, _vp]),
+    "minsnap_optimize_segment_times_soft": (_i, [_l, _i, _i, _i, _i, _vp, _vp, _vp, _i, _d, _i, _d, _d, _d, _i, _vp, _vp, _d,
+                                                 _d, _i, _vp, _vp, _vp]),
     "minsnap_collision_cost": (_i, [_l, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _d, _d, _vp, _vp, _i, _d, _d, _d, _d, _d, _vp, _vp,
                                     _vp, _vp]),
     "minsnap_collision_gradient": (_i, [_l, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _d, _d, _vp, _vp, _i, _d, _d, _d, _d, _d, _vp,

@@ -6,6 +6,7 @@
 #include <cuda_runtime.h>
 
 #include <algorithm>
+#include <cmath>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -573,6 +574,223 @@ int minsnap_optimize_segment_times(long B, int K, int D, int N, int derivative, 
       e = minsnap::launch_time_select(B, n_steps, K, cand, cost, time_penalty, d_times, incumbent,
                                       d_history ? d_history + (size_t)(it + 1) * nb : nullptr, st);
     if (rc == MINSNAP_OK && e != cudaSuccess) rc = cuda_fail(e, "time descent glue");
+  }
+  cudaFreeAsync(ws, st);
+  return rc;
+}
+
+// ---------------------------------------------------------------------------------------
+// The time-only objective with the reference's soft limits on max |p^(k)| (ref objectiveFunctionTime with
+// use_soft_constraints NL.i:765-832, evaluateMaximumMagnitudeAsSoftConstraint NL.i:2396-2426,
+// evaluateMaximumMagnitudeConstraint NL.i:2346-2392)
+// ---------------------------------------------------------------------------------------
+namespace {
+
+// The constraint arguments shared by the three entries, checked and copied into the launcher's arguments.
+int soft_args(int N, int n_constraints, const int32_t* h_derivatives, const double* h_limits, double weight,
+              double maximum_cost, int extrema_flags, minsnap::SoftConstraintArgs* a) {
+  if (n_constraints < 1 || n_constraints > minsnap::kMaxSoftConstraints || !h_derivatives || !h_limits ||
+      !(weight > 0.0 && std::isfinite(weight)) || !(maximum_cost > 0.0 && std::isfinite(maximum_cost)) ||
+      (extrema_flags != 0 && extrema_flags != MINSNAP_EXTREMA_KEEP_SMALL_COEFFICIENTS))
+    return MINSNAP_ERR_ARG;
+  a->n_constraints = n_constraints;
+  for (int c = 0; c < n_constraints; ++c) {
+    if (h_derivatives[c] < 0 || h_derivatives[c] > N - 2 || !(h_limits[c] > 0.0 && std::isfinite(h_limits[c])))
+      return MINSNAP_ERR_ARG;
+    a->derivative[c] = h_derivatives[c];
+    a->limit[c] = h_limits[c];
+  }
+  a->weight = weight;
+  a->maximum_cost = maximum_cost;
+  a->keep_small = extrema_flags == MINSNAP_EXTREMA_KEEP_SMALL_COEFFICIENTS;
+  return MINSNAP_OK;
+}
+
+// Scratch of the objective pipeline for up to n allocations: positions (and end derivatives) replicated per
+// allocation, coefficients, computeCost, solve status, per-segment maxima.
+struct SoftScratch {
+  double* positions;
+  double* end;
+  double* coeffs;
+  double* cost;
+  int32_t* status;
+  void* extrema;
+  static size_t bytes(size_t n, int K, int D, int N, bool with_end, int n_constraints) {
+    const size_t doubles = n * ((size_t)(K + 1) * D + (with_end ? (size_t)(N - 2) * D : 0) + (size_t)K * D * N + 1);
+    return align_up(sizeof(double) * doubles + sizeof(int32_t) * n, 256) +
+           minsnap::soft_constraint_scratch_bytes((long)n, K, n_constraints);
+  }
+  SoftScratch(void* base, size_t n, int K, int D, int N, bool with_end) {
+    positions = static_cast<double*>(base);
+    end = positions + n * (K + 1) * D;
+    coeffs = end + (with_end ? n * (N - 2) * D : 0);
+    cost = coeffs + n * K * D * N;
+    status = reinterpret_cast<int32_t*>(cost + n);
+    extrema = static_cast<char*>(base) + align_up(sizeof(double) * (size_t)(cost + n - positions) + sizeof(int32_t) * n, 256);
+  }
+};
+
+// Solves the R allocations d_times [B R][K] of every trajectory (coefficients, and computeCost and status when
+// want_cost) from its positions replicated R times.
+int solve_replicated(long B, int R, int K, int D, int N, int derivative, const double* d_positions,
+                     const double* d_end_derivatives, const double* d_times, bool want_cost, const SoftScratch& s,
+                     cudaStream_t st) {
+  CU(minsnap::launch_replicate_rows(B, R, (K + 1) * D, d_positions, s.positions, (N - 2) * D, d_end_derivatives, s.end,
+                                    st));
+  return minsnap_solve_standard(B * R, K, D, N, derivative, s.positions, d_end_derivatives ? s.end : nullptr, d_times,
+                                0.0, 0.0, 0.0, nullptr, s.coeffs, nullptr, want_cost ? s.cost : nullptr,
+                                want_cost ? s.status : nullptr, st);
+}
+
+// minsnap_time_objective_soft on the device: replicate, solve with cost and status, soft cost with the objective
+// epilogue.  d_cost (optional) receives computeCost; without it the scratch holds it.
+int soft_objective_device(long B, int S, int K, int D, int N, int derivative, const double* d_positions,
+                          const double* d_end_derivatives, const double* d_times, double time_penalty,
+                          minsnap::SoftConstraintArgs a, double* d_objective, double* d_cost, double* d_soft,
+                          double* d_terms, const SoftScratch& s, cudaStream_t st) {
+  SoftScratch sc = s;
+  if (d_cost) sc.cost = d_cost;
+  const int rc = solve_replicated(B, S, K, D, N, derivative, d_positions, d_end_derivatives, d_times, true, sc, st);
+  if (rc != MINSNAP_OK) return rc;
+  a.B = B * S; a.K = K; a.D = D; a.N = N;
+  a.d_coeffs = sc.coeffs; a.d_times = d_times; a.d_scratch = sc.extrema;
+  a.d_soft = d_soft; a.d_terms = d_terms; a.d_max_value = nullptr;
+  a.d_objective = d_objective; a.d_cost = sc.cost; a.d_status = sc.status; a.time_penalty = time_penalty;
+  CU(minsnap::launch_soft_constraint_cost(a, st));
+  return MINSNAP_OK;
+}
+
+}  // namespace
+
+int minsnap_soft_constraint_cost(long B, int K, int D, int N, const double* d_coeffs, const double* d_times,
+                                 int n_constraints, const int32_t* h_derivatives, const double* h_limits, double weight,
+                                 double maximum_cost, int extrema_flags, double* d_cost, double* d_terms,
+                                 double* d_max_value, minsnap_stream_t stream) {
+  if (B < 0 || K < 1 || D < 1 || D > 32 || !minsnap::supported_n(N)) return MINSNAP_ERR_ARG;
+  minsnap::SoftConstraintArgs a;
+  int rc = soft_args(N, n_constraints, h_derivatives, h_limits, weight, maximum_cost, extrema_flags, &a);
+  if (rc != MINSNAP_OK) return rc;
+  if (B == 0) return MINSNAP_OK;
+  if (!d_coeffs || !d_times || !d_cost) return MINSNAP_ERR_ARG;
+  cudaStream_t st = as_stream(stream);
+  void* scratch = nullptr;
+  retain_pool_memory();
+  CU(cudaMallocAsync(&scratch, minsnap::soft_constraint_scratch_bytes(B, K, n_constraints), st));
+  a.B = B; a.K = K; a.D = D; a.N = N;
+  a.d_coeffs = d_coeffs; a.d_times = d_times; a.d_scratch = scratch;
+  a.d_soft = d_cost; a.d_terms = d_terms; a.d_max_value = d_max_value;
+  const cudaError_t e = minsnap::launch_soft_constraint_cost(a, st);
+  if (e != cudaSuccess) rc = cuda_fail(e, "launch_soft_constraint_cost");
+  cudaFreeAsync(scratch, st);
+  return rc;
+}
+
+int minsnap_time_objective_soft(long B, int S, int K, int D, int N, int derivative, const double* d_positions,
+                                const double* d_end_derivatives, const double* d_times, double time_penalty,
+                                int n_constraints, const int32_t* h_derivatives, const double* h_limits, double weight,
+                                double maximum_cost, int extrema_flags, double* d_objective, double* d_cost,
+                                double* d_soft, double* d_terms, minsnap_stream_t stream) {
+  if (!shape_ok(B, K, D, N, derivative) || S < 1) return MINSNAP_ERR_ARG;
+  minsnap::SoftConstraintArgs a;
+  int rc = soft_args(N, n_constraints, h_derivatives, h_limits, weight, maximum_cost, extrema_flags, &a);
+  if (rc != MINSNAP_OK) return rc;
+  if (B == 0) return MINSNAP_OK;
+  if (!d_positions || !d_times || !d_objective) return MINSNAP_ERR_ARG;
+  if (!minsnap::standard_supported(K, D, N, derivative)) return MINSNAP_ERR_UNSUPPORTED;
+  cudaStream_t st = as_stream(stream);
+  const size_t n = (size_t)B * S;
+  const bool with_end = d_end_derivatives != nullptr;
+  void* ws = nullptr;
+  retain_pool_memory();
+  CU(cudaMallocAsync(&ws, SoftScratch::bytes(n, K, D, N, with_end, n_constraints), st));
+  const SoftScratch s(ws, n, K, D, N, with_end);
+  rc = soft_objective_device(B, S, K, D, N, derivative, d_positions, d_end_derivatives, d_times, time_penalty, a,
+                             d_objective, d_cost, d_soft, d_terms, s, st);
+  cudaFreeAsync(ws, st);
+  return rc;
+}
+
+// The descent of minsnap_optimize_segment_times on the objective with the soft terms, never leaving the device.
+// Per iteration: solve at the incumbent, time gradient, 2K re-solved allocations per trajectory and their soft cost,
+// the soft term's central difference added to the gradient, step ladder, the objective pipeline over the ladder,
+// select.  Workspace (one stream-ordered allocation), with R = max(2K, n_steps) and n_c constraints:
+//   8 B (R (K+1) D + R 2 (h-1) D [end derivatives given] + R K D N + R K + 3 R + K + 1) + 4 B R
+//   + 32 B R K n_c bytes (+ alignment),
+// 4.47 GB at B = 65,536, K = 10, n_steps = 16, D = 3, N = 10, two constraints, no end derivatives.
+int minsnap_optimize_segment_times_soft(long B, int K, int D, int N, int derivative, const double* d_positions,
+                                        const double* d_end_derivatives, double* d_times, int iterations,
+                                        double time_penalty, int n_steps, double max_relative_step, double min_time,
+                                        double gradient_increment, int n_constraints, const int32_t* h_derivatives,
+                                        const double* h_limits, double weight, double maximum_cost, int extrema_flags,
+                                        double* d_history, double* d_max_value, minsnap_stream_t stream) {
+  if (!shape_ok(B, K, D, N, derivative) || iterations < 0 || n_steps < 1 || !(max_relative_step > 0.0) ||
+      !(min_time > 0.0) || !(gradient_increment > 0.0))
+    return MINSNAP_ERR_ARG;
+  minsnap::SoftConstraintArgs a;
+  int rc = soft_args(N, n_constraints, h_derivatives, h_limits, weight, maximum_cost, extrema_flags, &a);
+  if (rc != MINSNAP_OK) return rc;
+  if (B == 0) return MINSNAP_OK;
+  if (!d_positions || !d_times) return MINSNAP_ERR_ARG;
+  if (!minsnap::standard_supported(K, D, N, derivative)) return MINSNAP_ERR_UNSUPPORTED;
+  cudaStream_t st = as_stream(stream);
+  const size_t nb = (size_t)B, R = std::max<size_t>(2 * (size_t)K, (size_t)n_steps), n = nb * R;
+  const bool with_end = d_end_derivatives != nullptr;
+  const size_t head = align_up(SoftScratch::bytes(n, K, D, N, with_end, n_constraints), 256);
+  char* ws = nullptr;
+  retain_pool_memory();
+  CU(cudaMallocAsync(reinterpret_cast<void**>(&ws), head + sizeof(double) * (n * K + 2 * n + nb * K + nb), st));
+  const SoftScratch s(ws, n, K, D, N, with_end);
+  double* cand = reinterpret_cast<double*>(ws + head);   // [B][R][K]: the 2K differences, then the ladder
+  double* soft = cand + n * K;                          // [B][2K] soft cost of the differences
+  double* obj = soft + n;                               // [B][n_steps] objective of the ladder
+  double* grad = obj + n;
+  double* incumbent = grad + nb * K;
+  a.K = K; a.D = D; a.N = N;
+  // the incumbent objective at the initial times: the candidate pipeline with one allocation per trajectory
+  rc = soft_objective_device(B, 1, K, D, N, derivative, d_positions, d_end_derivatives, d_times, time_penalty, a,
+                             incumbent, nullptr, nullptr, nullptr, s, st);
+  if (rc == MINSNAP_OK && d_history)
+    if (cudaMemcpyAsync(d_history, incumbent, sizeof(double) * nb, cudaMemcpyDeviceToDevice, st) != cudaSuccess) rc = MINSNAP_ERR_CUDA;
+  for (int it = 0; it < iterations && rc == MINSNAP_OK; ++it) {
+    rc = minsnap_solve_standard(B, K, D, N, derivative, d_positions, d_end_derivatives, d_times, 0.0, 0.0, 0.0, nullptr,
+                                s.coeffs, nullptr, nullptr, nullptr, st);
+    // d computeCost / dT = 0.5 dJ_d/dT (w_d = 0.5, w_t = 0), as minsnap_optimize_segment_times
+    if (rc == MINSNAP_OK)
+      rc = minsnap_time_gradient(B, K, D, N, derivative, s.coeffs, d_times, gradient_increment, 0.5, 0.0, grad, nullptr, st);
+    cudaError_t e = cudaSuccess;
+    if (rc == MINSNAP_OK) e = minsnap::launch_soft_gradient_candidates(B, K, d_times, gradient_increment, cand, st);
+    if (rc == MINSNAP_OK && e == cudaSuccess)
+      rc = solve_replicated(B, 2 * K, K, D, N, derivative, d_positions, d_end_derivatives, cand, false, s, st);
+    if (rc == MINSNAP_OK && e == cudaSuccess) {
+      minsnap::SoftConstraintArgs g = a;
+      g.B = B * 2 * K; g.d_coeffs = s.coeffs; g.d_times = cand; g.d_scratch = s.extrema;
+      g.d_soft = soft; g.d_terms = nullptr; g.d_max_value = nullptr;
+      e = minsnap::launch_soft_constraint_cost(g, st);
+    }
+    if (rc == MINSNAP_OK && e == cudaSuccess) e = minsnap::launch_soft_gradient_add(B, K, soft, gradient_increment, grad, st);
+    // the ladder adds the penalty's gradient 2 time_penalty sum(T)
+    if (rc == MINSNAP_OK && e == cudaSuccess)
+      e = minsnap::launch_time_candidates(B, n_steps, K, d_times, grad, time_penalty, max_relative_step, min_time, cand, st);
+    if (rc == MINSNAP_OK && e == cudaSuccess)
+      rc = soft_objective_device(B, n_steps, K, D, N, derivative, d_positions, d_end_derivatives, cand, time_penalty, a,
+                                 obj, nullptr, nullptr, nullptr, s, st);
+    // the first minimum among the finite objectives, accepted when strictly below the incumbent (no free values)
+    if (rc == MINSNAP_OK && e == cudaSuccess)
+      e = minsnap::launch_free_select(B, n_steps, 0, K, obj, nullptr, cand, nullptr, nullptr, d_times, incumbent, nullptr,
+                                      d_history ? d_history + (size_t)(it + 1) * nb : nullptr, st);
+    if (rc == MINSNAP_OK && e != cudaSuccess) rc = cuda_fail(e, "soft time descent glue");
+  }
+  // the maxima at the returned times, from the solve minsnap_solve_standard gives for this batch
+  if (rc == MINSNAP_OK && d_max_value) {
+    rc = minsnap_solve_standard(B, K, D, N, derivative, d_positions, d_end_derivatives, d_times, 0.0, 0.0, 0.0, nullptr,
+                                s.coeffs, nullptr, nullptr, nullptr, st);
+    if (rc == MINSNAP_OK) {
+      minsnap::SoftConstraintArgs m = a;
+      m.B = B; m.d_coeffs = s.coeffs; m.d_times = d_times; m.d_scratch = s.extrema;
+      m.d_soft = nullptr; m.d_terms = nullptr; m.d_max_value = d_max_value;
+      const cudaError_t e = minsnap::launch_soft_constraint_cost(m, st);
+      if (e != cudaSuccess) rc = cuda_fail(e, "launch_soft_constraint_cost");
+    }
   }
   cudaFreeAsync(ws, st);
   return rc;

@@ -360,6 +360,53 @@ __global__ void __launch_bounds__(128) fold_extrema_kernel(FoldParams p) {
   }
 }
 
+struct SoftFoldParams {
+  long B;
+  int K, n_constraints;
+  double limit[kMaxSoftConstraints];
+  double weight, maximum_cost;
+  const SegmentExtremum* per_segment;  // [n_constraints][B][K]
+  double *soft, *terms, *max_value;
+  double* objective;
+  const double* cost;
+  const int32_t* status;
+  const double* times;
+  double time_penalty;
+};
+
+// One thread per trajectory.  Each constraint's maximum is folded from its per-segment maxima with the comparisons
+// and order of fold_extrema_kernel in mode 0, so it is the same bits as minsnap_extrema's max_value.  The term is
+// std::min(maximum_cost, exp(...)) as the reference writes it (a NaN exponent gives maximum_cost), the soft cost
+// their sum from 0 in constraint order (NL.i:2396-2426).  Optional epilogue: the objective of objectiveFunctionTime
+// (NL.i:778-800), cost_trajectory + cost_time + cost_constraints in that order, each operation rounded on its own;
+// a non-zero solve status makes it NaN.
+__global__ void __launch_bounds__(128) soft_constraint_fold_kernel(SoftFoldParams p) {
+  const long b = (long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (b >= p.B) return;
+  double soft = 0.0;
+  for (int c = 0; c < p.n_constraints; ++c) {
+    const SegmentExtremum* e = p.per_segment + ((long)c * p.B + b) * p.K;
+    double max_v = 0.0;
+    for (int s = 0; s < p.K; ++s) {
+      const double v = e[s].max_v;
+      if (v > max_v) max_v = v;
+    }
+    const double x = exp(__dmul_rn(__ddiv_rn(__dsub_rn(max_v, p.limit[c]), p.limit[c]), p.weight));
+    const double term = x < p.maximum_cost ? x : p.maximum_cost;
+    soft = __dadd_rn(soft, term);
+    if (p.terms) p.terms[b * p.n_constraints + c] = term;
+    if (p.max_value) p.max_value[b * p.n_constraints + c] = max_v;
+  }
+  if (p.soft) p.soft[b] = soft;
+  if (p.objective) {
+    double total = 0.0;
+    for (int k = 0; k < p.K; ++k) total += p.times[b * p.K + k];   // ref computeTotalTrajectoryTime: left to right
+    double obj = __dadd_rn(__dadd_rn(p.cost[b], __dmul_rn(__dmul_rn(total, total), p.time_penalty)), soft);
+    if (p.status && p.status[b] != 0) obj = __longlong_as_double(0x7ff8000000000000ll);
+    p.objective[b] = obj;
+  }
+}
+
 template <int LEN>
 cudaError_t launch_segments(const ExtremaParams& p, cudaStream_t stream) {
   const long n = p.B * p.K;
@@ -410,6 +457,51 @@ cudaError_t launch_extrema(const ExtremaArgs& a, cudaStream_t stream) {
   }
   cudaFreeAsync(scratch, stream);
   return e;
+}
+
+size_t soft_constraint_scratch_bytes(long B, int K, int n_constraints) {
+  return sizeof(SegmentExtremum) * (size_t)n_constraints * B * K;
+}
+
+// One segment_extrema_kernel launch per constraint (mode 0, all dimensions) into its slab of the caller's scratch,
+// then one fold over all constraints.
+cudaError_t launch_soft_constraint_cost(const SoftConstraintArgs& a, cudaStream_t stream) {
+  if (a.B == 0) return cudaSuccess;
+  SegmentExtremum* per_segment = static_cast<SegmentExtremum*>(a.d_scratch);
+  const uint32_t all = a.D == 32 ? 0xffffffffu : ((1u << a.D) - 1u);
+  for (int c = 0; c < a.n_constraints; ++c) {
+    const int len = extrema_max_roots(a.N, a.derivative[c], a.D) + 1;
+    if (len > kMaxG) return cudaErrorInvalidValue;
+    ExtremaParams p;
+    p.B = a.B; p.K = a.K; p.D = a.D; p.N = a.N; p.derivative = a.derivative[c]; p.mode = 0;
+    p.keep_small = a.keep_small;
+    p.dim_mask = all;
+    p.coeffs = a.d_coeffs; p.times = a.d_times;
+    p.per_segment = per_segment + (size_t)c * a.B * a.K;
+    p.cand_times = nullptr; p.cand_values = nullptr; p.root_count = nullptr;
+    p.max_roots = len - 1;
+    const cudaError_t e = len <= 4    ? launch_segments<4>(p, stream)
+                          : len <= 6  ? launch_segments<6>(p, stream)
+                          : len <= 8  ? launch_segments<8>(p, stream)
+                          : len <= 10 ? launch_segments<10>(p, stream)
+                          : len <= 12 ? launch_segments<12>(p, stream)
+                          : len <= 14 ? launch_segments<14>(p, stream)
+                          : len <= 16 ? launch_segments<16>(p, stream)
+                          : len <= 18 ? launch_segments<18>(p, stream)
+                          : len <= 20 ? launch_segments<20>(p, stream)
+                                      : launch_segments<22>(p, stream);
+    if (e != cudaSuccess) return e;
+  }
+  SoftFoldParams f;
+  f.B = a.B; f.K = a.K; f.n_constraints = a.n_constraints;
+  for (int c = 0; c < kMaxSoftConstraints; ++c) f.limit[c] = c < a.n_constraints ? a.limit[c] : 0.0;
+  f.weight = a.weight; f.maximum_cost = a.maximum_cost;
+  f.per_segment = per_segment;
+  f.soft = a.d_soft; f.terms = a.d_terms; f.max_value = a.d_max_value;
+  f.objective = a.d_objective; f.cost = a.d_cost; f.status = a.d_status; f.times = a.d_times;
+  f.time_penalty = a.time_penalty;
+  soft_constraint_fold_kernel<<<(unsigned)((a.B + 127) / 128), 128, 0, stream>>>(f);
+  return cudaGetLastError();
 }
 
 }  // namespace minsnap

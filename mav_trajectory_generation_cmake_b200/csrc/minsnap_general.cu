@@ -839,4 +839,88 @@ cudaError_t launch_free_select(long B, int S, int n_fd, int K, const double* d_c
   return cudaGetLastError();
 }
 
+// =========================================================================================
+// The glue of the batched time descent with the reference's soft limits on max |p^(k)|, on the device.  See
+// minsnap_optimize_segment_times_soft.  The maximum is not a fixed quadratic form in the end-point derivatives, so
+// its gradient re-solves the 2K allocations T -/+ h e_n of every trajectory; they and the step ladder's candidates
+// go through minsnap_solve_standard, which takes one row of positions per allocation.
+// =========================================================================================
+// out_p[i] = positions[i / R], out_e[i] = end[i / R] for i < B R (rows of row_p / row_e doubles)
+__global__ void __launch_bounds__(256) replicate_rows_kernel(long B, int R, int row_p,
+                                                             const double* __restrict__ positions,
+                                                             double* __restrict__ out_p, int row_e,
+                                                             const double* __restrict__ end,
+                                                             double* __restrict__ out_e) {
+  const long n_p = B * R * row_p;
+  const long total = n_p + B * R * row_e;
+  for (long idx = (long)blockIdx.x * blockDim.x + threadIdx.x; idx < total; idx += (long)gridDim.x * blockDim.x) {
+    if (idx < n_p) {
+      const long i = idx / row_p;
+      out_p[idx] = positions[(i / R) * row_p + (idx - i * row_p)];
+    } else {
+      const long j = idx - n_p;
+      const long i = j / row_e;
+      out_e[j] = end[(i / R) * row_e + (j - i * row_e)];
+    }
+  }
+}
+
+// cand[(b K + n) 2 + j][k] = times[b][k], except k = n: T_n - increment (j = 0) or T_n + increment (j = 1), and
+// 0.1 on both sides when T_n <= 0.1 (the clamp of getCostAndGradientTime, NL.i:2186-2187, 2207-2208).
+__global__ void __launch_bounds__(256) soft_gradient_candidates_kernel(long B, int K, const double* __restrict__ times,
+                                                                       double increment, double* __restrict__ cand) {
+  const long total = B * K * 2 * K;
+  for (long idx = (long)blockIdx.x * blockDim.x + threadIdx.x; idx < total; idx += (long)gridDim.x * blockDim.x) {
+    const long row = idx / K;
+    const int k = (int)(idx - row * K);
+    const int j = (int)(row & 1);
+    const long bn = row >> 1;
+    const long b = bn / K;
+    const int n = (int)(bn - b * K);
+    const double T = times[b * K + k];
+    double v = T;
+    if (k == n) v = T <= 0.1 ? 0.1 : (j == 0 ? T - increment : T + increment);
+    cand[idx] = v;
+  }
+}
+
+__global__ void __launch_bounds__(256) soft_gradient_add_kernel(long n, const double* __restrict__ soft,
+                                                                double increment, double* __restrict__ gradient) {
+  const long i = (long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  gradient[i] = __dadd_rn(gradient[i], __ddiv_rn(__dsub_rn(soft[2 * i + 1], soft[2 * i]), 2.0 * increment));
+}
+
+static long glue_grid(long total) {
+  long grid = (total + 255) / 256;
+  if (grid > sm_count() * 32) grid = sm_count() * 32;
+  return grid;
+}
+
+cudaError_t launch_replicate_rows(long B, int R, int row_p, const double* d_positions, double* d_out_p, int row_e,
+                                  const double* d_end, double* d_out_e, cudaStream_t stream) {
+  if (!d_end) row_e = 0;
+  const long total = B * R * (long)(row_p + row_e);
+  if (total == 0) return cudaSuccess;
+  replicate_rows_kernel<<<(int)glue_grid(total), 256, 0, stream>>>(B, R, row_p, d_positions, d_out_p, row_e, d_end,
+                                                                    d_out_e);
+  return cudaGetLastError();
+}
+
+cudaError_t launch_soft_gradient_candidates(long B, int K, const double* d_times, double increment, double* d_cand,
+                                            cudaStream_t stream) {
+  const long total = B * K * 2 * K;
+  if (total == 0) return cudaSuccess;
+  soft_gradient_candidates_kernel<<<(int)glue_grid(total), 256, 0, stream>>>(B, K, d_times, increment, d_cand);
+  return cudaGetLastError();
+}
+
+cudaError_t launch_soft_gradient_add(long B, int K, const double* d_soft, double increment, double* d_gradient,
+                                     cudaStream_t stream) {
+  const long n = B * K;
+  if (n == 0) return cudaSuccess;
+  soft_gradient_add_kernel<<<(unsigned)((n + 255) / 256), 256, 0, stream>>>(n, d_soft, increment, d_gradient);
+  return cudaGetLastError();
+}
+
 }  // namespace minsnap

@@ -96,6 +96,17 @@ cudaError_t launch_free_select(long B, int S, int n_fd, int K, const double* d_c
                                const double* d_cand_times, const int32_t* d_cand_hit, double* d_free, double* d_times,
                                double* d_incumbent, int32_t* d_hit, double* d_history_row, cudaStream_t stream);
 
+// device-side glue of the time descent with soft limits (minsnap_optimize_segment_times_soft)
+// out_p[b R + r] = positions[b] (row_p doubles each), out_e likewise when d_end is set
+cudaError_t launch_replicate_rows(long B, int R, int row_p, const double* d_positions, double* d_out_p, int row_e,
+                                  const double* d_end, double* d_out_e, cudaStream_t stream);
+// cand[(b K + n) 2 + j] = times[b] with segment n moved by -/+ increment (j = 0 / 1); a time <= 0.1 moves to 0.1
+cudaError_t launch_soft_gradient_candidates(long B, int K, const double* d_times, double increment, double* d_cand,
+                                            cudaStream_t stream);
+// gradient[b K + n] += (soft[(b K + n) 2 + 1] - soft[(b K + n) 2]) / (2 increment)
+cudaError_t launch_soft_gradient_add(long B, int K, const double* d_soft, double increment, double* d_gradient,
+                                     cudaStream_t stream);
+
 // ---- minsnap_standard.cu ---------------------------------------------------------------
 // The kernels behind minsnap_solve_standard; choose_standard_route (minsnap_standard_route.cuh) picks one.
 enum class StandardRoute { Tm, Pair, PairLong, Bcr, Chunked, General, Unsupported };
@@ -174,6 +185,33 @@ struct ExtremaArgs {
 };
 int extrema_max_roots(int N, int derivative, int n_dims);
 cudaError_t launch_extrema(const ExtremaArgs& a, cudaStream_t stream);
+
+// Soft limits on max |p^(k)| over all dimensions (ref evaluateMaximumMagnitudeAsSoftConstraint NL.i:2396-2426 over
+// computeMaximumOfMagnitude, mode 0): soft = sum_c min(maximum_cost, exp((max_c - limit_c) / limit_c * weight)).
+// The constraints travel by value in the kernels' parameters.
+constexpr int kMaxSoftConstraints = 4;
+struct SoftConstraintArgs {
+  long B;
+  int K, D, N;
+  int n_constraints;
+  int derivative[kMaxSoftConstraints];
+  double limit[kMaxSoftConstraints];
+  double weight, maximum_cost;
+  bool keep_small;
+  const double* d_coeffs;   // [B][K][D][N]
+  const double* d_times;    // [B][K]
+  void* d_scratch;          // soft_constraint_scratch_bytes(B, K, n_constraints)
+  double* d_soft;           // optional [B]
+  double* d_terms;          // optional [B][n_constraints]
+  double* d_max_value;      // optional [B][n_constraints]
+  // objective epilogue, on when d_objective is set: cost + time_penalty (sum_k times)^2 + soft, NaN where status != 0
+  double* d_objective = nullptr;  // [B]
+  const double* d_cost = nullptr; // [B] computeCost
+  const int32_t* d_status = nullptr;  // optional [B]
+  double time_penalty = 0.0;
+};
+size_t soft_constraint_scratch_bytes(long B, int K, int n_constraints);
+cudaError_t launch_soft_constraint_cost(const SoftConstraintArgs& a, cudaStream_t stream);
 
 // ---- minsnap_collision.cu ---------------------------------------------------------------
 // SURVEY 8(f)3 (ref getCostAndGradientCollision NL.i:1523-1709): collision cost against a dense distance grid
