@@ -429,6 +429,77 @@ MINSNAP_API int minsnap_optimize_free_constraints(long B, int K, int D, int N, i
                                                   double* d_history, int32_t* d_is_collision,
                                                   minsnap_stream_t stream);
 
+/* ---- the soft limits of minsnap_soft_constraint_cost in the free-derivative problem ---------------------------
+ * minsnap_soft_constraint_gradient: the soft cost of solved trajectories d_coeffs [B][K][D][N], d_times [B][K]
+ * (D <= 32, any mask h_fixed_mask [(K+1)][N/2]) and its gradient in closed form, in the free derivatives d_p
+ * (d_grad_free [B][n_free][D], the layout of d_free_values; required when n_free > 0) and, with the end-point
+ * derivatives d held fixed as minsnap_time_gradient holds them, in the segment times (d_grad_times [B][K],
+ * optional).  It runs the extrema passes of minsnap_soft_constraint_cost once, then one gradient kernel on their
+ * per-segment maxima: for constraint c the maximum m is attained at segment s*, time t* (the first strict maximum in
+ * the fold's order: at ties the result is a subgradient), the term is tau = min(maximum_cost, exp((m - L) / L *
+ * weight)) and dtau/dm = exp(...) weight / L below maximum_cost, 0 when saturated or when m = 0.  Every mode-0
+ * candidate is a stationary point of |p^(k)|^2 in t or a segment start, so dm/dtheta is taken at fixed t*:
+ * sum_dim p_dim^(k)(t*) dp_dim^(k)(t*)/dtheta / m, plus the drift sum_dim p^(k) p^(k+1)(T) / m in T when t* is the
+ * end of the last segment.  Only segment s* contributes; rows of d_seg that map to fixed constraints drop out.  The
+ * terms add in constraint order without atomics, so every run gives the same bits.  d_cost [B] and d_max_value
+ * [B][n_constraints] (optional) are those of minsnap_soft_constraint_cost bit for bit; d_max_time and
+ * d_max_segment [B][n_constraints] (optional) are t* and s*.  The mask reaches the device in kernel parameters and
+ * the scratch is one cudaMallocAsync, so the call can be captured into a CUDA graph. */
+MINSNAP_API int minsnap_soft_constraint_gradient(long B, int K, int D, int N, const uint8_t* h_fixed_mask,
+                                                 const double* d_coeffs, const double* d_times, int n_constraints,
+                                                 const int32_t* h_derivatives, const double* h_limits,
+                                                 double weight, double maximum_cost, int extrema_flags,
+                                                 double* d_cost, double* d_grad_free, double* d_grad_times,
+                                                 double* d_max_value, double* d_max_time, int32_t* d_max_segment,
+                                                 minsnap_stream_t stream);
+
+/* minsnap_free_objective_soft: minsnap_free_objective plus w_sc times the soft cost of the recovered candidate
+ * coefficients, added last: J = ((w_d J_d + w_c J_c) + w_t sum(T)) + w_sc soft.  w_sc >= 0 and finite; with
+ * w_sc = 0 the objective is minsnap_free_objective's bit for bit.  d_soft (optional) [B][S]: the soft cost. */
+MINSNAP_API int minsnap_free_objective_soft(long B, int S, int K, int D, int N, int derivative,
+                                            const uint8_t* h_fixed_mask, const double* d_fixed_values,
+                                            const double* d_free_values, const double* d_times, double w_d,
+                                            double w_c, double w_t, const double* d_sdf, const int32_t* h_dims,
+                                            const double* h_origin, double resolution, double oob_value,
+                                            const double* h_min_bound, const double* h_max_bound,
+                                            int use_continuous_distance, double dt, double map_resolution,
+                                            double epsilon, double robot_radius, double coll_pot_multiplier,
+                                            int n_constraints, const int32_t* h_derivatives,
+                                            const double* h_limits, double weight, double maximum_cost,
+                                            int extrema_flags, double w_sc, double* d_objective, double* d_Jd,
+                                            double* d_Jc, int32_t* d_is_collision, double* d_soft,
+                                            minsnap_stream_t stream);
+
+/* minsnap_optimize_free_constraints_soft: minsnap_optimize_free_constraints on the objective of
+ * minsnap_free_objective_soft.  Per iteration, at the incumbent, the soft cost's maxima and the gradient of
+ * minsnap_soft_constraint_gradient join the other gradients:
+ *   d_p - 2^-s ((w_d g_d + w_c g_c) + w_sc g_sc) / (2 w_d diag(R_pp)),
+ *   with optimize_times the time ladder on (w_d dJ_d/dT + w_t) + w_sc dsoft/dT.
+ * The candidates go through minsnap_free_objective_soft and the same selection; with w_sc = 0 the call returns the
+ * bits of minsnap_optimize_free_constraints.  Shapes the recovery kernel refuses return MINSNAP_ERR_UNSUPPORTED before
+ * any device work.  The workspace is one cudaMallocAsync of, with S = n_steps, n_fd = n_free D, n_c = n_constraints,
+ *   that of minsnap_optimize_free_constraints, 8 B (K D N + 2 n_fd + n_free + K + 3) + 8 B S (n_fd + K + K D N + 3)
+ *   + 4 B (S + 1) (+ alignment), plus 8 B (n_fd + S) + 32 B S K n_c bytes:
+ * 2.06 GB + 0.40 GB at B = 65,536, K = 10, S = 8, standard mask, two constraints (computed from the shapes).
+ * d_max_value (optional) [B][n_constraints]: the maxima at the returned state. */
+MINSNAP_API int minsnap_optimize_free_constraints_soft(long B, int K, int D, int N, int derivative,
+                                                       const uint8_t* h_fixed_mask, const double* d_fixed_values,
+                                                       double* d_free_values, double* d_times, int optimize_times,
+                                                       double w_d, double w_c, double w_t, const double* d_sdf,
+                                                       const int32_t* h_dims, const double* h_origin,
+                                                       double resolution, double oob_value,
+                                                       const double* h_min_bound, const double* h_max_bound,
+                                                       int use_continuous_distance, double dt,
+                                                       double map_resolution, double epsilon, double robot_radius,
+                                                       double coll_pot_multiplier, int n_constraints,
+                                                       const int32_t* h_derivatives, const double* h_limits,
+                                                       double weight, double maximum_cost, int extrema_flags,
+                                                       double w_sc, int iterations, int n_steps,
+                                                       double max_relative_step, double min_time,
+                                                       double gradient_increment, double* d_history,
+                                                       int32_t* d_is_collision, double* d_max_value,
+                                                       minsnap_stream_t stream);
+
 /* ---- host-buffer entry points (synchronous; copies inside) -------------------------------
  * The calls a host program makes when its data lives in host memory.  Work is cut into
  * chunks that are copied and solved on alternating streams so that PCIe and the SMs overlap.

@@ -686,6 +686,160 @@ def optimize_free_constraints_reference_glue(mask, fixed_values, free_values, ti
     return free, times, torch.stack(history), hit
 
 
+# ---- the soft limits in the free-derivative problem: J + w_sc soft ----------------------------------------------------
+def soft_constraint_gradient(mask, coeffs, times, constraints, soft_constraint_weight=100.0, maximum_cost=1.0e12,
+                             keep_small=False, want_times=True):
+    """The soft cost of soft_constraint_cost and its closed-form gradient in the free derivatives and, with the
+    end-point derivatives held fixed, in the segment times (minsnap_soft_constraint_gradient).  mask: host uint8
+    [(K+1)][h]; coeffs [B][K][D][N], times [B][K] -> dict(cost [B], grad_free [B][n_free][D], grad_times [B][K] or
+    None, max_value, max_time, max_segment [B][n_constraints]: the maximum and its time and segment)."""
+    torch = _torch()
+    mask = np.ascontiguousarray(mask, np.uint8)
+    B, K, D, N = coeffs.shape
+    n_c = len(constraints)
+    _, n_free = mask_counts(mask)
+    dev = coeffs.device
+    out = dict(cost=torch.empty((B,), dtype=torch.float64, device=dev),
+               grad_free=torch.empty((B, n_free, D), dtype=torch.float64, device=dev),
+               grad_times=torch.empty((B, K), dtype=torch.float64, device=dev) if want_times else None,
+               max_value=torch.empty((B, n_c), dtype=torch.float64, device=dev),
+               max_time=torch.empty((B, n_c), dtype=torch.float64, device=dev),
+               max_segment=torch.empty((B, n_c), dtype=torch.int32, device=dev))
+    host, sargs = _soft_args(constraints, soft_constraint_weight, maximum_cost, keep_small)
+    capi.check(_lib().minsnap_soft_constraint_gradient(B, K, D, N, _hptr(mask), _dptr(coeffs, torch.float64),
+                                                       _dptr(times, torch.float64), *sargs, _dptr(out["cost"]),
+                                                       _dptr(out["grad_free"]), _dptr(out["grad_times"]),
+                                                       _dptr(out["max_value"]), _dptr(out["max_time"]),
+                                                       _dptr(out["max_segment"]), _stream()),
+               "minsnap_soft_constraint_gradient")
+    return out
+
+
+def free_objective_soft(mask, fixed_values, free_values, times, sdf, origin, resolution, min_bound, max_bound, w_c,
+                        constraints, w_sc, w_d=0.1, w_t=1.0, soft_constraint_weight=100.0, maximum_cost=1.0e12,
+                        keep_small=False, dt=0.1, map_resolution=None, epsilon=0.5, robot_radius=0.5,
+                        coll_pot_multiplier=1.0, use_continuous_distance=True, oob_value=0.0, N=10, derivative=SNAP,
+                        want_terms=False):
+    """free_objective plus w_sc times the soft cost of the recovered candidates, added last
+    (minsnap_free_objective_soft).  Shapes as free_objective; with want_terms also dict(Jd, Jc, is_collision, soft),
+    each [B][S]."""
+    torch = _torch()
+    mask = np.ascontiguousarray(mask, np.uint8)
+    K = mask.shape[0] - 1
+    B, S = times.shape[0], times.shape[1]
+    D = fixed_values.shape[2]
+    dev = times.device
+    obj = torch.empty((B, S), dtype=torch.float64, device=dev)
+    terms = dict(Jd=torch.empty((B, S), dtype=torch.float64, device=dev),
+                 Jc=torch.empty((B, S), dtype=torch.float64, device=dev),
+                 is_collision=torch.empty((B, S), dtype=torch.int32, device=dev),
+                 soft=torch.empty((B, S), dtype=torch.float64, device=dev)) if want_terms else {}
+    host, margs = _collision_map(sdf, origin, resolution, min_bound, max_bound, dt, map_resolution, epsilon, robot_radius,
+                                 coll_pot_multiplier, use_continuous_distance, oob_value)
+    shost, sargs = _soft_args(constraints, soft_constraint_weight, maximum_cost, keep_small)
+    capi.check(_lib().minsnap_free_objective_soft(B, S, K, D, N, derivative, _hptr(mask),
+                                                  _dptr(fixed_values, torch.float64), _dptr(free_values, torch.float64),
+                                                  _dptr(times, torch.float64), float(w_d), float(w_c), float(w_t), *margs,
+                                                  *sargs, float(w_sc), _dptr(obj), _dptr(terms.get("Jd")),
+                                                  _dptr(terms.get("Jc")), _dptr(terms.get("is_collision")),
+                                                  _dptr(terms.get("soft")), _stream()), "minsnap_free_objective_soft")
+    return (obj, terms) if want_terms else obj
+
+
+def optimize_free_constraints_soft(mask, fixed_values, free_values, times, sdf, origin, resolution, min_bound,
+                                   max_bound, w_c, constraints, w_sc, w_d=0.1, w_t=1.0, optimize_times=False,
+                                   iterations=20, n_steps=8, max_relative_step=0.5, min_time=0.1,
+                                   gradient_increment=1e-3, soft_constraint_weight=100.0, maximum_cost=1.0e12,
+                                   keep_small=False, dt=0.1, map_resolution=None, epsilon=0.5, robot_radius=0.5,
+                                   coll_pot_multiplier=1.0, use_continuous_distance=True, oob_value=0.0, N=10,
+                                   derivative=SNAP):
+    """optimize_free_constraints on the objective of free_objective_soft: the soft term's closed-form gradient joins
+    the step (and, with optimize_times, the time gradient).  One C-ABI call (minsnap_optimize_free_constraints_soft).
+    Returns (free_values, times, objective history [iterations + 1][B], is_collision [B], max_value
+    [B][n_constraints]), the last two at the returned state."""
+    torch = _torch()
+    mask = np.ascontiguousarray(mask, np.uint8)
+    K = mask.shape[0] - 1
+    B, _, D = fixed_values.shape
+    free_values = free_values.clone().contiguous()
+    times = times.clone().contiguous()
+    dev = times.device
+    history = torch.empty((iterations + 1, B), dtype=torch.float64, device=dev)
+    hit = torch.empty((B,), dtype=torch.int32, device=dev)
+    peak = torch.empty((B, len(constraints)), dtype=torch.float64, device=dev)
+    host, margs = _collision_map(sdf, origin, resolution, min_bound, max_bound, dt, map_resolution, epsilon, robot_radius,
+                                 coll_pot_multiplier, use_continuous_distance, oob_value)
+    shost, sargs = _soft_args(constraints, soft_constraint_weight, maximum_cost, keep_small)
+    capi.check(_lib().minsnap_optimize_free_constraints_soft(B, K, D, N, derivative, _hptr(mask),
+                                                             _dptr(fixed_values, torch.float64), _dptr(free_values),
+                                                             _dptr(times), int(bool(optimize_times)), float(w_d),
+                                                             float(w_c), float(w_t), *margs, *sargs, float(w_sc),
+                                                             int(iterations), int(n_steps), float(max_relative_step),
+                                                             float(min_time), float(gradient_increment), _dptr(history),
+                                                             _dptr(hit), _dptr(peak), _stream()),
+               "minsnap_optimize_free_constraints_soft")
+    return free_values, times, history, hit, peak
+
+
+def optimize_free_constraints_soft_reference_glue(mask, fixed_values, free_values, times, sdf, origin, resolution,
+                                                  min_bound, max_bound, w_c, constraints, w_sc, w_d=0.1, w_t=1.0,
+                                                  optimize_times=False, iterations=20, n_steps=8, max_relative_step=0.5,
+                                                  min_time=0.1, gradient_increment=1e-3, soft_constraint_weight=100.0,
+                                                  maximum_cost=1.0e12, keep_small=False, N=10, derivative=SNAP,
+                                                  **map_kw):
+    """The descent of optimize_free_constraints_soft with its glue written in elementwise torch operations around the
+    C-ABI calls (derivative_gradient, collision_gradient, time_gradient, soft_constraint_gradient,
+    free_objective_soft): kept as the checker of minsnap_optimize_free_constraints_soft in the tests."""
+    torch = _torch()
+    mask = np.ascontiguousarray(mask, np.uint8)
+    K = mask.shape[0] - 1
+    B, n_fixed, D = fixed_values.shape
+    dev = times.device
+    col, counts = reorder(torch.from_numpy(mask.reshape(1, -1)).to(dev), N, K)
+    n_free = int(counts[0, 1])
+    free, times = free_values.clone(), times.clone()
+    S = n_steps
+    soft_kw = dict(soft_constraint_weight=soft_constraint_weight, maximum_cost=maximum_cost, keep_small=keep_small)
+
+    def objective(f, t):
+        return free_objective_soft(mask, fixed_values, f.contiguous(), t.contiguous(), sdf, origin, resolution,
+                                   min_bound, max_bound, w_c, constraints, w_sc, w_d=w_d, w_t=w_t, N=N,
+                                   derivative=derivative, want_terms=True, **soft_kw, **map_kw)
+
+    obj0, terms0 = objective(free[:, None], times[:, None])
+    history, hit = [obj0[:, 0]], terms0["is_collision"][:, 0]
+    ladder = 0.5 ** torch.arange(S, dtype=torch.float64, device=dev)
+    rows = torch.arange(B, device=dev)
+    for _ in range(iterations):
+        dg = derivative_gradient(mask, fixed_values, free, times, N=N, derivative=derivative, want_coeffs=True,
+                                 want_diag=True)
+        cg = collision_gradient(dg["coeffs"], times, sdf, origin, resolution, min_bound, max_bound, col_of_row=col[0],
+                                n_fixed=n_fixed, n_free=n_free, **map_kw)
+        sg = soft_constraint_gradient(mask, dg["coeffs"], times, constraints, want_times=optimize_times, **soft_kw)
+        step = (w_d * dg["gradient"] + w_c * cg["gradient"] + w_sc * sg["grad_free"]) / ((2.0 * w_d) * dg["diag"][:, :, None])
+        cand_free = free[:, None] - ladder[None, :, None, None] * step[:, None]
+        if optimize_times:
+            g = time_gradient(dg["coeffs"], times, increment=gradient_increment, w_d=w_d, w_t=w_t, derivative=derivative)
+            g = g + w_sc * sg["grad_times"]
+            scale = (times / g.abs().clamp_min(1e-300)).min(1, keepdim=True).values
+            cand_t = times[:, None, :] - ((max_relative_step * ladder)[None, :, None] * scale[:, :, None]) * g[:, None, :]
+            cand_t = cand_t.clamp_min(min_time)
+        else:
+            cand_t = times[:, None, :].expand(B, S, K)
+        obj, terms = objective(cand_free, cand_t)
+        # the first minimum, as the select kernel takes it: a saturated soft term (maximum_cost) leaves the small
+        # ladder steps tied, and min(1) does not say which index it returns at a tie
+        obj = torch.where(torch.isfinite(obj), obj, torch.full_like(obj, float("inf")))
+        best = obj.min(1).values
+        arg = (obj == best[:, None]).to(torch.uint8).argmax(1)
+        improved = torch.isfinite(best) & (best < history[-1])
+        free = torch.where(improved[:, None, None], cand_free[rows, arg], free)
+        times = torch.where(improved[:, None], cand_t[rows, arg], times)
+        hit = torch.where(improved, terms["is_collision"][rows, arg], hit)
+        history.append(torch.where(improved, best, history[-1]))
+    return free, times, torch.stack(history), hit
+
+
 EXTREMA_OPTIMIZATION = 0   # PolynomialOptimization::computeMaximumOfMagnitude (ref LIN.i:470-503)
 EXTREMA_TRAJECTORY = 1     # Trajectory::computeMinMaxMagnitude (ref src/trajectory.cpp:181-217)
 EXTREMA_KEEP_SMALL_COEFFICIENTS = 16   # OR into mode: do not truncate coefficients below 2.2e-16

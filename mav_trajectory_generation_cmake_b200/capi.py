@@ -65,6 +65,14 @@ SIGNATURES = {
                                     _i, _d, _d, _d, _d, _d, _vp, _vp, _vp, _vp, _vp]),
     "minsnap_optimize_free_constraints": (_i, [_l, _i, _i, _i, _i, _vp, _vp, _vp, _vp, _i, _d, _d, _d, _vp, _vp, _vp, _d, _d,
                                                _vp, _vp, _i, _d, _d, _d, _d, _d, _i, _i, _d, _d, _d, _vp, _vp, _vp]),
+    "minsnap_soft_constraint_gradient": (_i, [_l, _i, _i, _i, _vp, _vp, _vp, _i, _vp, _vp, _d, _d, _i, _vp, _vp, _vp, _vp,
+                                              _vp, _vp, _vp]),
+    "minsnap_free_objective_soft": (_i, [_l, _i, _i, _i, _i, _i, _vp, _vp, _vp, _vp, _d, _d, _d, _vp, _vp, _vp, _d, _d, _vp,
+                                         _vp, _i, _d, _d, _d, _d, _d, _i, _vp, _vp, _d, _d, _i, _d, _vp, _vp, _vp, _vp, _vp,
+                                         _vp]),
+    "minsnap_optimize_free_constraints_soft": (_i, [_l, _i, _i, _i, _i, _vp, _vp, _vp, _vp, _i, _d, _d, _d, _vp, _vp, _vp, _d,
+                                                    _d, _vp, _vp, _i, _d, _d, _d, _d, _d, _i, _vp, _vp, _d, _d, _i, _d, _i,
+                                                    _i, _d, _d, _d, _vp, _vp, _vp, _vp]),
     "minsnap_host_alloc": (_i, [_vp, _sz]),
     "minsnap_host_free": (_i, [_vp]),
     "minsnap_reorder_host": (_i, [_i, _i, _l, _vp, _vp, _vp]),

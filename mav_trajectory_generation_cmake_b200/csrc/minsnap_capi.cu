@@ -915,14 +915,35 @@ minsnap::GeneralSolveArgs recovery_args(long B, int K, int D, int N, int derivat
   return a;
 }
 
+// The soft limits of the *_soft entries below: the constraints (shapes and pointers are set per launch), their weight
+// w_sc in J, the scratch of the per-segment maxima (soft_constraint_scratch_bytes for the largest batch) and [n] for
+// the soft cost of the candidates.
+struct SoftTerm {
+  minsnap::SoftConstraintArgs a;
+  double w_sc;
+  void* extrema;
+  double* soft;
+};
+
+// The soft cost of n recovered trajectories, with their maxima (d_max_value, optional) and the scratch left for
+// launch_soft_constraint_gradient.
+cudaError_t launch_soft_term(const SoftTerm& t, long n, int K, int D, int N, const double* coeffs, const double* times,
+                             double* d_soft, double* d_max_value, cudaStream_t st) {
+  minsnap::SoftConstraintArgs a = t.a;
+  a.B = n; a.K = K; a.D = D; a.N = N;
+  a.d_coeffs = coeffs; a.d_times = times; a.d_scratch = t.extrema;
+  a.d_soft = d_soft; a.d_terms = nullptr; a.d_max_value = d_max_value;
+  return minsnap::launch_soft_constraint_cost(a, st);
+}
+
 // minsnap_free_objective on the device, the index map already built: recovery of the B*S candidates (fixed values
-// shared by the S candidates of a trajectory), the collision walk, the combine kernel.  Scratch: coeffs
-// [B*S][K][D][N], cost and jc [B*S].
+// shared by the S candidates of a trajectory), the collision walk, the combine kernel; with a soft term, its soft cost
+// on the recovered coefficients, added last with weight w_sc.  Scratch: coeffs [B*S][K][D][N], cost and jc [B*S].
 int free_objective_device(long B, int S, int K, int D, int N, int derivative, int n_fixed, int n_free,
                           const int32_t* d_col_of_row, const double* d_fixed_values, const double* d_free_values,
                           const double* d_times, double w_d, double w_c, double w_t, const CollisionMap& map,
                           double* d_objective, double* d_Jd, double* d_jc, int32_t* d_is_collision, double* coeffs,
-                          double* cost, cudaStream_t st) {
+                          double* cost, cudaStream_t st, const SoftTerm* soft = nullptr) {
   const long n = B * S;
   minsnap::GeneralSolveArgs a =
       recovery_args(n, K, D, N, derivative, n_fixed, n_free, d_col_of_row, d_fixed_values, d_free_values, d_times);
@@ -933,6 +954,10 @@ int free_objective_device(long B, int S, int K, int D, int N, int derivative, in
   const int rc = map.cost(n, K, coeffs, d_times, d_jc, d_is_collision, st);
   if (rc != MINSNAP_OK) return rc;
   CU(minsnap::launch_free_combine(n, K, cost, d_jc, d_times, w_d, w_c, w_t, d_objective, d_Jd, st));
+  if (soft) {
+    CU(launch_soft_term(*soft, n, K, D, N, coeffs, d_times, soft->soft, nullptr, st));
+    CU(minsnap::launch_free_soft_add(n, soft->soft, soft->w_sc, d_objective, st));
+  }
   return MINSNAP_OK;
 }
 
@@ -959,76 +984,94 @@ int minsnap_derivative_gradient(long B, int K, int D, int N, int derivative, con
   return MINSNAP_OK;
 }
 
-int minsnap_free_objective(long B, int S, int K, int D, int N, int derivative, const uint8_t* h_fixed_mask,
-                           const double* d_fixed_values, const double* d_free_values, const double* d_times, double w_d,
-                           double w_c, double w_t, const double* d_sdf, const int32_t* h_dims, const double* h_origin,
-                           double resolution, double oob_value, const double* h_min_bound, const double* h_max_bound,
-                           int use_continuous_distance, double dt, double map_resolution, double epsilon,
-                           double robot_radius, double coll_pot_multiplier, double* d_objective, double* d_Jd,
-                           double* d_Jc, int32_t* d_is_collision, minsnap_stream_t stream) {
+namespace {
+
+// The limit on the mask launch_reorder_host_mask packs into kernel parameters.
+bool mask_fits(int N, int K) { return (long)(K + 1) * (N / 2) <= 32L * minsnap::MaskBits::kWords; }
+
+// The soft arguments of the *_soft free-derivative entries on top of soft_args: w_sc >= 0 and finite.
+int free_soft_args(int N, int n_constraints, const int32_t* h_derivatives, const double* h_limits, double weight,
+                   double maximum_cost, int extrema_flags, double w_sc, SoftTerm* t) {
+  const int rc = soft_args(N, n_constraints, h_derivatives, h_limits, weight, maximum_cost, extrema_flags, &t->a);
+  if (rc != MINSNAP_OK) return rc;
+  if (!(w_sc >= 0.0 && std::isfinite(w_sc))) return MINSNAP_ERR_ARG;
+  t->w_sc = w_sc;
+  return MINSNAP_OK;
+}
+
+int free_objective_call(long B, int S, int K, int D, int N, int derivative, const uint8_t* h_fixed_mask,
+                        const double* d_fixed_values, const double* d_free_values, const double* d_times, double w_d,
+                        double w_c, double w_t, const CollisionMap& map, SoftTerm* soft, double* d_objective,
+                        double* d_Jd, double* d_Jc, int32_t* d_is_collision, double* d_soft, cudaStream_t st) {
   if (!shape_ok(B, K, D, N, derivative) || S < 1 || !h_fixed_mask) return MINSNAP_ERR_ARG;
-  const CollisionMap map{d_sdf, h_dims, h_origin, resolution, oob_value, h_min_bound, h_max_bound,
-                         use_continuous_distance, dt, map_resolution, epsilon, robot_radius, coll_pot_multiplier};
   int rc = map.check(B, K, D, N);
   if (rc != MINSNAP_OK) return rc;
   int n_fixed, n_free;
   count_mask(h_fixed_mask, N, K, &n_fixed, &n_free);
+  if (soft && (!mask_fits(N, K) || minsnap::general_fits(N, K, D, n_fixed, n_free) != cudaSuccess))
+    return MINSNAP_ERR_UNSUPPORTED;
   if (B == 0) return MINSNAP_OK;
-  if (!d_times || !d_sdf || !d_objective || (n_fixed > 0 && !d_fixed_values) || (n_free > 0 && !d_free_values))
+  if (!d_times || !map.sdf || !d_objective || (n_fixed > 0 && !d_fixed_values) || (n_free > 0 && !d_free_values))
     return MINSNAP_ERR_ARG;
-  cudaStream_t st = as_stream(stream);
   const size_t n = (size_t)B * S;
   const size_t ws_head = align_up(SolveWorkspace::bytes(N, K), 256);
+  const size_t n_doubles = n * ((size_t)K * D * N + 2 + (soft ? 1 : 0));
+  const size_t extrema = soft ? minsnap::soft_constraint_scratch_bytes((long)n, K, soft->a.n_constraints) : 0;
   char* ws = nullptr;
   retain_pool_memory();
-  CU(cudaMallocAsync(reinterpret_cast<void**>(&ws), ws_head + sizeof(double) * n * ((size_t)K * D * N + 2), st));
+  CU(cudaMallocAsync(reinterpret_cast<void**>(&ws), ws_head + sizeof(double) * n_doubles + extrema, st));
   SolveWorkspace sw(ws, N, K);
   double* coeffs = reinterpret_cast<double*>(ws + ws_head);
   double* cost = coeffs + n * K * D * N;
   double* jc = cost + n;
+  if (soft) {
+    soft->soft = d_soft ? d_soft : jc + n;
+    soft->extrema = jc + 2 * n;
+  }
   const cudaError_t e = minsnap::launch_reorder_host_mask(N, K, h_fixed_mask, sw.mask, sw.col_of_row, sw.counts, st);
   if (e != cudaSuccess) rc = cuda_fail(e, "launch_reorder_host_mask");
   if (rc == MINSNAP_OK)
     rc = free_objective_device(B, S, K, D, N, derivative, n_fixed, n_free, sw.col_of_row, d_fixed_values,
                                d_free_values, d_times, w_d, w_c, w_t, map, d_objective, d_Jd, jc, d_is_collision,
-                               coeffs, cost, st);
+                               coeffs, cost, st, soft);
   if (rc == MINSNAP_OK && d_Jc && cudaMemcpyAsync(d_Jc, jc, sizeof(double) * n, cudaMemcpyDeviceToDevice, st) != cudaSuccess)
     rc = MINSNAP_ERR_CUDA;
   cudaFreeAsync(ws, st);
   return rc;
 }
 
-// A batched descent on the free derivatives (and optionally the segment times) that never leaves the device: every
-// iteration is launches on `stream` only (recovery with the gradient of J_d, collision gradient, [time gradient,
-// time ladder,] candidate ladder, recovery + walk + combine of the candidates, select); the workspace is one
-// stream-ordered allocation and the mask reaches the device by value, so the call can be captured into a CUDA graph.
-int minsnap_optimize_free_constraints(long B, int K, int D, int N, int derivative, const uint8_t* h_fixed_mask,
-                                      const double* d_fixed_values, double* d_free_values, double* d_times,
-                                      int optimize_times, double w_d, double w_c, double w_t, const double* d_sdf,
-                                      const int32_t* h_dims, const double* h_origin, double resolution,
-                                      double oob_value, const double* h_min_bound, const double* h_max_bound,
-                                      int use_continuous_distance, double dt, double map_resolution, double epsilon,
-                                      double robot_radius, double coll_pot_multiplier, int iterations, int n_steps,
-                                      double max_relative_step, double min_time, double gradient_increment,
-                                      double* d_history, int32_t* d_is_collision, minsnap_stream_t stream) {
+// The descent of minsnap_optimize_free_constraints; with a soft term (minsnap_optimize_free_constraints_soft) its
+// gradient joins the step and the time gradient, and its cost the objective.
+int free_descent(long B, int K, int D, int N, int derivative, const uint8_t* h_fixed_mask, const double* d_fixed_values,
+                 double* d_free_values, double* d_times, int optimize_times, double w_d, double w_c, double w_t,
+                 const CollisionMap& map, SoftTerm* soft, int iterations, int n_steps, double max_relative_step,
+                 double min_time, double gradient_increment, double* d_history, int32_t* d_is_collision,
+                 double* d_max_value, cudaStream_t st) {
   if (!shape_ok(B, K, D, N, derivative) || !h_fixed_mask || iterations < 0 || n_steps < 1 || !(w_d > 0.0) ||
       !(max_relative_step > 0.0) || !(min_time > 0.0) || !(gradient_increment > 0.0))
     return MINSNAP_ERR_ARG;
-  const CollisionMap map{d_sdf, h_dims, h_origin, resolution, oob_value, h_min_bound, h_max_bound,
-                         use_continuous_distance, dt, map_resolution, epsilon, robot_radius, coll_pot_multiplier};
   int rc = map.check(B, K, D, N);
   if (rc != MINSNAP_OK) return rc;
   int n_fixed, n_free;
   count_mask(h_fixed_mask, N, K, &n_fixed, &n_free);
+  if (soft && (!mask_fits(N, K) || minsnap::general_fits(N, K, D, n_fixed, n_free) != cudaSuccess))
+    return MINSNAP_ERR_UNSUPPORTED;
   if (B == 0) return MINSNAP_OK;
-  if (!d_times || !d_sdf || (n_fixed > 0 && !d_fixed_values) || (n_free > 0 && !d_free_values)) return MINSNAP_ERR_ARG;
-  cudaStream_t st = as_stream(stream);
+  if (!d_times || !map.sdf || (n_fixed > 0 && !d_fixed_values) || (n_free > 0 && !d_free_values)) return MINSNAP_ERR_ARG;
   const size_t nb = (size_t)B, S = (size_t)n_steps, nfd = (size_t)n_free * D, nc = (size_t)K * D * N;
   const size_t ws_head = align_up(SolveWorkspace::bytes(N, K), 256);
   const size_t n_doubles = nb * (nc + 2 * nfd + n_free + K + 3) + nb * S * (nfd + K + nc + 3);
+  const size_t n_ints = nb * (S + 1);
+  // soft term: g_sc [B][n_free][D], the candidates' soft cost [B S], per-segment maxima of B S trajectories
+  const size_t soft_doubles = soft ? nb * nfd + nb * S : 0;
+  const size_t soft_head = align_up(sizeof(double) * n_doubles + sizeof(int32_t) * n_ints, 256);
   char* ws = nullptr;
   retain_pool_memory();
-  CU(cudaMallocAsync(reinterpret_cast<void**>(&ws), ws_head + sizeof(double) * n_doubles + sizeof(int32_t) * nb * (S + 1), st));
+  if (soft)
+    CU(cudaMallocAsync(reinterpret_cast<void**>(&ws), ws_head + soft_head + sizeof(double) * soft_doubles +
+                       minsnap::soft_constraint_scratch_bytes((long)(nb * S), K, soft->a.n_constraints), st));
+  else
+    CU(cudaMallocAsync(reinterpret_cast<void**>(&ws), ws_head + sizeof(double) * n_doubles + sizeof(int32_t) * n_ints, st));
   SolveWorkspace sw(ws, N, K);
   double* coeffs = reinterpret_cast<double*>(ws + ws_head);   // the incumbent's
   double* grad_d = coeffs + nb * nc;
@@ -1046,12 +1089,19 @@ int minsnap_optimize_free_constraints(long B, int K, int D, int N, int derivativ
   double* cand_obj = cand_jc + nb * S;
   int32_t* cand_hit = reinterpret_cast<int32_t*>(cand_obj + nb * S);
   int32_t* hit = d_is_collision ? d_is_collision : cand_hit + nb * S;
+  double* grad_sc = nullptr;
+  if (soft) {
+    grad_sc = reinterpret_cast<double*>(ws + ws_head + soft_head);
+    soft->soft = grad_sc + nb * nfd;
+    soft->extrema = soft->soft + nb * S;
+  }
   cudaError_t e = minsnap::launch_reorder_host_mask(N, K, h_fixed_mask, sw.mask, sw.col_of_row, sw.counts, st);
   if (e != cudaSuccess) rc = cuda_fail(e, "launch_reorder_host_mask");
   // the incumbent objective at the initial state: the candidate pipeline with one candidate per trajectory
   if (rc == MINSNAP_OK)
     rc = free_objective_device(B, 1, K, D, N, derivative, n_fixed, n_free, sw.col_of_row, d_fixed_values, d_free_values,
-                               d_times, w_d, w_c, w_t, map, incumbent, nullptr, cand_jc, hit, cand_coeffs, cand_cost, st);
+                               d_times, w_d, w_c, w_t, map, incumbent, nullptr, cand_jc, hit, cand_coeffs, cand_cost, st,
+                               soft);
   if (rc == MINSNAP_OK && d_history)
     if (cudaMemcpyAsync(d_history, incumbent, sizeof(double) * nb, cudaMemcpyDeviceToDevice, st) != cudaSuccess) rc = MINSNAP_ERR_CUDA;
   for (int it = 0; it < iterations && rc == MINSNAP_OK; ++it) {
@@ -1060,26 +1110,170 @@ int minsnap_optimize_free_constraints(long B, int K, int D, int N, int derivativ
     a.d_coeffs = coeffs; a.d_cost = jd; a.d_grad_free = grad_d; a.d_diag_free = diag;
     e = minsnap::launch_derivative_gradient(a, st);
     if (e == cudaSuccess) rc = map.gradient(B, K, coeffs, d_times, sw.col_of_row, n_fixed, n_free, jc, grad_c, st);
-    if (e == cudaSuccess && rc == MINSNAP_OK && optimize_times) {
+    if (e == cudaSuccess && rc == MINSNAP_OK && optimize_times)
       rc = minsnap_time_gradient(B, K, D, N, derivative, coeffs, d_times, gradient_increment, w_d, w_t, grad_t, nullptr, st);
-      if (rc == MINSNAP_OK)
-        e = minsnap::launch_time_candidates(B, n_steps, K, d_times, grad_t, 0.0, max_relative_step, min_time, cand_times, st);
+    // the soft term at the incumbent: its maxima, then g_sc, and w_sc dsoft/dT added to the time gradient
+    if (e == cudaSuccess && rc == MINSNAP_OK && soft) {
+      e = launch_soft_term(*soft, B, K, D, N, coeffs, d_times, nullptr, nullptr, st);
+      if (e == cudaSuccess) {
+        minsnap::SoftGradientArgs g;
+        g.soft = soft->a;
+        g.soft.B = B; g.soft.K = K; g.soft.D = D; g.soft.N = N;
+        g.soft.d_coeffs = coeffs; g.soft.d_times = d_times; g.soft.d_scratch = soft->extrema;
+        g.d_col_of_row = sw.col_of_row; g.n_fixed = n_fixed; g.n_free = n_free;
+        g.d_grad_free = grad_sc;
+        g.d_grad_times = optimize_times ? grad_t : nullptr;
+        g.add_times = true;
+        g.times_weight = soft->w_sc;
+        e = minsnap::launch_soft_constraint_gradient(g, st);
+      }
     }
+    if (e == cudaSuccess && rc == MINSNAP_OK && optimize_times)
+      e = minsnap::launch_time_candidates(B, n_steps, K, d_times, grad_t, 0.0, max_relative_step, min_time, cand_times, st);
     if (e == cudaSuccess && rc == MINSNAP_OK)
       e = minsnap::launch_free_candidates(B, n_steps, n_free, D, K, d_free_values, grad_d, grad_c, diag, w_d, w_c, d_times,
-                                          cand_free, optimize_times ? nullptr : cand_times, st);
+                                          cand_free, optimize_times ? nullptr : cand_times, st, grad_sc,
+                                          soft ? soft->w_sc : 0.0);
     if (e == cudaSuccess && rc == MINSNAP_OK)
       rc = free_objective_device(B, n_steps, K, D, N, derivative, n_fixed, n_free, sw.col_of_row, d_fixed_values,
                                  cand_free, cand_times, w_d, w_c, w_t, map, cand_obj, nullptr, cand_jc, cand_hit,
-                                 cand_coeffs, cand_cost, st);
+                                 cand_coeffs, cand_cost, st, soft);
     if (e == cudaSuccess && rc == MINSNAP_OK)
       e = minsnap::launch_free_select(B, n_steps, (int)nfd, K, cand_obj, cand_free, cand_times, cand_hit, d_free_values,
                                       d_times, incumbent, hit, d_history ? d_history + (size_t)(it + 1) * nb : nullptr, st);
     if (rc == MINSNAP_OK && e != cudaSuccess) rc = cuda_fail(e, "free-constraint descent");
   }
+  // the maxima at the returned state, from its recovered coefficients
+  if (rc == MINSNAP_OK && soft && d_max_value) {
+    minsnap::GeneralSolveArgs a =
+        recovery_args(B, K, D, N, derivative, n_fixed, n_free, sw.col_of_row, d_fixed_values, d_free_values, d_times);
+    a.d_coeffs = coeffs;
+    e = minsnap::launch_coeffs_from_constraints(a, st);
+    if (e == cudaSuccess) e = launch_soft_term(*soft, B, K, D, N, coeffs, d_times, nullptr, d_max_value, st);
+    if (e != cudaSuccess) rc = cuda_fail(e, "soft-limit maxima");
+  }
   cudaFreeAsync(ws, st);
   return rc;
 }
+
+}  // namespace
+
+int minsnap_free_objective(long B, int S, int K, int D, int N, int derivative, const uint8_t* h_fixed_mask,
+                           const double* d_fixed_values, const double* d_free_values, const double* d_times, double w_d,
+                           double w_c, double w_t, const double* d_sdf, const int32_t* h_dims, const double* h_origin,
+                           double resolution, double oob_value, const double* h_min_bound, const double* h_max_bound,
+                           int use_continuous_distance, double dt, double map_resolution, double epsilon,
+                           double robot_radius, double coll_pot_multiplier, double* d_objective, double* d_Jd,
+                           double* d_Jc, int32_t* d_is_collision, minsnap_stream_t stream) {
+  const CollisionMap map{d_sdf, h_dims, h_origin, resolution, oob_value, h_min_bound, h_max_bound,
+                         use_continuous_distance, dt, map_resolution, epsilon, robot_radius, coll_pot_multiplier};
+  return free_objective_call(B, S, K, D, N, derivative, h_fixed_mask, d_fixed_values, d_free_values, d_times, w_d, w_c,
+                             w_t, map, nullptr, d_objective, d_Jd, d_Jc, d_is_collision, nullptr, as_stream(stream));
+}
+
+// A batched descent on the free derivatives (and optionally the segment times) that never leaves the device: every
+// iteration is launches on `stream` only (recovery with the gradient of J_d, collision gradient, [time gradient,
+// time ladder,] candidate ladder, recovery + walk + combine of the candidates, select); the workspace is one
+// stream-ordered allocation and the mask reaches the device by value, so the call can be captured into a CUDA graph.
+int minsnap_optimize_free_constraints(long B, int K, int D, int N, int derivative, const uint8_t* h_fixed_mask,
+                                      const double* d_fixed_values, double* d_free_values, double* d_times,
+                                      int optimize_times, double w_d, double w_c, double w_t, const double* d_sdf,
+                                      const int32_t* h_dims, const double* h_origin, double resolution,
+                                      double oob_value, const double* h_min_bound, const double* h_max_bound,
+                                      int use_continuous_distance, double dt, double map_resolution, double epsilon,
+                                      double robot_radius, double coll_pot_multiplier, int iterations, int n_steps,
+                                      double max_relative_step, double min_time, double gradient_increment,
+                                      double* d_history, int32_t* d_is_collision, minsnap_stream_t stream) {
+  const CollisionMap map{d_sdf, h_dims, h_origin, resolution, oob_value, h_min_bound, h_max_bound,
+                         use_continuous_distance, dt, map_resolution, epsilon, robot_radius, coll_pot_multiplier};
+  return free_descent(B, K, D, N, derivative, h_fixed_mask, d_fixed_values, d_free_values, d_times, optimize_times, w_d,
+                      w_c, w_t, map, nullptr, iterations, n_steps, max_relative_step, min_time, gradient_increment,
+                      d_history, d_is_collision, nullptr, as_stream(stream));
+}
+
+// ---------------------------------------------------------------------------------------
+// The soft limits of minsnap_soft_constraint_cost in the free-derivative problem: their analytic gradient, the
+// objective J + w_sc soft and the descent on it
+// ---------------------------------------------------------------------------------------
+int minsnap_soft_constraint_gradient(long B, int K, int D, int N, const uint8_t* h_fixed_mask, const double* d_coeffs,
+                                     const double* d_times, int n_constraints, const int32_t* h_derivatives,
+                                     const double* h_limits, double weight, double maximum_cost, int extrema_flags,
+                                     double* d_cost, double* d_grad_free, double* d_grad_times, double* d_max_value,
+                                     double* d_max_time, int32_t* d_max_segment, minsnap_stream_t stream) {
+  if (B < 0 || K < 1 || D < 1 || D > 32 || !minsnap::supported_n(N) || !h_fixed_mask) return MINSNAP_ERR_ARG;
+  SoftTerm t;
+  int rc = free_soft_args(N, n_constraints, h_derivatives, h_limits, weight, maximum_cost, extrema_flags, 0.0, &t);
+  if (rc != MINSNAP_OK) return rc;
+  if (!mask_fits(N, K)) return MINSNAP_ERR_UNSUPPORTED;
+  int n_fixed, n_free;
+  count_mask(h_fixed_mask, N, K, &n_fixed, &n_free);
+  if (B == 0) return MINSNAP_OK;
+  if (!d_coeffs || !d_times || (n_free > 0 && !d_grad_free)) return MINSNAP_ERR_ARG;
+  cudaStream_t st = as_stream(stream);
+  const size_t ws_head = align_up(SolveWorkspace::bytes(N, K), 256);
+  char* ws = nullptr;
+  retain_pool_memory();
+  CU(cudaMallocAsync(reinterpret_cast<void**>(&ws), ws_head + minsnap::soft_constraint_scratch_bytes(B, K, n_constraints),
+                     st));
+  SolveWorkspace sw(ws, N, K);
+  t.extrema = ws + ws_head;
+  cudaError_t e = minsnap::launch_reorder_host_mask(N, K, h_fixed_mask, sw.mask, sw.col_of_row, sw.counts, st);
+  if (e == cudaSuccess) e = launch_soft_term(t, B, K, D, N, d_coeffs, d_times, d_cost, d_max_value, st);
+  if (e == cudaSuccess) {
+    minsnap::SoftGradientArgs g;
+    g.soft = t.a;
+    g.soft.B = B; g.soft.K = K; g.soft.D = D; g.soft.N = N;
+    g.soft.d_coeffs = d_coeffs; g.soft.d_times = d_times; g.soft.d_scratch = t.extrema;
+    g.d_col_of_row = sw.col_of_row; g.n_fixed = n_fixed; g.n_free = n_free;
+    g.d_grad_free = d_grad_free; g.d_grad_times = d_grad_times;
+    g.d_max_time = d_max_time; g.d_max_segment = d_max_segment;
+    e = minsnap::launch_soft_constraint_gradient(g, st);
+  }
+  if (e != cudaSuccess) rc = cuda_fail(e, "soft-limit gradient");
+  cudaFreeAsync(ws, st);
+  return rc;
+}
+
+int minsnap_free_objective_soft(long B, int S, int K, int D, int N, int derivative, const uint8_t* h_fixed_mask,
+                                const double* d_fixed_values, const double* d_free_values, const double* d_times,
+                                double w_d, double w_c, double w_t, const double* d_sdf, const int32_t* h_dims,
+                                const double* h_origin, double resolution, double oob_value, const double* h_min_bound,
+                                const double* h_max_bound, int use_continuous_distance, double dt, double map_resolution,
+                                double epsilon, double robot_radius, double coll_pot_multiplier, int n_constraints,
+                                const int32_t* h_derivatives, const double* h_limits, double weight,
+                                double maximum_cost, int extrema_flags, double w_sc, double* d_objective, double* d_Jd,
+                                double* d_Jc, int32_t* d_is_collision, double* d_soft, minsnap_stream_t stream) {
+  SoftTerm t;
+  const int rc = free_soft_args(N, n_constraints, h_derivatives, h_limits, weight, maximum_cost, extrema_flags, w_sc, &t);
+  if (rc != MINSNAP_OK) return rc;
+  const CollisionMap map{d_sdf, h_dims, h_origin, resolution, oob_value, h_min_bound, h_max_bound,
+                         use_continuous_distance, dt, map_resolution, epsilon, robot_radius, coll_pot_multiplier};
+  return free_objective_call(B, S, K, D, N, derivative, h_fixed_mask, d_fixed_values, d_free_values, d_times, w_d, w_c,
+                             w_t, map, &t, d_objective, d_Jd, d_Jc, d_is_collision, d_soft, as_stream(stream));
+}
+
+int minsnap_optimize_free_constraints_soft(long B, int K, int D, int N, int derivative, const uint8_t* h_fixed_mask,
+                                           const double* d_fixed_values, double* d_free_values, double* d_times,
+                                           int optimize_times, double w_d, double w_c, double w_t, const double* d_sdf,
+                                           const int32_t* h_dims, const double* h_origin, double resolution,
+                                           double oob_value, const double* h_min_bound, const double* h_max_bound,
+                                           int use_continuous_distance, double dt, double map_resolution,
+                                           double epsilon, double robot_radius, double coll_pot_multiplier,
+                                           int n_constraints, const int32_t* h_derivatives, const double* h_limits,
+                                           double weight, double maximum_cost, int extrema_flags, double w_sc,
+                                           int iterations, int n_steps, double max_relative_step, double min_time,
+                                           double gradient_increment, double* d_history, int32_t* d_is_collision,
+                                           double* d_max_value, minsnap_stream_t stream) {
+  SoftTerm t;
+  const int rc = free_soft_args(N, n_constraints, h_derivatives, h_limits, weight, maximum_cost, extrema_flags, w_sc, &t);
+  if (rc != MINSNAP_OK) return rc;
+  const CollisionMap map{d_sdf, h_dims, h_origin, resolution, oob_value, h_min_bound, h_max_bound,
+                         use_continuous_distance, dt, map_resolution, epsilon, robot_radius, coll_pot_multiplier};
+  return free_descent(B, K, D, N, derivative, h_fixed_mask, d_fixed_values, d_free_values, d_times, optimize_times, w_d,
+                      w_c, w_t, map, &t, iterations, n_steps, max_relative_step, min_time, gradient_increment, d_history,
+                      d_is_collision, d_max_value, as_stream(stream));
+}
+
 
 // ---------------------------------------------------------------------------------------
 // Host-buffer entry points

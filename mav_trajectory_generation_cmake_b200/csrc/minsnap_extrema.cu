@@ -407,6 +407,119 @@ __global__ void __launch_bounds__(128) soft_constraint_fold_kernel(SoftFoldParam
   }
 }
 
+struct SoftGradientParams {
+  long B;
+  int K, D, n_constraints, n_fixed, n_free;
+  int derivative[kMaxSoftConstraints];
+  double limit[kMaxSoftConstraints];
+  double weight, maximum_cost;
+  const SegmentExtremum* per_segment;  // [n_constraints][B][K], as launch_soft_constraint_cost left it
+  const double* coeffs;                // [B][K][D][N]
+  const double* times;                 // [B][K]
+  const int32_t* col_of_row;           // [N K]
+  double* grad_free;                   // [B][n_free][D], or null when n_free == 0
+  double* grad_times;                  // optional [B][K]
+  bool add_times;                      // grad_times += times_weight g_T instead of grad_times = g_T
+  double times_weight;
+  double* max_time;                    // optional [B][n_constraints]
+  int32_t* max_segment;                // optional [B][n_constraints]
+};
+
+// Gradient of the soft cost in the free derivatives and in the segment times with the end-point derivatives d held
+// fixed.  One warp per trajectory.  Each constraint's argmax (segment s*, time t*) is folded from its per-segment
+// maxima with the comparisons of fold_extrema_kernel, so ties go to the first strict maximum (a subgradient).  With
+// x = exp((m - L) / L weight), dtau/dm = x weight / L below maximum_cost and 0 when saturated or at m = 0.  Every
+// mode-0 candidate is a stationary point of m^2 in t or a segment start, so (envelope theorem) dm/dtheta is taken at
+// fixed t*: sum_dim p_dim^(k)(t*) dp_dim^(k)(t*)/dtheta / m, plus the drift sum_dim p^(k) p^(k+1)(T) / m when t* is
+// the end of the last segment and theta is its time.  With c = A^-1(T) d_seg, u = t*/T and k_r the derivative order
+// of end-point row r:
+//   dp^(k)(t*)/dd_r = T^(k_r - k)     sum_n b(k, n) u^(n-k) A1inv[n][r]
+//   dp^(k)(t*)/dT   = sum_r d_r T^(k_r - k - 1) sum_n b(k, n) u^(n-k) (k_r - n) A1inv[n][r]
+// Lanes run over (row, dimension) of s*; row r lands on its free column through col_of_row (fixed rows drop out).
+// The constraints add in constraint order, each free entry on one lane and each time on one lane: no atomics.
+template <int N>
+__global__ void __launch_bounds__(128) soft_constraint_gradient_kernel(SoftGradientParams p) {
+  constexpr int h = N / 2;
+  const int lane = threadIdx.x & 31;
+  const long warps = (long)gridDim.x * (blockDim.x / 32);
+  const double* A1inv = UnitTables<N>::a1inv();
+  const long nfd = (long)p.n_free * p.D;
+  for (long b = (long)blockIdx.x * (blockDim.x / 32) + uniform_warp_index(); b < p.B; b += warps) {
+    double* gf = p.grad_free ? p.grad_free + b * nfd : nullptr;
+    if (gf)
+      for (long j = lane; j < nfd; j += 32) gf[j] = 0.0;
+    // lane c keeps constraint c's segment s* and its time derivative
+    int my_seg = -1;
+    double my_gt = 0.0;
+    for (int c = 0; c < p.n_constraints; ++c) {
+      __syncwarp();   // this constraint's additions to the free columns see the zeroing and the previous constraints'
+      const SegmentExtremum* e = p.per_segment + ((long)c * p.B + b) * p.K;
+      double max_v = 0.0, max_t = 0.0;
+      int max_s = 0;
+      for (int s = 0; s < p.K; ++s) {
+        const SegmentExtremum x = e[s];
+        if (x.max_v > max_v) { max_v = x.max_v; max_t = x.max_t; max_s = s; }
+      }
+      if (lane == 0) {
+        if (p.max_time) p.max_time[b * p.n_constraints + c] = max_t;
+        if (p.max_segment) p.max_segment[b * p.n_constraints + c] = max_s;
+      }
+      const int k = p.derivative[c];
+      const double L = p.limit[c];
+      const double x = exp(__dmul_rn(__ddiv_rn(__dsub_rn(max_v, L), L), p.weight));
+      const double dtau_over_m = (x < p.maximum_cost && max_v > 0.0) ? x * p.weight / L / max_v : 0.0;
+      if (lane == c) my_seg = max_s;
+      if (dtau_over_m == 0.0) continue;
+      const long si = b * p.K + max_s;
+      const double T = p.times[si];
+      const double* seg = p.coeffs + si * p.D * N;
+      const double u = max_t / T;
+      const bool drift = max_s == p.K - 1 && max_t == T;
+      double acc_t = 0.0;
+      for (int q = lane; q < N * p.D; q += 32) {
+        const int r = q / p.D, dim = q - r * p.D;
+        const int kr = r % h;
+        const double* cd = seg + dim * N;
+        const double w = dtau_over_m * evaluate_derivative(cd, N, k, max_t);   // dtau/dm p_dim^(k)(t*) / m
+        double bd = 0.0, bt = 0.0, up = 1.0;
+        for (int n = k; n < N; ++n) {
+          const double f = falling_factorial(k, n) * up * A1inv[n * N + r];
+          bd += f;
+          bt += (double)(kr - n) * f;
+          up *= u;
+        }
+        const double Tp = int_power(T, kr - k);
+        if (gf) {
+          const int col = p.col_of_row[max_s * N + r] - p.n_fixed;
+          if (col >= 0) gf[col * p.D + dim] += w * (bd * Tp);
+        }
+        if (p.grad_times) {
+          acc_t += w * evaluate_derivative(cd, N, kr, r < h ? 0.0 : T) * (bt * Tp / T);
+          if (drift && r == 0) acc_t += w * evaluate_derivative(cd, N, k + 1, T);
+        }
+      }
+      if (p.grad_times) {
+        acc_t = warp_sum(acc_t);
+        if (lane == c) my_gt = acc_t;
+      }
+    }
+    if (p.grad_times) {
+      for (int s0 = 0; s0 < p.K; s0 += 32) {
+        const int s = s0 + lane;
+        double g = 0.0;
+        for (int c = 0; c < p.n_constraints; ++c) {
+          const int sc = __shfl_sync(0xffffffffu, my_seg, c);
+          const double gc = __shfl_sync(0xffffffffu, my_gt, c);
+          if (sc == s) g += gc;
+        }
+        if (s >= p.K) continue;
+        double* dst = p.grad_times + b * p.K + s;
+        *dst = p.add_times ? __dadd_rn(*dst, __dmul_rn(p.times_weight, g)) : g;
+      }
+    }
+  }
+}
+
 template <int LEN>
 cudaError_t launch_segments(const ExtremaParams& p, cudaStream_t stream) {
   const long n = p.B * p.K;
@@ -501,6 +614,34 @@ cudaError_t launch_soft_constraint_cost(const SoftConstraintArgs& a, cudaStream_
   f.objective = a.d_objective; f.cost = a.d_cost; f.status = a.d_status; f.times = a.d_times;
   f.time_penalty = a.time_penalty;
   soft_constraint_fold_kernel<<<(unsigned)((a.B + 127) / 128), 128, 0, stream>>>(f);
+  return cudaGetLastError();
+}
+
+cudaError_t launch_soft_constraint_gradient(const SoftGradientArgs& a, cudaStream_t stream) {
+  const SoftConstraintArgs& s = a.soft;
+  if (s.B == 0) return cudaSuccess;
+  SoftGradientParams p;
+  p.B = s.B; p.K = s.K; p.D = s.D; p.n_constraints = s.n_constraints; p.n_fixed = a.n_fixed; p.n_free = a.n_free;
+  for (int c = 0; c < kMaxSoftConstraints; ++c) {
+    p.derivative[c] = c < s.n_constraints ? s.derivative[c] : 0;
+    p.limit[c] = c < s.n_constraints ? s.limit[c] : 0.0;
+  }
+  p.weight = s.weight; p.maximum_cost = s.maximum_cost;
+  p.per_segment = static_cast<const SegmentExtremum*>(s.d_scratch);
+  p.coeffs = s.d_coeffs; p.times = s.d_times; p.col_of_row = a.d_col_of_row;
+  p.grad_free = a.n_free > 0 ? a.d_grad_free : nullptr;
+  p.grad_times = a.d_grad_times; p.add_times = a.add_times; p.times_weight = a.times_weight;
+  p.max_time = a.d_max_time; p.max_segment = a.d_max_segment;
+  long grid = (s.B + 3) / 4;
+  if (grid > sm_count() * 32) grid = sm_count() * 32;
+  switch (s.N) {
+    case 4: soft_constraint_gradient_kernel<4><<<(unsigned)grid, 128, 0, stream>>>(p); break;
+    case 6: soft_constraint_gradient_kernel<6><<<(unsigned)grid, 128, 0, stream>>>(p); break;
+    case 8: soft_constraint_gradient_kernel<8><<<(unsigned)grid, 128, 0, stream>>>(p); break;
+    case 10: soft_constraint_gradient_kernel<10><<<(unsigned)grid, 128, 0, stream>>>(p); break;
+    case 12: soft_constraint_gradient_kernel<12><<<(unsigned)grid, 128, 0, stream>>>(p); break;
+    default: return cudaErrorInvalidValue;
+  }
   return cudaGetLastError();
 }
 

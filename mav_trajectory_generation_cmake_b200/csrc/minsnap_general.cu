@@ -733,6 +733,8 @@ cudaError_t launch_time_select(long B, int S, int K, const double* d_cand, const
 // cand_free[b][s][j] = d_p[b][j] - 2^-s (w_d g_d[b][j] + w_c g_c[b][j]) / (2 w_d diag[b][j / D]): a Jacobi-scaled
 // step, in the units of each free derivative.  Every operation is rounded on its own (no contraction), the sequence
 // an elementwise torch version of the step performs.  cand_times (optional) [b][s] = times[b]: the times stay.
+// kSoft: the numerator is (w_d g_d + w_c g_c) + w_sc g_sc, with the soft cost's gradient g_sc.
+template <bool kSoft>
 __global__ void __launch_bounds__(256) free_candidates_kernel(long B, int S, int n_fd, int D, int K,
                                                               const double* __restrict__ free_values,
                                                               const double* __restrict__ grad_d,
@@ -740,7 +742,8 @@ __global__ void __launch_bounds__(256) free_candidates_kernel(long B, int S, int
                                                               const double* __restrict__ diag, double w_d, double w_c,
                                                               const double* __restrict__ times,
                                                               double* __restrict__ cand_free,
-                                                              double* __restrict__ cand_times) {
+                                                              double* __restrict__ cand_times,
+                                                              const double* __restrict__ grad_sc, double w_sc) {
   const long n_free_total = B * S * n_fd;
   const long total = n_free_total + (cand_times ? B * S * K : 0);
   for (long idx = (long)blockIdx.x * blockDim.x + threadIdx.x; idx < total; idx += (long)gridDim.x * blockDim.x) {
@@ -750,7 +753,8 @@ __global__ void __launch_bounds__(256) free_candidates_kernel(long B, int S, int
       const long b = bs / S;
       const int s = (int)(bs - b * S);
       const long g = b * n_fd + j;
-      const double num = __dadd_rn(__dmul_rn(w_d, grad_d[g]), __dmul_rn(w_c, grad_c[g]));
+      double num = __dadd_rn(__dmul_rn(w_d, grad_d[g]), __dmul_rn(w_c, grad_c[g]));
+      if constexpr (kSoft) num = __dadd_rn(num, __dmul_rn(w_sc, grad_sc[g]));
       const double step = __ddiv_rn(num, __dmul_rn(2.0 * w_d, diag[b * (n_fd / D) + j / D]));
       cand_free[idx] = __dsub_rn(free_values[g], __dmul_rn(ldexp(1.0, -s), step));
     } else {
@@ -810,13 +814,33 @@ __global__ void __launch_bounds__(128) free_select_kernel(long B, int S, int n_f
 cudaError_t launch_free_candidates(long B, int S, int n_free, int D, int K, const double* d_free, const double* d_grad_d,
                                    const double* d_grad_c, const double* d_diag, double w_d, double w_c,
                                    const double* d_times, double* d_cand_free, double* d_cand_times,
-                                   cudaStream_t stream) {
+                                   cudaStream_t stream, const double* d_grad_sc, double w_sc) {
   const long total = B * S * ((long)n_free * D + (d_cand_times ? K : 0));
   if (total == 0) return cudaSuccess;
   long grid = (total + 255) / 256;
   if (grid > sm_count() * 32) grid = sm_count() * 32;
-  free_candidates_kernel<<<(int)grid, 256, 0, stream>>>(B, S, n_free * D, D, K, d_free, d_grad_d, d_grad_c, d_diag, w_d,
-                                                        w_c, d_times, d_cand_free, d_cand_times);
+  if (d_grad_sc)
+    free_candidates_kernel<true><<<(int)grid, 256, 0, stream>>>(B, S, n_free * D, D, K, d_free, d_grad_d, d_grad_c,
+                                                                d_diag, w_d, w_c, d_times, d_cand_free, d_cand_times,
+                                                                d_grad_sc, w_sc);
+  else
+    free_candidates_kernel<false><<<(int)grid, 256, 0, stream>>>(B, S, n_free * D, D, K, d_free, d_grad_d, d_grad_c,
+                                                                 d_diag, w_d, w_c, d_times, d_cand_free, d_cand_times,
+                                                                 nullptr, 0.0);
+  return cudaGetLastError();
+}
+
+// objective[i] += w_sc soft[i], rounded on its own: the soft term is added last
+__global__ void __launch_bounds__(256) free_soft_add_kernel(long n, const double* __restrict__ soft, double w_sc,
+                                                            double* __restrict__ objective) {
+  const long i = (long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  objective[i] = __dadd_rn(objective[i], __dmul_rn(w_sc, soft[i]));
+}
+
+cudaError_t launch_free_soft_add(long n, const double* d_soft, double w_sc, double* d_objective, cudaStream_t stream) {
+  if (n == 0) return cudaSuccess;
+  free_soft_add_kernel<<<(unsigned)((n + 255) / 256), 256, 0, stream>>>(n, d_soft, w_sc, d_objective);
   return cudaGetLastError();
 }
 

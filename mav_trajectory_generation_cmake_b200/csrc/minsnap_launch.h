@@ -88,10 +88,12 @@ cudaError_t launch_time_select(long B, int S, int K, const double* d_cand, const
 cudaError_t launch_free_candidates(long B, int S, int n_free, int D, int K, const double* d_free, const double* d_grad_d,
                                    const double* d_grad_c, const double* d_diag, double w_d, double w_c,
                                    const double* d_times, double* d_cand_free, double* d_cand_times,
-                                   cudaStream_t stream);
+                                   cudaStream_t stream, const double* d_grad_sc = nullptr, double w_sc = 0.0);
 cudaError_t launch_free_combine(long n, int K, const double* d_cost, const double* d_jc, const double* d_times,
                                 double w_d, double w_c, double w_t, double* d_objective, double* d_jd,
                                 cudaStream_t stream);
+// objective[i] += w_sc soft[i] (minsnap_free_objective_soft: the soft term added last)
+cudaError_t launch_free_soft_add(long n, const double* d_soft, double w_sc, double* d_objective, cudaStream_t stream);
 cudaError_t launch_free_select(long B, int S, int n_fd, int K, const double* d_cand_obj, const double* d_cand_free,
                                const double* d_cand_times, const int32_t* d_cand_hit, double* d_free, double* d_times,
                                double* d_incumbent, int32_t* d_hit, double* d_history_row, cudaStream_t stream);
@@ -212,6 +214,21 @@ struct SoftConstraintArgs {
 };
 size_t soft_constraint_scratch_bytes(long B, int K, int n_constraints);
 cudaError_t launch_soft_constraint_cost(const SoftConstraintArgs& a, cudaStream_t stream);
+
+// The soft cost's gradient in the free derivatives and in the segment times (d held fixed), from the per-segment
+// maxima launch_soft_constraint_cost left in soft.d_scratch for the same coefficients and times.
+struct SoftGradientArgs {
+  SoftConstraintArgs soft;
+  const int32_t* d_col_of_row;   // [N K] constraint index map
+  int n_fixed, n_free;
+  double* d_grad_free;           // [B][n_free][D]
+  double* d_grad_times;          // optional [B][K]
+  bool add_times = false;        // d_grad_times += times_weight g_T instead of d_grad_times = g_T
+  double times_weight = 1.0;
+  double* d_max_time = nullptr;  // optional [B][n_constraints]
+  int32_t* d_max_segment = nullptr;
+};
+cudaError_t launch_soft_constraint_gradient(const SoftGradientArgs& a, cudaStream_t stream);
 
 // ---- minsnap_collision.cu ---------------------------------------------------------------
 // SURVEY 8(f)3 (ref getCostAndGradientCollision NL.i:1523-1709): collision cost against a dense distance grid
