@@ -32,6 +32,13 @@ int cuda_fail(cudaError_t e, const char* what) {
     if (e__ != cudaSuccess) return cuda_fail(e__, #call); \
   } while (0)
 
+// returns the MINSNAP_* code of a step that fails
+#define RC(call)                            \
+  do {                                      \
+    const int rc__ = (call);                \
+    if (rc__ != MINSNAP_OK) return rc__;    \
+  } while (0)
+
 inline cudaStream_t as_stream(minsnap_stream_t s) { return static_cast<cudaStream_t>(s); }
 
 inline size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
@@ -57,6 +64,11 @@ bool shape_ok(long B, int K, int D, int N, int derivative) {
   return B >= 0 && K >= 1 && D >= 1 && minsnap::supported_n(N) && derivative >= 0 && derivative <= N / 2 - 1;
 }
 
+// The parameters of the step ladder the descents share.
+bool descent_ok(int iterations, int n_steps, double max_relative_step, double min_time, double gradient_increment) {
+  return iterations >= 0 && n_steps >= 1 && max_relative_step > 0.0 && min_time > 0.0 && gradient_increment > 0.0;
+}
+
 void count_mask(const uint8_t* mask, int N, int K, int* n_fixed, int* n_free) {
   int f = 0;
   const int nc = (K + 1) * (N / 2);
@@ -80,6 +92,31 @@ void retain_pool_memory() {
   if (cudaDeviceGetDefaultMemPool(&pool, dev) != cudaSuccess) return;
   uint64_t threshold = ~0ull;
   cudaMemPoolSetAttribute(pool, cudaMemPoolAttrReleaseThreshold, &threshold);
+}
+
+// The regions of one device block, each max(bytes, 16) rounded up to 256 bytes.  A layout takes every region in
+// order; run without a base it only counts the bytes, so a block's size and its pointers come from the same code.
+struct Regions {
+  char* base = nullptr;
+  size_t bytes = 0;
+  template <typename T>
+  T* take(size_t count) {
+    T* p = base ? reinterpret_cast<T*>(base + bytes) : nullptr;
+    bytes += align_up(std::max(sizeof(T) * count, size_t(16)), 256);
+    return p;
+  }
+};
+
+// The one stream-ordered allocation of a call, carved by `layout`; `buf` frees it on `st` on every return path.
+template <typename Layout>
+int alloc_scratch(minsnap::AsyncBuffer& buf, cudaStream_t st, Layout&& layout) {
+  Regions size;
+  layout(size);
+  retain_pool_memory();
+  CU(buf.alloc(size.bytes, st));
+  Regions at{static_cast<char*>(buf.ptr)};
+  layout(at);
+  return MINSNAP_OK;
 }
 
 // ---------------------------------------------------------------------------------------
@@ -206,11 +243,16 @@ class HostCall {
       for (auto& b : ins_)
         if (b.host && b.bytes) std::memcpy(g_arena.h + b.off, b.host, b.bytes);
       if (in_end_ > 0) CU(cudaMemcpyAsync(g_arena.d, g_arena.h, in_end_, cudaMemcpyHostToDevice, st_));
-      const int rc = launch(st_);
+      int rc = launch(st_);
+      if (rc == MINSNAP_OK && out_end_ > in_end_) {
+        const cudaError_t e =
+            cudaMemcpyAsync(g_arena.h + in_end_, g_arena.d + in_end_, out_end_ - in_end_, cudaMemcpyDeviceToHost, st_);
+        if (e != cudaSuccess) rc = cuda_fail(e, "cudaMemcpyAsync(D2H)");
+      }
+      // on every path: the next call on this thread overwrites the arena, and ensure() may free it
+      const cudaError_t es = cudaStreamSynchronize(st_);
+      if (rc == MINSNAP_OK && es != cudaSuccess) rc = cuda_fail(es, "cudaStreamSynchronize");
       if (rc != MINSNAP_OK) return rc;
-      if (out_end_ > in_end_)
-        CU(cudaMemcpyAsync(g_arena.h + in_end_, g_arena.d + in_end_, out_end_ - in_end_, cudaMemcpyDeviceToHost, st_));
-      CU(cudaStreamSynchronize(st_));
       for (auto& b : outs_)
         if (b.host && b.bytes) std::memcpy(b.host, g_arena.h + b.off, b.bytes);
       return MINSNAP_OK;
@@ -513,9 +555,7 @@ int minsnap_time_objective(long B, int S, int K, int D, int N, int derivative, c
   if (!d_positions || !d_times || !d_objective) return MINSNAP_ERR_ARG;
   // the cost lands in d_cost when given, else in d_objective, and is completed in place
   double* cost = d_cost ? d_cost : d_objective;
-  const int rc = minsnap_cost_sweep(B, S, K, D, N, derivative, d_positions, d_end_derivatives, d_times, cost, d_status,
-                                    stream);
-  if (rc != MINSNAP_OK) return rc;
+  RC(minsnap_cost_sweep(B, S, K, D, N, derivative, d_positions, d_end_derivatives, d_times, cost, d_status, stream));
   CU(minsnap::launch_add_time_penalty(B * S, K, d_times, cost, time_penalty, d_objective, as_stream(stream)));
   return MINSNAP_OK;
 }
@@ -538,45 +578,39 @@ int minsnap_optimize_segment_times(long B, int K, int D, int N, int derivative, 
                                    const double* d_end_derivatives, double* d_times, int iterations, double time_penalty,
                                    int n_steps, double max_relative_step, double min_time, double gradient_increment,
                                    double* d_history, minsnap_stream_t stream) {
-  if (!shape_ok(B, K, D, N, derivative) || iterations < 0 || n_steps < 1 || !(max_relative_step > 0.0) ||
-      !(min_time > 0.0) || !(gradient_increment > 0.0))
+  if (!shape_ok(B, K, D, N, derivative) ||
+      !descent_ok(iterations, n_steps, max_relative_step, min_time, gradient_increment))
     return MINSNAP_ERR_ARG;
   if (B == 0) return MINSNAP_OK;
   if (!d_positions || !d_times) return MINSNAP_ERR_ARG;
   if (!minsnap::standard_supported(K, D, N, derivative)) return MINSNAP_ERR_UNSUPPORTED;
   cudaStream_t st = as_stream(stream);
   const size_t nb = (size_t)B, S = (size_t)n_steps;
-  const size_t n_coeffs = nb * K * D * N, n_grad = nb * K, n_cand = nb * S * K, n_cost = nb * S;
-  double* ws = nullptr;
-  retain_pool_memory();
-  CU(cudaMallocAsync(reinterpret_cast<void**>(&ws), sizeof(double) * (n_coeffs + n_grad + n_cand + n_cost + nb), st));
-  double* coeffs = ws;
-  double* grad = coeffs + n_coeffs;
-  double* cand = grad + n_grad;
-  double* cost = cand + n_cand;
-  double* incumbent = cost + n_cost;
-  int rc = MINSNAP_OK;
+  double *coeffs, *grad, *cand, *cost, *incumbent;
+  minsnap::AsyncBuffer ws;
+  RC(alloc_scratch(ws, st, [&](Regions& r) {
+    coeffs = r.take<double>(nb * K * D * N);
+    grad = r.take<double>(nb * K);
+    cand = r.take<double>(nb * S * K);
+    cost = r.take<double>(nb * S);
+    incumbent = r.take<double>(nb);
+  }));
   // the incumbent objective at the initial times: one allocation per trajectory through the same sweep + penalty
-  rc = minsnap_time_objective(B, 1, K, D, N, derivative, d_positions, d_end_derivatives, d_times, time_penalty, incumbent,
-                              nullptr, nullptr, st);
-  if (rc == MINSNAP_OK && d_history)
-    if (cudaMemcpyAsync(d_history, incumbent, sizeof(double) * nb, cudaMemcpyDeviceToDevice, st) != cudaSuccess) rc = MINSNAP_ERR_CUDA;
-  for (int it = 0; it < iterations && rc == MINSNAP_OK; ++it) {
-    rc = minsnap_solve_standard(B, K, D, N, derivative, d_positions, d_end_derivatives, d_times, 0.0, 0.0, 0.0, nullptr,
-                                coeffs, nullptr, nullptr, nullptr, st);
+  RC(minsnap_time_objective(B, 1, K, D, N, derivative, d_positions, d_end_derivatives, d_times, time_penalty, incumbent,
+                            nullptr, nullptr, st));
+  if (d_history) CU(cudaMemcpyAsync(d_history, incumbent, sizeof(double) * nb, cudaMemcpyDeviceToDevice, st));
+  for (int it = 0; it < iterations; ++it) {
+    RC(minsnap_solve_standard(B, K, D, N, derivative, d_positions, d_end_derivatives, d_times, 0.0, 0.0, 0.0, nullptr,
+                              coeffs, nullptr, nullptr, nullptr, st));
     // d cost / dT = 0.5 dJ_d/dT (w_d = 0.5, w_t = 0); the penalty's gradient is added by the ladder kernel
-    if (rc == MINSNAP_OK) rc = minsnap_time_gradient(B, K, D, N, derivative, coeffs, d_times, gradient_increment, 0.5, 0.0, grad, nullptr, st);
-    cudaError_t e = cudaSuccess;
-    if (rc == MINSNAP_OK) e = minsnap::launch_time_candidates(B, n_steps, K, d_times, grad, time_penalty, max_relative_step, min_time, cand, st);
-    if (rc == MINSNAP_OK && e == cudaSuccess)
-      rc = minsnap_cost_sweep(B, n_steps, K, D, N, derivative, d_positions, d_end_derivatives, cand, cost, nullptr, st);
-    if (rc == MINSNAP_OK && e == cudaSuccess)
-      e = minsnap::launch_time_select(B, n_steps, K, cand, cost, time_penalty, d_times, incumbent,
-                                      d_history ? d_history + (size_t)(it + 1) * nb : nullptr, st);
-    if (rc == MINSNAP_OK && e != cudaSuccess) rc = cuda_fail(e, "time descent glue");
+    RC(minsnap_time_gradient(B, K, D, N, derivative, coeffs, d_times, gradient_increment, 0.5, 0.0, grad, nullptr, st));
+    CU(minsnap::launch_time_candidates(B, n_steps, K, d_times, grad, time_penalty, max_relative_step, min_time, cand,
+                                       st));
+    RC(minsnap_cost_sweep(B, n_steps, K, D, N, derivative, d_positions, d_end_derivatives, cand, cost, nullptr, st));
+    CU(minsnap::launch_time_select(B, n_steps, K, cand, cost, time_penalty, d_times, incumbent,
+                                   d_history ? d_history + (size_t)(it + 1) * nb : nullptr, st));
   }
-  cudaFreeAsync(ws, st);
-  return rc;
+  return MINSNAP_OK;
 }
 
 // ---------------------------------------------------------------------------------------
@@ -606,57 +640,69 @@ int soft_args(int N, int n_constraints, const int32_t* h_derivatives, const doub
   return MINSNAP_OK;
 }
 
+// The launch arguments of one soft-cost pass of the constraints `c` (soft_args) over n trajectories; with `objective`
+// set, the pass ends in the objective epilogue on `cost` and `status`.
+minsnap::SoftConstraintArgs soft_cost_args(minsnap::SoftConstraintArgs c, long n, int K, int D, int N,
+                                           const double* coeffs, const double* times, void* scratch, double* soft,
+                                           double* terms, double* max_value, double* objective = nullptr,
+                                           const double* cost = nullptr, const int32_t* status = nullptr,
+                                           double time_penalty = 0.0) {
+  c.B = n; c.K = K; c.D = D; c.N = N;
+  c.d_coeffs = coeffs; c.d_times = times; c.d_scratch = scratch;
+  c.d_soft = soft; c.d_terms = terms; c.d_max_value = max_value;
+  c.d_objective = objective; c.d_cost = cost; c.d_status = status; c.time_penalty = time_penalty;
+  return c;
+}
+
+// The launch arguments of the soft cost's gradient, from the maxima the pass `cost` left in its scratch.
+minsnap::SoftGradientArgs soft_gradient_args(const minsnap::SoftConstraintArgs& cost, const int32_t* col_of_row,
+                                             int n_fixed, int n_free, double* grad_free, double* grad_times,
+                                             bool add_times, double times_weight, double* max_time,
+                                             int32_t* max_segment) {
+  return {cost, col_of_row, n_fixed, n_free, grad_free, grad_times, add_times, times_weight, max_time, max_segment};
+}
+
 // Scratch of the objective pipeline for up to n allocations: positions (and end derivatives) replicated per
 // allocation, coefficients, computeCost, solve status, per-segment maxima.
-struct SoftScratch {
+struct ObjectiveScratch {
   double* positions;
   double* end;
   double* coeffs;
   double* cost;
   int32_t* status;
   void* extrema;
-  static size_t bytes(size_t n, int K, int D, int N, bool with_end, int n_constraints) {
-    const size_t doubles = n * ((size_t)(K + 1) * D + (with_end ? (size_t)(N - 2) * D : 0) + (size_t)K * D * N + 1);
-    return align_up(sizeof(double) * doubles + sizeof(int32_t) * n, 256) +
-           minsnap::soft_constraint_scratch_bytes((long)n, K, n_constraints);
-  }
-  SoftScratch(void* base, size_t n, int K, int D, int N, bool with_end) {
-    positions = static_cast<double*>(base);
-    end = positions + n * (K + 1) * D;
-    coeffs = end + (with_end ? n * (N - 2) * D : 0);
-    cost = coeffs + n * K * D * N;
-    status = reinterpret_cast<int32_t*>(cost + n);
-    extrema = static_cast<char*>(base) + align_up(sizeof(double) * (size_t)(cost + n - positions) + sizeof(int32_t) * n, 256);
+  void take(Regions& r, size_t n, int K, int D, int N, bool with_end, int n_constraints) {
+    positions = r.take<double>(n * (K + 1) * D);
+    end = with_end ? r.take<double>(n * (N - 2) * D) : nullptr;
+    coeffs = r.take<double>(n * K * D * N);
+    cost = r.take<double>(n);
+    status = r.take<int32_t>(n);
+    extrema = r.take<char>(minsnap::soft_constraint_scratch_bytes((long)n, K, n_constraints));
   }
 };
 
-// Solves the R allocations d_times [B R][K] of every trajectory (coefficients, and computeCost and status when
-// want_cost) from its positions replicated R times.
+// Solves the R allocations d_times [B R][K] of every trajectory from its positions replicated R times: coefficients
+// into s.coeffs, computeCost and status into `cost` and `status` when given.
 int solve_replicated(long B, int R, int K, int D, int N, int derivative, const double* d_positions,
-                     const double* d_end_derivatives, const double* d_times, bool want_cost, const SoftScratch& s,
-                     cudaStream_t st) {
+                     const double* d_end_derivatives, const double* d_times, const ObjectiveScratch& s, double* cost,
+                     int32_t* status, cudaStream_t st) {
   CU(minsnap::launch_replicate_rows(B, R, (K + 1) * D, d_positions, s.positions, (N - 2) * D, d_end_derivatives, s.end,
                                     st));
-  return minsnap_solve_standard(B * R, K, D, N, derivative, s.positions, d_end_derivatives ? s.end : nullptr, d_times,
-                                0.0, 0.0, 0.0, nullptr, s.coeffs, nullptr, want_cost ? s.cost : nullptr,
-                                want_cost ? s.status : nullptr, st);
+  return minsnap_solve_standard(B * R, K, D, N, derivative, s.positions, s.end, d_times, 0.0, 0.0, 0.0, nullptr,
+                                s.coeffs, nullptr, cost, status, st);
 }
 
 // minsnap_time_objective_soft on the device: replicate, solve with cost and status, soft cost with the objective
 // epilogue.  d_cost (optional) receives computeCost; without it the scratch holds it.
 int soft_objective_device(long B, int S, int K, int D, int N, int derivative, const double* d_positions,
                           const double* d_end_derivatives, const double* d_times, double time_penalty,
-                          minsnap::SoftConstraintArgs a, double* d_objective, double* d_cost, double* d_soft,
-                          double* d_terms, const SoftScratch& s, cudaStream_t st) {
-  SoftScratch sc = s;
-  if (d_cost) sc.cost = d_cost;
-  const int rc = solve_replicated(B, S, K, D, N, derivative, d_positions, d_end_derivatives, d_times, true, sc, st);
-  if (rc != MINSNAP_OK) return rc;
-  a.B = B * S; a.K = K; a.D = D; a.N = N;
-  a.d_coeffs = sc.coeffs; a.d_times = d_times; a.d_scratch = sc.extrema;
-  a.d_soft = d_soft; a.d_terms = d_terms; a.d_max_value = nullptr;
-  a.d_objective = d_objective; a.d_cost = sc.cost; a.d_status = sc.status; a.time_penalty = time_penalty;
-  CU(minsnap::launch_soft_constraint_cost(a, st));
+                          const minsnap::SoftConstraintArgs& c, double* d_objective, double* d_cost, double* d_soft,
+                          double* d_terms, const ObjectiveScratch& s, cudaStream_t st) {
+  double* cost = d_cost ? d_cost : s.cost;
+  RC(solve_replicated(B, S, K, D, N, derivative, d_positions, d_end_derivatives, d_times, s, cost, s.status, st));
+  CU(minsnap::launch_soft_constraint_cost(soft_cost_args(c, B * S, K, D, N, s.coeffs, d_times, s.extrema, d_soft,
+                                                         d_terms, nullptr, d_objective, cost, s.status, time_penalty),
+                                          st));
   return MINSNAP_OK;
 }
 
@@ -668,21 +714,18 @@ int minsnap_soft_constraint_cost(long B, int K, int D, int N, const double* d_co
                                  double* d_max_value, minsnap_stream_t stream) {
   if (B < 0 || K < 1 || D < 1 || D > 32 || !minsnap::supported_n(N)) return MINSNAP_ERR_ARG;
   minsnap::SoftConstraintArgs a;
-  int rc = soft_args(N, n_constraints, h_derivatives, h_limits, weight, maximum_cost, extrema_flags, &a);
-  if (rc != MINSNAP_OK) return rc;
+  RC(soft_args(N, n_constraints, h_derivatives, h_limits, weight, maximum_cost, extrema_flags, &a));
   if (B == 0) return MINSNAP_OK;
   if (!d_coeffs || !d_times || !d_cost) return MINSNAP_ERR_ARG;
   cudaStream_t st = as_stream(stream);
-  void* scratch = nullptr;
-  retain_pool_memory();
-  CU(cudaMallocAsync(&scratch, minsnap::soft_constraint_scratch_bytes(B, K, n_constraints), st));
-  a.B = B; a.K = K; a.D = D; a.N = N;
-  a.d_coeffs = d_coeffs; a.d_times = d_times; a.d_scratch = scratch;
-  a.d_soft = d_cost; a.d_terms = d_terms; a.d_max_value = d_max_value;
-  const cudaError_t e = minsnap::launch_soft_constraint_cost(a, st);
-  if (e != cudaSuccess) rc = cuda_fail(e, "launch_soft_constraint_cost");
-  cudaFreeAsync(scratch, st);
-  return rc;
+  void* extrema;
+  minsnap::AsyncBuffer ws;
+  RC(alloc_scratch(ws, st, [&](Regions& r) {
+    extrema = r.take<char>(minsnap::soft_constraint_scratch_bytes(B, K, n_constraints));
+  }));
+  CU(minsnap::launch_soft_constraint_cost(
+      soft_cost_args(a, B, K, D, N, d_coeffs, d_times, extrema, d_cost, d_terms, d_max_value), st));
+  return MINSNAP_OK;
 }
 
 int minsnap_time_objective_soft(long B, int S, int K, int D, int N, int derivative, const double* d_positions,
@@ -692,22 +735,18 @@ int minsnap_time_objective_soft(long B, int S, int K, int D, int N, int derivati
                                 double* d_soft, double* d_terms, minsnap_stream_t stream) {
   if (!shape_ok(B, K, D, N, derivative) || S < 1) return MINSNAP_ERR_ARG;
   minsnap::SoftConstraintArgs a;
-  int rc = soft_args(N, n_constraints, h_derivatives, h_limits, weight, maximum_cost, extrema_flags, &a);
-  if (rc != MINSNAP_OK) return rc;
+  RC(soft_args(N, n_constraints, h_derivatives, h_limits, weight, maximum_cost, extrema_flags, &a));
   if (B == 0) return MINSNAP_OK;
   if (!d_positions || !d_times || !d_objective) return MINSNAP_ERR_ARG;
   if (!minsnap::standard_supported(K, D, N, derivative)) return MINSNAP_ERR_UNSUPPORTED;
   cudaStream_t st = as_stream(stream);
-  const size_t n = (size_t)B * S;
-  const bool with_end = d_end_derivatives != nullptr;
-  void* ws = nullptr;
-  retain_pool_memory();
-  CU(cudaMallocAsync(&ws, SoftScratch::bytes(n, K, D, N, with_end, n_constraints), st));
-  const SoftScratch s(ws, n, K, D, N, with_end);
-  rc = soft_objective_device(B, S, K, D, N, derivative, d_positions, d_end_derivatives, d_times, time_penalty, a,
-                             d_objective, d_cost, d_soft, d_terms, s, st);
-  cudaFreeAsync(ws, st);
-  return rc;
+  ObjectiveScratch s;
+  minsnap::AsyncBuffer ws;
+  RC(alloc_scratch(ws, st, [&](Regions& r) {
+    s.take(r, (size_t)B * S, K, D, N, d_end_derivatives != nullptr, n_constraints);
+  }));
+  return soft_objective_device(B, S, K, D, N, derivative, d_positions, d_end_derivatives, d_times, time_penalty, a,
+                               d_objective, d_cost, d_soft, d_terms, s, st);
 }
 
 // The descent of minsnap_optimize_segment_times on the objective with the soft terms, never leaving the device.
@@ -723,77 +762,59 @@ int minsnap_optimize_segment_times_soft(long B, int K, int D, int N, int derivat
                                         double gradient_increment, int n_constraints, const int32_t* h_derivatives,
                                         const double* h_limits, double weight, double maximum_cost, int extrema_flags,
                                         double* d_history, double* d_max_value, minsnap_stream_t stream) {
-  if (!shape_ok(B, K, D, N, derivative) || iterations < 0 || n_steps < 1 || !(max_relative_step > 0.0) ||
-      !(min_time > 0.0) || !(gradient_increment > 0.0))
+  if (!shape_ok(B, K, D, N, derivative) ||
+      !descent_ok(iterations, n_steps, max_relative_step, min_time, gradient_increment))
     return MINSNAP_ERR_ARG;
   minsnap::SoftConstraintArgs a;
-  int rc = soft_args(N, n_constraints, h_derivatives, h_limits, weight, maximum_cost, extrema_flags, &a);
-  if (rc != MINSNAP_OK) return rc;
+  RC(soft_args(N, n_constraints, h_derivatives, h_limits, weight, maximum_cost, extrema_flags, &a));
   if (B == 0) return MINSNAP_OK;
   if (!d_positions || !d_times) return MINSNAP_ERR_ARG;
   if (!minsnap::standard_supported(K, D, N, derivative)) return MINSNAP_ERR_UNSUPPORTED;
   cudaStream_t st = as_stream(stream);
   const size_t nb = (size_t)B, R = std::max<size_t>(2 * (size_t)K, (size_t)n_steps), n = nb * R;
-  const bool with_end = d_end_derivatives != nullptr;
-  const size_t head = align_up(SoftScratch::bytes(n, K, D, N, with_end, n_constraints), 256);
-  char* ws = nullptr;
-  retain_pool_memory();
-  CU(cudaMallocAsync(reinterpret_cast<void**>(&ws), head + sizeof(double) * (n * K + 2 * n + nb * K + nb), st));
-  const SoftScratch s(ws, n, K, D, N, with_end);
-  double* cand = reinterpret_cast<double*>(ws + head);   // [B][R][K]: the 2K differences, then the ladder
-  double* soft = cand + n * K;                          // [B][2K] soft cost of the differences
-  double* obj = soft + n;                               // [B][n_steps] objective of the ladder
-  double* grad = obj + n;
-  double* incumbent = grad + nb * K;
-  a.K = K; a.D = D; a.N = N;
+  ObjectiveScratch s;   // sized for B R allocations: the incumbent, the 2K re-solves and the ladder
+  double *cand, *soft, *obj, *grad, *incumbent;
+  minsnap::AsyncBuffer ws;
+  RC(alloc_scratch(ws, st, [&](Regions& r) {
+    s.take(r, n, K, D, N, d_end_derivatives != nullptr, n_constraints);
+    cand = r.take<double>(n * K);   // [B][R][K]: the 2K differences, then the ladder
+    soft = r.take<double>(n);       // [B][2K] soft cost of the differences
+    obj = r.take<double>(n);        // [B][n_steps] objective of the ladder
+    grad = r.take<double>(nb * K);
+    incumbent = r.take<double>(nb);
+  }));
   // the incumbent objective at the initial times: the candidate pipeline with one allocation per trajectory
-  rc = soft_objective_device(B, 1, K, D, N, derivative, d_positions, d_end_derivatives, d_times, time_penalty, a,
-                             incumbent, nullptr, nullptr, nullptr, s, st);
-  if (rc == MINSNAP_OK && d_history)
-    if (cudaMemcpyAsync(d_history, incumbent, sizeof(double) * nb, cudaMemcpyDeviceToDevice, st) != cudaSuccess) rc = MINSNAP_ERR_CUDA;
-  for (int it = 0; it < iterations && rc == MINSNAP_OK; ++it) {
-    rc = minsnap_solve_standard(B, K, D, N, derivative, d_positions, d_end_derivatives, d_times, 0.0, 0.0, 0.0, nullptr,
-                                s.coeffs, nullptr, nullptr, nullptr, st);
+  RC(soft_objective_device(B, 1, K, D, N, derivative, d_positions, d_end_derivatives, d_times, time_penalty, a,
+                           incumbent, nullptr, nullptr, nullptr, s, st));
+  if (d_history) CU(cudaMemcpyAsync(d_history, incumbent, sizeof(double) * nb, cudaMemcpyDeviceToDevice, st));
+  for (int it = 0; it < iterations; ++it) {
+    RC(minsnap_solve_standard(B, K, D, N, derivative, d_positions, d_end_derivatives, d_times, 0.0, 0.0, 0.0, nullptr,
+                              s.coeffs, nullptr, nullptr, nullptr, st));
     // d computeCost / dT = 0.5 dJ_d/dT (w_d = 0.5, w_t = 0), as minsnap_optimize_segment_times
-    if (rc == MINSNAP_OK)
-      rc = minsnap_time_gradient(B, K, D, N, derivative, s.coeffs, d_times, gradient_increment, 0.5, 0.0, grad, nullptr, st);
-    cudaError_t e = cudaSuccess;
-    if (rc == MINSNAP_OK) e = minsnap::launch_soft_gradient_candidates(B, K, d_times, gradient_increment, cand, st);
-    if (rc == MINSNAP_OK && e == cudaSuccess)
-      rc = solve_replicated(B, 2 * K, K, D, N, derivative, d_positions, d_end_derivatives, cand, false, s, st);
-    if (rc == MINSNAP_OK && e == cudaSuccess) {
-      minsnap::SoftConstraintArgs g = a;
-      g.B = B * 2 * K; g.d_coeffs = s.coeffs; g.d_times = cand; g.d_scratch = s.extrema;
-      g.d_soft = soft; g.d_terms = nullptr; g.d_max_value = nullptr;
-      e = minsnap::launch_soft_constraint_cost(g, st);
-    }
-    if (rc == MINSNAP_OK && e == cudaSuccess) e = minsnap::launch_soft_gradient_add(B, K, soft, gradient_increment, grad, st);
+    RC(minsnap_time_gradient(B, K, D, N, derivative, s.coeffs, d_times, gradient_increment, 0.5, 0.0, grad, nullptr,
+                             st));
+    CU(minsnap::launch_soft_gradient_candidates(B, K, d_times, gradient_increment, cand, st));
+    RC(solve_replicated(B, 2 * K, K, D, N, derivative, d_positions, d_end_derivatives, cand, s, nullptr, nullptr, st));
+    CU(minsnap::launch_soft_constraint_cost(
+        soft_cost_args(a, B * 2 * K, K, D, N, s.coeffs, cand, s.extrema, soft, nullptr, nullptr), st));
+    CU(minsnap::launch_soft_gradient_add(B, K, soft, gradient_increment, grad, st));
     // the ladder adds the penalty's gradient 2 time_penalty sum(T)
-    if (rc == MINSNAP_OK && e == cudaSuccess)
-      e = minsnap::launch_time_candidates(B, n_steps, K, d_times, grad, time_penalty, max_relative_step, min_time, cand, st);
-    if (rc == MINSNAP_OK && e == cudaSuccess)
-      rc = soft_objective_device(B, n_steps, K, D, N, derivative, d_positions, d_end_derivatives, cand, time_penalty, a,
-                                 obj, nullptr, nullptr, nullptr, s, st);
+    CU(minsnap::launch_time_candidates(B, n_steps, K, d_times, grad, time_penalty, max_relative_step, min_time, cand,
+                                       st));
+    RC(soft_objective_device(B, n_steps, K, D, N, derivative, d_positions, d_end_derivatives, cand, time_penalty, a,
+                             obj, nullptr, nullptr, nullptr, s, st));
     // the first minimum among the finite objectives, accepted when strictly below the incumbent (no free values)
-    if (rc == MINSNAP_OK && e == cudaSuccess)
-      e = minsnap::launch_free_select(B, n_steps, 0, K, obj, nullptr, cand, nullptr, nullptr, d_times, incumbent, nullptr,
-                                      d_history ? d_history + (size_t)(it + 1) * nb : nullptr, st);
-    if (rc == MINSNAP_OK && e != cudaSuccess) rc = cuda_fail(e, "soft time descent glue");
+    CU(minsnap::launch_free_select(B, n_steps, 0, K, obj, nullptr, cand, nullptr, nullptr, d_times, incumbent, nullptr,
+                                   d_history ? d_history + (size_t)(it + 1) * nb : nullptr, st));
   }
-  // the maxima at the returned times, from the solve minsnap_solve_standard gives for this batch
-  if (rc == MINSNAP_OK && d_max_value) {
-    rc = minsnap_solve_standard(B, K, D, N, derivative, d_positions, d_end_derivatives, d_times, 0.0, 0.0, 0.0, nullptr,
-                                s.coeffs, nullptr, nullptr, nullptr, st);
-    if (rc == MINSNAP_OK) {
-      minsnap::SoftConstraintArgs m = a;
-      m.B = B; m.d_coeffs = s.coeffs; m.d_times = d_times; m.d_scratch = s.extrema;
-      m.d_soft = nullptr; m.d_terms = nullptr; m.d_max_value = d_max_value;
-      const cudaError_t e = minsnap::launch_soft_constraint_cost(m, st);
-      if (e != cudaSuccess) rc = cuda_fail(e, "launch_soft_constraint_cost");
-    }
+  // the maxima at the returned times, from the solve minsnap_solve_standard gives for this batch; s.coeffs is reused
+  if (d_max_value) {
+    RC(minsnap_solve_standard(B, K, D, N, derivative, d_positions, d_end_derivatives, d_times, 0.0, 0.0, 0.0, nullptr,
+                              s.coeffs, nullptr, nullptr, nullptr, st));
+    CU(minsnap::launch_soft_constraint_cost(
+        soft_cost_args(a, B, K, D, N, s.coeffs, d_times, s.extrema, nullptr, nullptr, d_max_value), st));
   }
-  cudaFreeAsync(ws, st);
-  return rc;
+  return MINSNAP_OK;
 }
 
 // SURVEY 8(f)3: collision cost and its gradient against a dense distance grid (ref NL.i:1523-1709)
@@ -925,17 +946,6 @@ struct SoftTerm {
   double* soft;
 };
 
-// The soft cost of n recovered trajectories, with their maxima (d_max_value, optional) and the scratch left for
-// launch_soft_constraint_gradient.
-cudaError_t launch_soft_term(const SoftTerm& t, long n, int K, int D, int N, const double* coeffs, const double* times,
-                             double* d_soft, double* d_max_value, cudaStream_t st) {
-  minsnap::SoftConstraintArgs a = t.a;
-  a.B = n; a.K = K; a.D = D; a.N = N;
-  a.d_coeffs = coeffs; a.d_times = times; a.d_scratch = t.extrema;
-  a.d_soft = d_soft; a.d_terms = nullptr; a.d_max_value = d_max_value;
-  return minsnap::launch_soft_constraint_cost(a, st);
-}
-
 // minsnap_free_objective on the device, the index map already built: recovery of the B*S candidates (fixed values
 // shared by the S candidates of a trajectory), the collision walk, the combine kernel; with a soft term, its soft cost
 // on the recovered coefficients, added last with weight w_sc.  Scratch: coeffs [B*S][K][D][N], cost and jc [B*S].
@@ -951,11 +961,11 @@ int free_objective_device(long B, int S, int K, int D, int N, int derivative, in
   a.d_coeffs = coeffs;
   a.d_cost = cost;
   CU(minsnap::launch_coeffs_from_constraints(a, st));
-  const int rc = map.cost(n, K, coeffs, d_times, d_jc, d_is_collision, st);
-  if (rc != MINSNAP_OK) return rc;
+  RC(map.cost(n, K, coeffs, d_times, d_jc, d_is_collision, st));
   CU(minsnap::launch_free_combine(n, K, cost, d_jc, d_times, w_d, w_c, w_t, d_objective, d_Jd, st));
   if (soft) {
-    CU(launch_soft_term(*soft, n, K, D, N, coeffs, d_times, soft->soft, nullptr, st));
+    CU(minsnap::launch_soft_constraint_cost(
+        soft_cost_args(soft->a, n, K, D, N, coeffs, d_times, soft->extrema, soft->soft, nullptr, nullptr), st));
     CU(minsnap::launch_free_soft_add(n, soft->soft, soft->w_sc, d_objective, st));
   }
   return MINSNAP_OK;
@@ -992,10 +1002,20 @@ bool mask_fits(int N, int K) { return (long)(K + 1) * (N / 2) <= 32L * minsnap::
 // The soft arguments of the *_soft free-derivative entries on top of soft_args: w_sc >= 0 and finite.
 int free_soft_args(int N, int n_constraints, const int32_t* h_derivatives, const double* h_limits, double weight,
                    double maximum_cost, int extrema_flags, double w_sc, SoftTerm* t) {
-  const int rc = soft_args(N, n_constraints, h_derivatives, h_limits, weight, maximum_cost, extrema_flags, &t->a);
-  if (rc != MINSNAP_OK) return rc;
+  RC(soft_args(N, n_constraints, h_derivatives, h_limits, weight, maximum_cost, extrema_flags, &t->a));
   if (!(w_sc >= 0.0 && std::isfinite(w_sc))) return MINSNAP_ERR_ARG;
   t->w_sc = w_sc;
+  return MINSNAP_OK;
+}
+
+// The checks free_objective_call and free_descent share after their own arguments': the map's, then the mask's
+// counts and, with a soft term, the shapes the mask packing and the recovery kernel take.
+int free_mask_args(long B, int K, int D, int N, const uint8_t* h_fixed_mask, const CollisionMap& map, bool soft,
+                   int* n_fixed, int* n_free) {
+  RC(map.check(B, K, D, N));
+  count_mask(h_fixed_mask, N, K, n_fixed, n_free);
+  if (soft && (!mask_fits(N, K) || minsnap::general_fits(N, K, D, *n_fixed, *n_free) != cudaSuccess))
+    return MINSNAP_ERR_UNSUPPORTED;
   return MINSNAP_OK;
 }
 
@@ -1004,40 +1024,31 @@ int free_objective_call(long B, int S, int K, int D, int N, int derivative, cons
                         double w_c, double w_t, const CollisionMap& map, SoftTerm* soft, double* d_objective,
                         double* d_Jd, double* d_Jc, int32_t* d_is_collision, double* d_soft, cudaStream_t st) {
   if (!shape_ok(B, K, D, N, derivative) || S < 1 || !h_fixed_mask) return MINSNAP_ERR_ARG;
-  int rc = map.check(B, K, D, N);
-  if (rc != MINSNAP_OK) return rc;
   int n_fixed, n_free;
-  count_mask(h_fixed_mask, N, K, &n_fixed, &n_free);
-  if (soft && (!mask_fits(N, K) || minsnap::general_fits(N, K, D, n_fixed, n_free) != cudaSuccess))
-    return MINSNAP_ERR_UNSUPPORTED;
+  RC(free_mask_args(B, K, D, N, h_fixed_mask, map, soft != nullptr, &n_fixed, &n_free));
   if (B == 0) return MINSNAP_OK;
   if (!d_times || !map.sdf || !d_objective || (n_fixed > 0 && !d_fixed_values) || (n_free > 0 && !d_free_values))
     return MINSNAP_ERR_ARG;
   const size_t n = (size_t)B * S;
-  const size_t ws_head = align_up(SolveWorkspace::bytes(N, K), 256);
-  const size_t n_doubles = n * ((size_t)K * D * N + 2 + (soft ? 1 : 0));
-  const size_t extrema = soft ? minsnap::soft_constraint_scratch_bytes((long)n, K, soft->a.n_constraints) : 0;
-  char* ws = nullptr;
-  retain_pool_memory();
-  CU(cudaMallocAsync(reinterpret_cast<void**>(&ws), ws_head + sizeof(double) * n_doubles + extrema, st));
-  SolveWorkspace sw(ws, N, K);
-  double* coeffs = reinterpret_cast<double*>(ws + ws_head);
-  double* cost = coeffs + n * K * D * N;
-  double* jc = cost + n;
-  if (soft) {
-    soft->soft = d_soft ? d_soft : jc + n;
-    soft->extrema = jc + 2 * n;
-  }
-  const cudaError_t e = minsnap::launch_reorder_host_mask(N, K, h_fixed_mask, sw.mask, sw.col_of_row, sw.counts, st);
-  if (e != cudaSuccess) rc = cuda_fail(e, "launch_reorder_host_mask");
-  if (rc == MINSNAP_OK)
-    rc = free_objective_device(B, S, K, D, N, derivative, n_fixed, n_free, sw.col_of_row, d_fixed_values,
-                               d_free_values, d_times, w_d, w_c, w_t, map, d_objective, d_Jd, jc, d_is_collision,
-                               coeffs, cost, st, soft);
-  if (rc == MINSNAP_OK && d_Jc && cudaMemcpyAsync(d_Jc, jc, sizeof(double) * n, cudaMemcpyDeviceToDevice, st) != cudaSuccess)
-    rc = MINSNAP_ERR_CUDA;
-  cudaFreeAsync(ws, st);
-  return rc;
+  char* solve_ws;
+  double *coeffs, *cost, *jc;
+  minsnap::AsyncBuffer ws;
+  RC(alloc_scratch(ws, st, [&](Regions& r) {
+    solve_ws = r.take<char>(SolveWorkspace::bytes(N, K));
+    coeffs = r.take<double>(n * K * D * N);
+    cost = r.take<double>(n);
+    jc = r.take<double>(n);
+    if (soft) {
+      soft->soft = d_soft ? d_soft : r.take<double>(n);
+      soft->extrema = r.take<char>(minsnap::soft_constraint_scratch_bytes((long)n, K, soft->a.n_constraints));
+    }
+  }));
+  const SolveWorkspace sw(solve_ws, N, K);
+  CU(minsnap::launch_reorder_host_mask(N, K, h_fixed_mask, sw.mask, sw.col_of_row, sw.counts, st));
+  RC(free_objective_device(B, S, K, D, N, derivative, n_fixed, n_free, sw.col_of_row, d_fixed_values, d_free_values,
+                           d_times, w_d, w_c, w_t, map, d_objective, d_Jd, jc, d_is_collision, coeffs, cost, st, soft));
+  if (d_Jc) CU(cudaMemcpyAsync(d_Jc, jc, sizeof(double) * n, cudaMemcpyDeviceToDevice, st));
+  return MINSNAP_OK;
 }
 
 // The descent of minsnap_optimize_free_constraints; with a soft term (minsnap_optimize_free_constraints_soft) its
@@ -1047,113 +1058,95 @@ int free_descent(long B, int K, int D, int N, int derivative, const uint8_t* h_f
                  const CollisionMap& map, SoftTerm* soft, int iterations, int n_steps, double max_relative_step,
                  double min_time, double gradient_increment, double* d_history, int32_t* d_is_collision,
                  double* d_max_value, cudaStream_t st) {
-  if (!shape_ok(B, K, D, N, derivative) || !h_fixed_mask || iterations < 0 || n_steps < 1 || !(w_d > 0.0) ||
-      !(max_relative_step > 0.0) || !(min_time > 0.0) || !(gradient_increment > 0.0))
+  if (!shape_ok(B, K, D, N, derivative) || !h_fixed_mask || !(w_d > 0.0) ||
+      !descent_ok(iterations, n_steps, max_relative_step, min_time, gradient_increment))
     return MINSNAP_ERR_ARG;
-  int rc = map.check(B, K, D, N);
-  if (rc != MINSNAP_OK) return rc;
   int n_fixed, n_free;
-  count_mask(h_fixed_mask, N, K, &n_fixed, &n_free);
-  if (soft && (!mask_fits(N, K) || minsnap::general_fits(N, K, D, n_fixed, n_free) != cudaSuccess))
-    return MINSNAP_ERR_UNSUPPORTED;
+  RC(free_mask_args(B, K, D, N, h_fixed_mask, map, soft != nullptr, &n_fixed, &n_free));
   if (B == 0) return MINSNAP_OK;
   if (!d_times || !map.sdf || (n_fixed > 0 && !d_fixed_values) || (n_free > 0 && !d_free_values)) return MINSNAP_ERR_ARG;
   const size_t nb = (size_t)B, S = (size_t)n_steps, nfd = (size_t)n_free * D, nc = (size_t)K * D * N;
-  const size_t ws_head = align_up(SolveWorkspace::bytes(N, K), 256);
-  const size_t n_doubles = nb * (nc + 2 * nfd + n_free + K + 3) + nb * S * (nfd + K + nc + 3);
-  const size_t n_ints = nb * (S + 1);
-  // soft term: g_sc [B][n_free][D], the candidates' soft cost [B S], per-segment maxima of B S trajectories
-  const size_t soft_doubles = soft ? nb * nfd + nb * S : 0;
-  const size_t soft_head = align_up(sizeof(double) * n_doubles + sizeof(int32_t) * n_ints, 256);
-  char* ws = nullptr;
-  retain_pool_memory();
-  if (soft)
-    CU(cudaMallocAsync(reinterpret_cast<void**>(&ws), ws_head + soft_head + sizeof(double) * soft_doubles +
-                       minsnap::soft_constraint_scratch_bytes((long)(nb * S), K, soft->a.n_constraints), st));
-  else
-    CU(cudaMallocAsync(reinterpret_cast<void**>(&ws), ws_head + sizeof(double) * n_doubles + sizeof(int32_t) * n_ints, st));
-  SolveWorkspace sw(ws, N, K);
-  double* coeffs = reinterpret_cast<double*>(ws + ws_head);   // the incumbent's
-  double* grad_d = coeffs + nb * nc;
-  double* grad_c = grad_d + nb * nfd;
-  double* diag = grad_c + nb * nfd;
-  double* grad_t = diag + nb * n_free;
-  double* jd = grad_t + nb * K;
-  double* jc = jd + nb;
-  double* incumbent = jc + nb;
-  double* cand_free = incumbent + nb;
-  double* cand_times = cand_free + nb * S * nfd;
-  double* cand_coeffs = cand_times + nb * S * K;
-  double* cand_cost = cand_coeffs + nb * S * nc;
-  double* cand_jc = cand_cost + nb * S;
-  double* cand_obj = cand_jc + nb * S;
-  int32_t* cand_hit = reinterpret_cast<int32_t*>(cand_obj + nb * S);
-  int32_t* hit = d_is_collision ? d_is_collision : cand_hit + nb * S;
-  double* grad_sc = nullptr;
-  if (soft) {
-    grad_sc = reinterpret_cast<double*>(ws + ws_head + soft_head);
-    soft->soft = grad_sc + nb * nfd;
-    soft->extrema = soft->soft + nb * S;
-  }
-  cudaError_t e = minsnap::launch_reorder_host_mask(N, K, h_fixed_mask, sw.mask, sw.col_of_row, sw.counts, st);
-  if (e != cudaSuccess) rc = cuda_fail(e, "launch_reorder_host_mask");
+  char* solve_ws;
+  double *coeffs, *grad_d, *grad_c, *diag, *grad_t, *jd, *jc, *incumbent;
+  double *cand_free, *cand_times, *cand_coeffs, *cand_cost, *cand_jc, *cand_obj, *grad_sc = nullptr;
+  int32_t *cand_hit, *hit;
+  minsnap::AsyncBuffer ws;
+  RC(alloc_scratch(ws, st, [&](Regions& r) {
+    solve_ws = r.take<char>(SolveWorkspace::bytes(N, K));
+    coeffs = r.take<double>(nb * nc);   // the incumbent's
+    grad_d = r.take<double>(nb * nfd);
+    grad_c = r.take<double>(nb * nfd);
+    diag = r.take<double>(nb * n_free);
+    grad_t = r.take<double>(nb * K);
+    jd = r.take<double>(nb);
+    jc = r.take<double>(nb);
+    incumbent = r.take<double>(nb);
+    // the candidates' buffers, shared by the incumbent's evaluation (one candidate per trajectory) and the ladder
+    cand_free = r.take<double>(nb * S * nfd);
+    cand_times = r.take<double>(nb * S * K);
+    cand_coeffs = r.take<double>(nb * S * nc);
+    cand_cost = r.take<double>(nb * S);
+    cand_jc = r.take<double>(nb * S);
+    cand_obj = r.take<double>(nb * S);
+    cand_hit = r.take<int32_t>(nb * S);
+    int32_t* own_hit = r.take<int32_t>(nb);
+    hit = d_is_collision ? d_is_collision : own_hit;
+    // soft term: g_sc [B][n_free][D], the candidates' soft cost [B S], per-segment maxima of B S trajectories
+    if (soft) {
+      grad_sc = r.take<double>(nb * nfd);
+      soft->soft = r.take<double>(nb * S);
+      soft->extrema = r.take<char>(minsnap::soft_constraint_scratch_bytes((long)(nb * S), K, soft->a.n_constraints));
+    }
+  }));
+  const SolveWorkspace sw(solve_ws, N, K);
+  CU(minsnap::launch_reorder_host_mask(N, K, h_fixed_mask, sw.mask, sw.col_of_row, sw.counts, st));
   // the incumbent objective at the initial state: the candidate pipeline with one candidate per trajectory
-  if (rc == MINSNAP_OK)
-    rc = free_objective_device(B, 1, K, D, N, derivative, n_fixed, n_free, sw.col_of_row, d_fixed_values, d_free_values,
-                               d_times, w_d, w_c, w_t, map, incumbent, nullptr, cand_jc, hit, cand_coeffs, cand_cost, st,
-                               soft);
-  if (rc == MINSNAP_OK && d_history)
-    if (cudaMemcpyAsync(d_history, incumbent, sizeof(double) * nb, cudaMemcpyDeviceToDevice, st) != cudaSuccess) rc = MINSNAP_ERR_CUDA;
-  for (int it = 0; it < iterations && rc == MINSNAP_OK; ++it) {
+  RC(free_objective_device(B, 1, K, D, N, derivative, n_fixed, n_free, sw.col_of_row, d_fixed_values, d_free_values,
+                           d_times, w_d, w_c, w_t, map, incumbent, nullptr, cand_jc, hit, cand_coeffs, cand_cost, st,
+                           soft));
+  if (d_history) CU(cudaMemcpyAsync(d_history, incumbent, sizeof(double) * nb, cudaMemcpyDeviceToDevice, st));
+  for (int it = 0; it < iterations; ++it) {
     minsnap::GeneralSolveArgs a =
         recovery_args(B, K, D, N, derivative, n_fixed, n_free, sw.col_of_row, d_fixed_values, d_free_values, d_times);
     a.d_coeffs = coeffs; a.d_cost = jd; a.d_grad_free = grad_d; a.d_diag_free = diag;
-    e = minsnap::launch_derivative_gradient(a, st);
-    if (e == cudaSuccess) rc = map.gradient(B, K, coeffs, d_times, sw.col_of_row, n_fixed, n_free, jc, grad_c, st);
-    if (e == cudaSuccess && rc == MINSNAP_OK && optimize_times)
-      rc = minsnap_time_gradient(B, K, D, N, derivative, coeffs, d_times, gradient_increment, w_d, w_t, grad_t, nullptr, st);
+    CU(minsnap::launch_derivative_gradient(a, st));
+    RC(map.gradient(B, K, coeffs, d_times, sw.col_of_row, n_fixed, n_free, jc, grad_c, st));
+    if (optimize_times)
+      RC(minsnap_time_gradient(B, K, D, N, derivative, coeffs, d_times, gradient_increment, w_d, w_t, grad_t, nullptr,
+                               st));
     // the soft term at the incumbent: its maxima, then g_sc, and w_sc dsoft/dT added to the time gradient
-    if (e == cudaSuccess && rc == MINSNAP_OK && soft) {
-      e = launch_soft_term(*soft, B, K, D, N, coeffs, d_times, nullptr, nullptr, st);
-      if (e == cudaSuccess) {
-        minsnap::SoftGradientArgs g;
-        g.soft = soft->a;
-        g.soft.B = B; g.soft.K = K; g.soft.D = D; g.soft.N = N;
-        g.soft.d_coeffs = coeffs; g.soft.d_times = d_times; g.soft.d_scratch = soft->extrema;
-        g.d_col_of_row = sw.col_of_row; g.n_fixed = n_fixed; g.n_free = n_free;
-        g.d_grad_free = grad_sc;
-        g.d_grad_times = optimize_times ? grad_t : nullptr;
-        g.add_times = true;
-        g.times_weight = soft->w_sc;
-        e = minsnap::launch_soft_constraint_gradient(g, st);
-      }
+    if (soft) {
+      const minsnap::SoftConstraintArgs c =
+          soft_cost_args(soft->a, B, K, D, N, coeffs, d_times, soft->extrema, nullptr, nullptr, nullptr);
+      CU(minsnap::launch_soft_constraint_cost(c, st));
+      CU(minsnap::launch_soft_constraint_gradient(
+          soft_gradient_args(c, sw.col_of_row, n_fixed, n_free, grad_sc, optimize_times ? grad_t : nullptr, true,
+                             soft->w_sc, nullptr, nullptr),
+          st));
     }
-    if (e == cudaSuccess && rc == MINSNAP_OK && optimize_times)
-      e = minsnap::launch_time_candidates(B, n_steps, K, d_times, grad_t, 0.0, max_relative_step, min_time, cand_times, st);
-    if (e == cudaSuccess && rc == MINSNAP_OK)
-      e = minsnap::launch_free_candidates(B, n_steps, n_free, D, K, d_free_values, grad_d, grad_c, diag, w_d, w_c, d_times,
-                                          cand_free, optimize_times ? nullptr : cand_times, st, grad_sc,
-                                          soft ? soft->w_sc : 0.0);
-    if (e == cudaSuccess && rc == MINSNAP_OK)
-      rc = free_objective_device(B, n_steps, K, D, N, derivative, n_fixed, n_free, sw.col_of_row, d_fixed_values,
-                                 cand_free, cand_times, w_d, w_c, w_t, map, cand_obj, nullptr, cand_jc, cand_hit,
-                                 cand_coeffs, cand_cost, st, soft);
-    if (e == cudaSuccess && rc == MINSNAP_OK)
-      e = minsnap::launch_free_select(B, n_steps, (int)nfd, K, cand_obj, cand_free, cand_times, cand_hit, d_free_values,
-                                      d_times, incumbent, hit, d_history ? d_history + (size_t)(it + 1) * nb : nullptr, st);
-    if (rc == MINSNAP_OK && e != cudaSuccess) rc = cuda_fail(e, "free-constraint descent");
+    if (optimize_times)
+      CU(minsnap::launch_time_candidates(B, n_steps, K, d_times, grad_t, 0.0, max_relative_step, min_time, cand_times,
+                                         st));
+    CU(minsnap::launch_free_candidates(B, n_steps, n_free, D, K, d_free_values, grad_d, grad_c, diag, w_d, w_c, d_times,
+                                       cand_free, optimize_times ? nullptr : cand_times, st, grad_sc,
+                                       soft ? soft->w_sc : 0.0));
+    RC(free_objective_device(B, n_steps, K, D, N, derivative, n_fixed, n_free, sw.col_of_row, d_fixed_values, cand_free,
+                             cand_times, w_d, w_c, w_t, map, cand_obj, nullptr, cand_jc, cand_hit, cand_coeffs,
+                             cand_cost, st, soft));
+    CU(minsnap::launch_free_select(B, n_steps, (int)nfd, K, cand_obj, cand_free, cand_times, cand_hit, d_free_values,
+                                   d_times, incumbent, hit, d_history ? d_history + (size_t)(it + 1) * nb : nullptr,
+                                   st));
   }
   // the maxima at the returned state, from its recovered coefficients
-  if (rc == MINSNAP_OK && soft && d_max_value) {
+  if (soft && d_max_value) {
     minsnap::GeneralSolveArgs a =
         recovery_args(B, K, D, N, derivative, n_fixed, n_free, sw.col_of_row, d_fixed_values, d_free_values, d_times);
     a.d_coeffs = coeffs;
-    e = minsnap::launch_coeffs_from_constraints(a, st);
-    if (e == cudaSuccess) e = launch_soft_term(*soft, B, K, D, N, coeffs, d_times, nullptr, d_max_value, st);
-    if (e != cudaSuccess) rc = cuda_fail(e, "soft-limit maxima");
+    CU(minsnap::launch_coeffs_from_constraints(a, st));
+    CU(minsnap::launch_soft_constraint_cost(
+        soft_cost_args(soft->a, B, K, D, N, coeffs, d_times, soft->extrema, nullptr, nullptr, d_max_value), st));
   }
-  cudaFreeAsync(ws, st);
-  return rc;
+  return MINSNAP_OK;
 }
 
 }  // namespace
@@ -1202,36 +1195,28 @@ int minsnap_soft_constraint_gradient(long B, int K, int D, int N, const uint8_t*
                                      double* d_max_time, int32_t* d_max_segment, minsnap_stream_t stream) {
   if (B < 0 || K < 1 || D < 1 || D > 32 || !minsnap::supported_n(N) || !h_fixed_mask) return MINSNAP_ERR_ARG;
   SoftTerm t;
-  int rc = free_soft_args(N, n_constraints, h_derivatives, h_limits, weight, maximum_cost, extrema_flags, 0.0, &t);
-  if (rc != MINSNAP_OK) return rc;
+  RC(free_soft_args(N, n_constraints, h_derivatives, h_limits, weight, maximum_cost, extrema_flags, 0.0, &t));
   if (!mask_fits(N, K)) return MINSNAP_ERR_UNSUPPORTED;
   int n_fixed, n_free;
   count_mask(h_fixed_mask, N, K, &n_fixed, &n_free);
   if (B == 0) return MINSNAP_OK;
   if (!d_coeffs || !d_times || (n_free > 0 && !d_grad_free)) return MINSNAP_ERR_ARG;
   cudaStream_t st = as_stream(stream);
-  const size_t ws_head = align_up(SolveWorkspace::bytes(N, K), 256);
-  char* ws = nullptr;
-  retain_pool_memory();
-  CU(cudaMallocAsync(reinterpret_cast<void**>(&ws), ws_head + minsnap::soft_constraint_scratch_bytes(B, K, n_constraints),
-                     st));
-  SolveWorkspace sw(ws, N, K);
-  t.extrema = ws + ws_head;
-  cudaError_t e = minsnap::launch_reorder_host_mask(N, K, h_fixed_mask, sw.mask, sw.col_of_row, sw.counts, st);
-  if (e == cudaSuccess) e = launch_soft_term(t, B, K, D, N, d_coeffs, d_times, d_cost, d_max_value, st);
-  if (e == cudaSuccess) {
-    minsnap::SoftGradientArgs g;
-    g.soft = t.a;
-    g.soft.B = B; g.soft.K = K; g.soft.D = D; g.soft.N = N;
-    g.soft.d_coeffs = d_coeffs; g.soft.d_times = d_times; g.soft.d_scratch = t.extrema;
-    g.d_col_of_row = sw.col_of_row; g.n_fixed = n_fixed; g.n_free = n_free;
-    g.d_grad_free = d_grad_free; g.d_grad_times = d_grad_times;
-    g.d_max_time = d_max_time; g.d_max_segment = d_max_segment;
-    e = minsnap::launch_soft_constraint_gradient(g, st);
-  }
-  if (e != cudaSuccess) rc = cuda_fail(e, "soft-limit gradient");
-  cudaFreeAsync(ws, st);
-  return rc;
+  char* solve_ws;
+  minsnap::AsyncBuffer ws;
+  RC(alloc_scratch(ws, st, [&](Regions& r) {
+    solve_ws = r.take<char>(SolveWorkspace::bytes(N, K));
+    t.extrema = r.take<char>(minsnap::soft_constraint_scratch_bytes(B, K, n_constraints));
+  }));
+  const SolveWorkspace sw(solve_ws, N, K);
+  CU(minsnap::launch_reorder_host_mask(N, K, h_fixed_mask, sw.mask, sw.col_of_row, sw.counts, st));
+  const minsnap::SoftConstraintArgs c =
+      soft_cost_args(t.a, B, K, D, N, d_coeffs, d_times, t.extrema, d_cost, nullptr, d_max_value);
+  CU(minsnap::launch_soft_constraint_cost(c, st));
+  CU(minsnap::launch_soft_constraint_gradient(soft_gradient_args(c, sw.col_of_row, n_fixed, n_free, d_grad_free,
+                                                                 d_grad_times, false, 1.0, d_max_time, d_max_segment),
+                                              st));
+  return MINSNAP_OK;
 }
 
 int minsnap_free_objective_soft(long B, int S, int K, int D, int N, int derivative, const uint8_t* h_fixed_mask,
@@ -1244,8 +1229,7 @@ int minsnap_free_objective_soft(long B, int S, int K, int D, int N, int derivati
                                 double maximum_cost, int extrema_flags, double w_sc, double* d_objective, double* d_Jd,
                                 double* d_Jc, int32_t* d_is_collision, double* d_soft, minsnap_stream_t stream) {
   SoftTerm t;
-  const int rc = free_soft_args(N, n_constraints, h_derivatives, h_limits, weight, maximum_cost, extrema_flags, w_sc, &t);
-  if (rc != MINSNAP_OK) return rc;
+  RC(free_soft_args(N, n_constraints, h_derivatives, h_limits, weight, maximum_cost, extrema_flags, w_sc, &t));
   const CollisionMap map{d_sdf, h_dims, h_origin, resolution, oob_value, h_min_bound, h_max_bound,
                          use_continuous_distance, dt, map_resolution, epsilon, robot_radius, coll_pot_multiplier};
   return free_objective_call(B, S, K, D, N, derivative, h_fixed_mask, d_fixed_values, d_free_values, d_times, w_d, w_c,
@@ -1265,8 +1249,7 @@ int minsnap_optimize_free_constraints_soft(long B, int K, int D, int N, int deri
                                            double gradient_increment, double* d_history, int32_t* d_is_collision,
                                            double* d_max_value, minsnap_stream_t stream) {
   SoftTerm t;
-  const int rc = free_soft_args(N, n_constraints, h_derivatives, h_limits, weight, maximum_cost, extrema_flags, w_sc, &t);
-  if (rc != MINSNAP_OK) return rc;
+  RC(free_soft_args(N, n_constraints, h_derivatives, h_limits, weight, maximum_cost, extrema_flags, w_sc, &t));
   const CollisionMap map{d_sdf, h_dims, h_origin, resolution, oob_value, h_min_bound, h_max_bound,
                          use_continuous_distance, dt, map_resolution, epsilon, robot_radius, coll_pot_multiplier};
   return free_descent(B, K, D, N, derivative, h_fixed_mask, d_fixed_values, d_free_values, d_times, optimize_times, w_d,
@@ -1471,30 +1454,28 @@ int minsnap_solve_standard_host(long B, int K, int D, int N, int derivative, con
   const long chunk = std::min<long>(B, 4096);
   // Stage layout: one device block per pipeline stage, carved into the per-chunk arrays.
   const size_t nc = (size_t)chunk;
-  size_t off = 0;
-  auto carve = [&off](size_t bytes) { const size_t at = off; off += align_up(bytes ? bytes : 16, 256); return at; };
-  const size_t o_pos = carve(sizeof(double) * nc * (K + 1) * D);
-  const size_t o_end = carve(h_end_derivatives ? sizeof(double) * nc * 2 * (h - 1) * D : 0);
-  const size_t o_tm = carve(sizeof(double) * nc * K);
-  const size_t o_co = carve(sizeof(double) * nc * K * D * N);
-  const size_t o_fr = carve(h_free_values ? sizeof(double) * nc * (n_free > 0 ? n_free : 1) * D : 0);
-  const size_t o_cs = carve(h_cost ? sizeof(double) * nc : 0);
-  const size_t o_ss = carve(h_status ? sizeof(int32_t) * nc : 0);
-  CU(g_pipeline.ensure(off));
+  double *d_pos, *d_end, *d_tm, *d_co, *d_fr, *d_cs;
+  int32_t* d_ss;
+  auto layout = [&](Regions& r) {
+    d_pos = r.take<double>(nc * (K + 1) * D);
+    d_end = r.take<double>(h_end_derivatives ? nc * 2 * (h - 1) * D : 0);
+    d_tm = r.take<double>(nc * K);
+    d_co = r.take<double>(nc * K * D * N);
+    d_fr = r.take<double>(h_free_values ? nc * (n_free > 0 ? n_free : 1) * D : 0);
+    d_cs = r.take<double>(h_cost ? nc : 0);
+    d_ss = r.take<int32_t>(h_status ? nc : 0);
+  };
+  Regions stage_size;
+  layout(stage_size);
+  CU(g_pipeline.ensure(stage_size.bytes));
   int rc = MINSNAP_OK;
   {
     int stage = 0;
     for (long b0 = 0; b0 < B; b0 += chunk, stage = (stage + 1) % HostPipeline::kDepth) {
       const long nb = std::min(chunk, B - b0);
       cudaStream_t st = g_pipeline.stream[stage];
-      char* base = g_pipeline.block[stage];
-      double* d_pos = reinterpret_cast<double*>(base + o_pos);
-      double* d_end = reinterpret_cast<double*>(base + o_end);
-      double* d_tm = reinterpret_cast<double*>(base + o_tm);
-      double* d_co = reinterpret_cast<double*>(base + o_co);
-      double* d_fr = reinterpret_cast<double*>(base + o_fr);
-      double* d_cs = reinterpret_cast<double*>(base + o_cs);
-      int32_t* d_ss = reinterpret_cast<int32_t*>(base + o_ss);
+      Regions at{g_pipeline.block[stage]};
+      layout(at);
       TRY(cudaMemcpyAsync(d_pos, h_positions + (size_t)b0 * (K + 1) * D, sizeof(double) * nb * (K + 1) * D,
                           cudaMemcpyHostToDevice, st));
       if (h_end_derivatives)

@@ -128,19 +128,6 @@ __device__ inline double warp_sum(double v) {
   return v;
 }
 
-// Stream-ordered scratch memory, freed on `stream` when it goes out of scope (after the work enqueued so far).
-struct AsyncBuffer {
-  void* ptr = nullptr;
-  cudaStream_t stream = nullptr;
-  cudaError_t alloc(size_t bytes, cudaStream_t s) {
-    stream = s;
-    return cudaMallocAsync(&ptr, bytes ? bytes : 16, s);
-  }
-  ~AsyncBuffer() {
-    if (ptr) cudaFreeAsync(ptr, stream);
-  }
-};
-
 // f(std::integral_constant<int, D>) for the dimension counts D = 1..3 the standard-mask kernels are compiled for.
 template <class F>
 inline cudaError_t with_dim(int D, F&& f) {

@@ -27,6 +27,19 @@ inline long sm_count() {
 
 bool supported_n(int N);
 
+// Stream-ordered scratch memory, freed on `stream` when it goes out of scope (after the work enqueued so far).
+struct AsyncBuffer {
+  void* ptr = nullptr;
+  cudaStream_t stream = nullptr;
+  cudaError_t alloc(size_t bytes, cudaStream_t s) {
+    stream = s;
+    return cudaMallocAsync(&ptr, bytes ? bytes : 16, s);
+  }
+  ~AsyncBuffer() {
+    if (ptr) cudaFreeAsync(ptr, stream);
+  }
+};
+
 // ---- minsnap_general.cu ----------------------------------------------------------------
 cudaError_t launch_reorder(int N, int K, long n_masks, const uint8_t* d_mask, int32_t* d_col_of_row,
                            int32_t* d_counts, cudaStream_t stream);
